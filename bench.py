@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: STARK proofs per second (and ms per proof) for the reference's proving path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl zkb200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl zkb200|reference] [--dump-outputs DIR]
 
 A step is `--inflight` (default 4) complete proofs per GPU (`Prover::prove`, /root/reference src/main.rs:228), each of its own
 seeded synthetic trace, kept in flight on separate contexts; `prove_ms` is the latency of one proof proved alone.
@@ -153,13 +153,33 @@ def mimc_air(opts, w, n, first, last):
     return Z.MimcAir(w, n, pub, opts).describe()
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(path, results):
+    """--dump-outputs: what the timed path returned in its last step, one row per proof of that step.  `proof.npy` holds the
+    proof bytes (float32, one byte per element) and `transcript_<field>.npy` the Fiat-Shamir transcript returned with each proof
+    (float64; every field is an integer below 2^53).  The proofs are deterministic (the smallest proof-of-work nonce), so two
+    builds run with the same arguments must write the same arrays.  Rows beyond 64 MB in all are left out."""
+    import ctypes
+    row_bytes = 4 * len(results[0][0]) + 8 * ctypes.sizeof(results[0][1])  # a transcript has fewer fields than bytes
+    results = results[:max(1, DUMP_LIMIT // row_bytes)]
+    arrays = {"proof": np.stack([np.frombuffer(p, dtype=np.uint8) for p, _ in results]).astype(np.float32)}
+    for name, _ in results[0][1]._fields_:
+        if not name.startswith("_"):
+            vals = [getattr(ts, name) for _, ts in results]
+            arrays["transcript_" + name] = np.array([np.ctypeslib.as_array(v) if hasattr(v, "_length_") else v for v in vals], dtype=np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_reference(args, rank, world):
     """CPU arm: the oracle prover (restatement of Winterfell's CPU prover) on all host cores."""
     if rank != 0:
         return
     from oracle import pyoracle as O
     import zk_stark_project_b200 as Z
-    O.build()
     cores = os.cpu_count() or 1
     O.set_threads(cores)
     kind, n, w, beta, desc = WORKLOADS[args.workload]
@@ -175,8 +195,10 @@ def run_reference(args, rank, world):
         O.prove(air, tb)
     t0 = time.time()
     for _ in range(args.steps):
-        O.prove(air, tb)
+        proof, ts, _ = O.prove(air, tb)
     dt = (time.time() - t0) / args.steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [(proof, ts)])
     val = 1.0 / dt
     line = {
         "impl": "reference", "metric": "stark_proofs_per_sec", "value": val, "unit": "proofs/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -384,7 +406,13 @@ def main():
     ap.add_argument("--sharded", action="store_true",
                     help="make the column-sharded proof of --workload the MAIN arm (ONE proof per step across all ranks, strong scaling) "
                          "instead of one independent proof stream per rank")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the proofs of the last step of the throughput arm (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.workload == "mimc_helpers":
+        ap.error("--dump-outputs covers the proof workloads")
     capture_stdout()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -538,6 +566,7 @@ def main():
     launches = launches_per_proof * args.steps * inflight
     ms = e0.elapsed_time(e1)
     assert all(r[0] == proof for r in res), "in-flight proofs differ from the single-stream proof"
+    last_step = res
     # ---- end-to-end arm: host columns in pinned memory through zkb_prove, same concurrency ----------------------------------------
     run_lanes(host_fn, min(args.warmup, 2))
     barrier()
@@ -747,7 +776,6 @@ def main():
                 line["sharded_training_2p20"] = sharded_recs[1]
         if world == 1 and not args.no_cpu_baseline:
             from oracle import pyoracle as O
-            O.build()
             cores = os.cpu_count() or 1
             O.set_threads(cores)
             t0 = time.time()
@@ -757,6 +785,8 @@ def main():
                                     "sample": "1 full proof of the same workload (C++ restatement of Winterfell's CPU prover: std::thread over columns / rows on "
                                               "all host cores, portable scalar BLAKE3 - upstream uses the SIMD blake3 crate; not Winterfell itself)",
                                     "proof_identical_to_gpu": ref == proof}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_step)
         emit(line)
     if world > 1:
         dist.destroy_process_group()

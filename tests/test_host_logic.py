@@ -197,6 +197,26 @@ def test_bench_counter_trace_is_seekable_and_canonical():
     assert a == b
 
 
+def test_bench_dump_outputs(oracle, tmp_path):
+    """bench.py --dump-outputs (CPU arm, so no GPU is needed): float arrays that decode back to the proof of the last timed
+    step, which the verifier accepts, and the transcript that came with it; --steps is the number of timed steps."""
+    import json
+    import subprocess
+    import sys
+    import bench
+    cmd = [sys.executable, bench.__file__, "--impl", "reference", "--workload", "aggregation_16", "--warmup", "0", "--dump-outputs", str(tmp_path)]
+    r = subprocess.run(cmd + ["--steps", "2"], capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout)["steps"] == 2
+    arrays = {p.stem: np.load(p) for p in tmp_path.glob("*.npy")}
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values()) and sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    proof = arrays["proof"][0].astype(np.uint8).tobytes()
+    air, _, _ = bench.build_workload("aggregation_16", 0x5EED0000)
+    ts = oracle.verify(air, proof)
+    assert arrays["transcript_z"][0].astype(np.uint8).tobytes() == bytes(ts.z)
+    assert subprocess.run(cmd + ["--steps", "0"], capture_output=True).returncode == 2
+
+
 def test_bench_algorithmic_bytes_match_survey():
     """SURVEY §8(d) totals: 9.47 GiB at configs[1], 33.5 GiB / 151.6 GiB at the two 2^20-row headline shapes."""
     import bench
