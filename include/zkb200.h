@@ -161,7 +161,8 @@ int32_t zkb_grind(zkb_ctx* ctx, const uint8_t seed[32], uint32_t bits, uint64_t*
 /* TraceLde::query / ConstraintCommitment::query / FriProver::build_proof: K11.
  * which: 0 = trace (any time after zkb_trace_commit), 1 = constraint composition (after zkb_constraints_commit),
  *        2+l = FRI layer l (after zkb_fri_remainder; positions already folded by the caller).
- * rows_out: n_pos rows, row-major; proof_out: BatchMerkleProof::to_bytes(), allocated by the library. */
+ * rows_out: n_pos rows, row-major; proof_out: BatchMerkleProof::to_bytes(), allocated by the library.
+ * After a column-sharded proof (zkb_mg_prove*) the context holds only this rank's share of the trace: ZKB_ERR_STATE. */
 int32_t zkb_query(zkb_ctx* ctx, uint32_t which, const uint32_t* positions, uint32_t n_pos, uint8_t* rows_out,
                   uint8_t** proof_out, uint64_t* proof_len);
 
@@ -171,7 +172,7 @@ int32_t zkb_query(zkb_ctx* ctx, uint32_t which, const uint32_t* positions, uint3
  * roots are all-gathered; constraint evaluation, OOD and DEEP are column-local partial sums combined by an all-gather.
  * `air` describes the WHOLE trace (global width, all assertions); `local_cols` holds this rank's w/G columns.
  * The Fiat-Shamir channel runs replicated on every rank's device (all ranks hold the same commitments, OOD frame and
- * remainder); the host is met twice per proof: for the query positions and for the batched openings.
+ * remainder) and the openings are completed by one all-reduce: the host is met once per proof, for the final download.
  * Every rank returns the same proof bytes.  G must be a power of two that divides w (and at most the LDE panel size);
  * the aggregation AIR couples columns i and i+60 and is not shardable. */
 int32_t zkb_mg_unique_id(uint8_t out[128]);                                         /* ncclGetUniqueId, on rank 0 */

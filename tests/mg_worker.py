@@ -12,6 +12,7 @@ import time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 import numpy as np  # noqa: E402
+import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 
 import zk_stark_project_b200 as Z  # noqa: E402
@@ -22,7 +23,12 @@ from zk_stark_project_b200 import synthetic as S  # noqa: E402
 def main():
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ.get("LOCAL_RANK", "0"))
     dist.init_process_group("gloo")
-    ctx = L.Context(local)
+    ndev = torch.cuda.device_count()
+    if ndev < world:
+        # more ranks than GPUs (the sharded path tested on one GPU): NCCL refuses two ranks of one host on one device, so each
+        # rank presents its own host id and the ranks exchange data over NCCL's socket transport
+        os.environ["NCCL_HOSTID"] = f"zkb-mg-worker-rank-{rank}"
+    ctx = L.Context(local % ndev)
     ids = [L.mg_unique_id() if rank == 0 else None]
     dist.broadcast_object_list(ids, src=0)
     ctx.mg_init(rank, world, ids[0])

@@ -215,6 +215,23 @@ def test_column_sharded_proof_two_gpus():
     assert r.returncode == 0 and "mg ok" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
 
 
+def test_column_sharded_proof_ranks_share_one_gpu():
+    """The sharded path with 2 and 4 ranks on one GPU, the ranks talking over NCCL's socket transport: rows and authentication
+    nodes owned by one rank, the cap levels of the trace paths, the all-reduce of the openings, the OOD frame reorder and, with
+    more ranks than the blowup, the replicated composition commitment.  The proofs must equal the single-GPU proof."""
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES=os.environ.get("CUDA_VISIBLE_DEVICES", "0").split(",")[0], NCCL_SOCKET_IFNAME="lo",
+               GLOO_SOCKET_IFNAME="lo", NCCL_IB_DISABLE="1")
+    for g, port, cases in ((2, 29613, '[["mimc", 64, 1024, 8], ["training", 128, 512, 16], ["mimc", 6, 128, 8]]'),
+                           (4, 29615, '[["training", 128, 1024, 2], ["mimc", 16, 256, 8]]')):
+        r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(g), "--master-addr", "127.0.0.1",
+                            "--master-port", str(port), "tests/mg_worker.py", cases], cwd=root, env=env, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0 and "mg ok" in r.stdout, f"{g} ranks: " + r.stdout[-2000:] + r.stderr[-2000:]
+
+
 def _training_shaped(oracle, gpu_ctx, w, n, opts, seed):
     data = T.random_felts(w * n, seed).reshape(w, n, 2)
     air = T.synthetic_training_air(n, opts, data)

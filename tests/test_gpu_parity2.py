@@ -9,7 +9,7 @@ import pytest
 
 import zk_stark_project_b200 as Z
 from zk_stark_project_b200 import lib as L
-from zk_stark_project_b200.verifier import _Reader
+from zk_stark_project_b200.verifier import _Reader, _fold_positions
 from tests import common as T
 
 pytestmark = pytest.mark.gpu
@@ -61,6 +61,19 @@ def _parse_queries(proof, w, c):
     t_rows, t_paths = r.take(r.usize()), r.take(r.usize())
     c_rows, c_paths = r.take(r.usize()), r.take(r.usize())
     return t_rows, t_paths, c_rows, c_paths
+
+
+def _parse_fri_layers(proof):
+    """FriProof layers of Proof::to_bytes(): (rows bytes, BatchMerkleProof bytes) per layer."""
+    r = _Reader(proof)
+    r.take(4 + 2 + 1 + 16 + 8 + 2)
+    r.u8()
+    r.take(r.uint(2))
+    for _ in range(4):  # trace and constraint Queries
+        r.take(r.usize())
+    for _ in range(3):  # OOD trace frame, Lagrange kernel frame, OOD constraint evaluations
+        r.take(r.uint(2))
+    return [(r.take(r.uint(4)), r.take(r.uint(4))) for _ in range(r.u8())]
 
 
 def _staged_values(ctx, oracle, air, data, ce):
@@ -130,6 +143,20 @@ def _staged_values(ctx, oracle, air, data, ce):
     rem, cnt = C.create_string_buffer(16 * 256), C.c_uint64()
     ctx.check(lib.zkb_fri_remainder(h, rem, C.byref(cnt), root))
     assert root.raw == bytes(ts.remainder_commitment)
+    # FriProver::build_proof: every layer at the positions folded as winter-fri's fold_positions does
+    layers = _parse_fri_layers(ref_proof)
+    assert len(layers) == nl.value
+    fpos, dom = list(ts.positions)[:ts.n_positions], N
+    for l, (want_rows, want_paths) in enumerate(layers):
+        fpos, dom = _fold_positions(fpos, dom, 16), dom // 16
+        arr = (C.c_uint32 * len(fpos))(*fpos)
+        rows = C.create_string_buffer(16 * 16 * len(fpos))
+        po, ln = C.c_void_p(), C.c_uint64()
+        ctx.check(lib.zkb_query(h, C.c_uint32(2 + l), arr, C.c_uint32(len(fpos)), rows, C.byref(po), C.byref(ln)))
+        paths = C.string_at(po, ln.value)
+        lib.zkb_free(po)
+        assert rows.raw == want_rows, f"queried rows of FRI layer {l} differ"
+        assert paths == want_paths, f"batch Merkle proof of FRI layer {l} differs"
 
 
 def test_staged_values_aggregation(gpu_ctx, oracle):
@@ -151,6 +178,26 @@ def test_staged_values_mimc(gpu_ctx, oracle):
     """MiMC (ce = beta = 8, six composition columns) through the staged surface, two NTT passes."""
     air, data = _mimc_case(gpu_ctx, oracle, 16, 1 << 12, T.options(blowup=8))
     _staged_values(gpu_ctx, oracle, air, data, 8)
+
+
+def test_one_rank_sharded_proof(oracle):
+    """A column-sharded proof on a one-rank communicator (row view of the LDE, Merkle cap, all-reduce of the openings) equals the
+    single-GPU proof, and zkb_query refuses to open the commitments of a sharded proof."""
+    ctx = L.Context(0)
+    try:
+        ctx.mg_init(0, 1, L.mg_unique_id())
+        mimc = _mimc_case(ctx, oracle, 16, 1 << 10, T.options(blowup=8), check_trace=False)
+        data = T.random_felts(32 * 512, 0x5EED0005).reshape(32, 512, 2)
+        for air, trace in (mimc, (T.synthetic_training_air(512, T.options(blowup=16), data), data)):
+            ptr = np.ascontiguousarray(trace).ctypes.data
+            single, _ = ctx.prove_host(air, ptr)
+            sharded, _ = ctx.mg_prove_host(air, ptr, 1)
+            assert sharded == single
+        pos = (C.c_uint32 * 1)(0)
+        rows, po, ln = C.create_string_buffer(16 * 32), C.c_void_p(), C.c_uint64()
+        assert ctx.lib.zkb_query(ctx.handle, C.c_uint32(0), pos, C.c_uint32(1), rows, C.byref(po), C.byref(ln)) == -3
+    finally:
+        ctx.close()
 
 
 def test_non_canonical_trace_is_reduced(gpu_ctx, oracle):

@@ -103,38 +103,11 @@ struct AirSpec {
     }
 };
 
-// ---- DefaultRandomCoin<Blake3_256> (src/training/prover.rs:227)  [A.5] ----------------------------------------
+// ---- DefaultRandomCoin<Blake3_256> (src/training/prover.rs:227)  [A.5]: the seed; the channel itself runs on the device
+// (csrc/coin.cuh) -----------------------------------------------------------------------------------------------------------
 struct HostCoin {
     uint8_t seed[32];
-    uint64_t counter = 0;
-    static void hash_elems(const std::vector<HF>& e, uint8_t out[32]) { b3_hash_host((const uint8_t*)e.data(), e.size() * 16, out); }
-    void init(const std::vector<HF>& e) { hash_elems(e, seed); counter = 0; }
-    void reseed(const uint8_t d[32]) { uint8_t buf[64]; memcpy(buf, seed, 32); memcpy(buf + 32, d, 32); b3_hash_host(buf, 64, seed); counter = 0; }
-    void with_int(uint64_t v, uint8_t out[32]) const { uint8_t buf[40]; memcpy(buf, seed, 32); memcpy(buf + 32, &v, 8); b3_hash_host(buf, 40, out); }
-    HF draw() {
-        for (int i = 0; i < 1000; i++) {
-            uint8_t d[32]; counter++; with_int(counter, d);
-            u128 v; memcpy(&v, d, 16);
-            if (v < HF::modulus()) return HF::raw(v);
-        }
-        throw std::runtime_error("random coin failed to draw a field element");
-    }
-    uint32_t leading_zeros(uint64_t nonce) const {
-        uint8_t d[32]; with_int(nonce, d);
-        uint64_t h; memcpy(&h, d, 8);
-        return h == 0 ? 64 : (uint32_t)__builtin_ctzll(h);
-    }
-    std::vector<uint32_t> draw_integers(uint32_t num, uint64_t domain, uint64_t nonce) {
-        uint8_t d[32]; with_int(nonce, d); memcpy(seed, d, 32); counter = 0;
-        std::vector<uint32_t> v;
-        for (int i = 0; i < 1000 && v.size() < num; i++) {
-            counter++; with_int(counter, d);
-            uint64_t x; memcpy(&x, d, 8);
-            v.push_back((uint32_t)(x & (domain - 1)));
-        }
-        if (v.size() != num) throw std::runtime_error("random coin failed to draw integers");
-        return v;
-    }
+    void init(const std::vector<HF>& e) { b3_hash_host((const uint8_t*)e.data(), e.size() * 16, seed); }
 };
 
 // ---- MerkleTree::prove_batch as an index plan  [A.6] ---------------------------------------------------------

@@ -922,20 +922,16 @@ __global__ void k_gather_lde_rows(const LdeMat m, const uint32_t* __restrict__ p
     if (k - m.k0 >= (1u << m.log_kc)) { fe_store(out + idx, fe_zero()); return; }   // coset held by another rank
     fe_store(out + idx, fe_load(m.data + lde_addr(m, k, i, j)));
 }
-// FriProver::build_proof / query_layer: rows [e[p + j*rows]]_{j<16}
-// (positions are reduced into the layer's row range: folding a position is p mod rows, rows a power of two)
-__global__ void k_gather_fri_rows(const fe* __restrict__ e, uint64_t rows, const uint32_t* __restrict__ pos, uint32_t npos, fe* __restrict__ out) {
-    const uint32_t idx = blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= npos * 16) return;
-    const uint32_t q = idx >> 4, j = idx & 15;
-    fe_store(out + idx, fe_load(e + (__ldg(pos + q) & (uint32_t)(rows - 1)) + (uint64_t)j * rows));
-}
-// All openings of a one-shot proof in ONE launch (blockIdx.y = commitment): rows at the raw query positions plus the full
-// authentication path of each — k_gather_lde_rows / k_gather_fri_rows / k_gather_paths fused, because for small proofs every
-// launch is a measurable part of the latency.  Commitments 0, 1: LDE matrices (trace, constraint composition); 2 + l: FRI layer l.
+// Openings in ONE launch (blockIdx.y + first = commitment): rows at the raw query positions plus the full authentication path
+// of each, because for small proofs every launch is a measurable part of the latency.  Commitments 0, 1: LDE matrices (trace,
+// constraint composition); 2 + l: FRI layer l, rows [e[p + j*rows]]_{j<16} (folding a position is p mod rows).
+// Sharded proofs: an entry this rank does not hold is written as zeros, every other entry is the same on all ranks, so a
+// byte-wise max over the ranks assembles the openings.  Trace rows and the path levels below lsub belong to the rank that owns
+// the queried row (r >> lsub); the levels at or above lsub are read from the replicated cap heap.  A composition row is held
+// by the rank that stores its coset.
 #define ZKB_MAX_OPEN 18
 struct OpenJobs {
-    uint32_t n_trees, q;
+    uint32_t first, q;
     const uint32_t* pos;                 // raw positions (device transcript)
     LdeMat mat[2];
     const fe* fri_evals[ZKB_MAX_OPEN - 2];
@@ -944,9 +940,11 @@ struct OpenJobs {
     uint32_t depth[ZKB_MAX_OPEN], width[ZKB_MAX_OPEN];
     fe* rows_out[ZKB_MAX_OPEN];
     uint32_t* paths_out[ZKB_MAX_OPEN];
+    const uint32_t* cap;                 // trace commitment: heap of the top depth - lsub levels (one GPU: lsub = depth)
+    uint32_t lsub, rank;                 // trace commitment: log2 rows per rank, this rank
 };
 __global__ void __launch_bounds__(128) k_open_all(const OpenJobs J) {
-    const uint32_t t = blockIdx.y;
+    const uint32_t t = blockIdx.y + J.first;
     const uint32_t idx = blockIdx.x * blockDim.x + threadIdx.x;
     const uint32_t w = J.width[t], depth = J.depth[t];
     const uint32_t nrow = J.q * w, npath = J.q * depth * 2;
@@ -956,7 +954,8 @@ __global__ void __launch_bounds__(128) k_open_all(const OpenJobs J) {
         if (t < 2) {
             const LdeMat& m = J.mat[t];
             const uint32_t k = r & ((1u << m.log_beta) - 1u), i = r >> m.log_beta;
-            fe_store(J.rows_out[t] + idx, fe_load(m.data + lde_addr(m, k, i, j)));
+            const bool held = k - m.k0 < (1u << m.log_kc) && (t != 0 || (r >> J.lsub) == J.rank);
+            fe_store(J.rows_out[t] + idx, held ? fe_load(m.data + lde_addr(m, k, i, j)) : fe_zero());
         } else {
             const uint64_t rows = J.fri_rows[t - 2];
             fe_store(J.rows_out[t] + idx, fe_load(J.fri_evals[t - 2] + (r & (uint32_t)(rows - 1)) + (uint64_t)j * rows));
@@ -964,17 +963,18 @@ __global__ void __launch_bounds__(128) k_open_all(const OpenJobs J) {
     } else if (idx - nrow < npath) {
         const uint32_t tt = idx - nrow;
         const uint32_t half = tt & 1u, ql = tt >> 1, q = ql / depth, level = ql - q * depth;
-        const uint64_t node = ((((uint64_t)1 << depth) + (__ldg(J.pos + q) & ((1u << depth) - 1u))) >> level) ^ 1ull;
-        reinterpret_cast<uint4*>(J.paths_out[t])[tt] = reinterpret_cast<const uint4*>(J.heap[t])[node * 2 + half];
+        const uint32_t r = __ldg(J.pos + q) & ((1u << depth) - 1u);
+        const uint32_t lsub = t == 0 ? J.lsub : depth;
+        uint4 v = make_uint4(0, 0, 0, 0);
+        if (level >= lsub) {   // the top levels of a heap coincide with the heap of its cap
+            const uint64_t node = ((((uint64_t)1 << depth) + r) >> level) ^ 1ull;
+            v = reinterpret_cast<const uint4*>(J.cap)[node * 2 + half];
+        } else if (t != 0 || (r >> lsub) == J.rank) {
+            const uint64_t node = ((((uint64_t)1 << lsub) + (r & ((1u << lsub) - 1u))) >> level) ^ 1ull;
+            v = reinterpret_cast<const uint4*>(J.heap[t])[node * 2 + half];
+        }
+        reinterpret_cast<uint4*>(J.paths_out[t])[tt] = v;
     }
-}
-
-// Merkle authentication nodes: out[i] = digests[idx[i]]
-__global__ void k_gather_digests(const uint32_t* __restrict__ digests, const uint64_t* __restrict__ idx, uint32_t count, uint32_t* __restrict__ out) {
-    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= count * 2) return;
-    const uint64_t src = __ldg(idx + (t >> 1));
-    reinterpret_cast<uint4*>(out)[t] = reinterpret_cast<const uint4*>(digests)[src * 2 + (t & 1)];
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -18,6 +18,7 @@ struct NcclApi {
     ncclResult_t (*Send)(const void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
     ncclResult_t (*Recv)(void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
     ncclResult_t (*AllGather)(const void*, void*, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
+    ncclResult_t (*AllReduce)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
     const char* (*GetErrorString)(ncclResult_t) = nullptr;
     void load() {
         if (h) return;
@@ -32,6 +33,7 @@ struct NcclApi {
         Send = (decltype(Send))sym("ncclSend");
         Recv = (decltype(Recv))sym("ncclRecv");
         AllGather = (decltype(AllGather))sym("ncclAllGather");
+        AllReduce = (decltype(AllReduce))sym("ncclAllReduce");
         GetErrorString = (decltype(GetErrorString))sym("ncclGetErrorString");
     }
 };

@@ -144,12 +144,6 @@ struct zkb_ctx {
     struct GraphEntry { cudaGraphExec_t exec = nullptr; uint64_t epoch = 0; uint32_t seen = 0; uint64_t launches = 0; };
     std::map<std::string, GraphEntry> graphs;
     bool capturing = false;
-    // Deferred openings (sharded proofs): every query enqueues its gathers, collectives and a copy into pinned memory and
-    // leaves a finisher behind; the stream is synchronised ONCE for all commitments, then the finishers build rows and paths.
-    bool q_defer = false;
-    size_t q_goff = 0, q_moff = 0, q_hoff = 0;
-    uint8_t* h_q = nullptr; size_t h_q_cap = 0;
-    std::vector<std::function<void()>> q_finish;
     uint8_t* h_out = nullptr;           // pinned landing area of the final download
     size_t h_out_cap = 0;
     cudaEvent_t ev_done = nullptr;      // blocking-sync event: the host thread sleeps instead of spinning while the device works
@@ -158,8 +152,7 @@ struct zkb_ctx {
     const fe* d_aval() const { return d_in.as<fe>(); }
     const fe* d_params() const { return d_in.as<fe>() + air.assertions.size(); }
     DevBuf d_lde_rows, d_mg_a, d_mg_b;  // recv view of the LDE; all-gather staging
-    DevBuf d_cap;                       // sharded trace commitment: heap of the replicated top log G levels on the device
-    std::vector<Digest32> mg_cap;       // heap of the replicated top log G levels: cap[1] = root, cap[G + q] = subtree root q
+    DevBuf d_cap;                       // sharded trace commitment: heap of the replicated top log G levels, cap[1] = root
 
     // ==========================================================================================================
     void count() { launches++; }
@@ -232,7 +225,6 @@ struct zkb_ctx {
         if (ev_ok) { for (auto& pr : tev) for (auto& x : pr) cudaEventDestroy(x); for (auto& x : ev_group) cudaEventDestroy(x); cudaStreamDestroy(copy_stream); cudaStreamDestroy(xchg_stream); }
         if (h_stage) cudaFreeHost(h_stage);
         if (h_out) cudaFreeHost(h_out);
-        if (h_q) cudaFreeHost(h_q);
         if (ev_done) cudaEventDestroy(ev_done);
         if (owns_stream && stream) { cudaStreamDestroy(stream); stream = nullptr; }
     }
@@ -268,47 +260,6 @@ struct zkb_ctx {
         CK(cudaStreamSynchronize(stream));
     }
     void check_launch() { CK(cudaGetLastError()); count(); }
-    // scratch of one query: `bytes` of d_gather, `mbytes` of d_mg_b (all-gather landing) — bump-allocated while openings are deferred
-    uint8_t* q_scratch(DevBuf& buf, size_t& off, size_t bytes) {
-        if (!q_defer) { buf.ensure(bytes); return buf.as<uint8_t>(); }
-        const size_t need = (bytes + 255) & ~(size_t)255;
-        if (off + need > buf.cap) throw StateError("internal error: deferred-query scratch exhausted");
-        uint8_t* ptr = buf.as<uint8_t>() + off;
-        off += need;
-        return ptr;
-    }
-    // device -> host read whose consumer `fin(host pointer)` runs now (after a synchronisation) or, deferred, after the batch's one
-    void q_read(const void* dsrc, size_t bytes, std::function<void(const uint8_t*)> fin) {
-        if (!q_defer) {
-            std::vector<uint8_t> host(bytes);
-            d2h(host.data(), dsrc, bytes);
-            fin(host.data());
-            return;
-        }
-        const size_t need = (bytes + 255) & ~(size_t)255;
-        if (q_hoff + need > h_q_cap) throw StateError("internal error: deferred-query landing area exhausted");
-        uint8_t* dst = h_q + q_hoff;
-        q_hoff += need;
-        CK(cudaMemcpyAsync(dst, dsrc, bytes, cudaMemcpyDeviceToHost, stream));
-        q_finish.push_back([fin, dst] { fin(dst); });
-    }
-    void q_begin_batch() {
-        const size_t G = mg_active ? (size_t)mg_world : 1, dev = (size_t)8 << 20;
-        d_gather.ensure(dev); d_mg_b.ensure(dev * G);
-        if (h_q_cap < dev * (G + 1)) {
-            if (h_q) cudaFreeHost(h_q);
-            h_q = nullptr; h_q_cap = 0;
-            CK(cudaHostAlloc((void**)&h_q, dev * (G + 1), cudaHostAllocDefault));
-            h_q_cap = dev * (G + 1);
-        }
-        q_defer = true; q_goff = q_moff = q_hoff = 0; q_finish.clear();
-    }
-    void q_end_batch() {
-        q_defer = false;
-        CK(cudaStreamSynchronize(stream));
-        for (auto& f : q_finish) f();
-        q_finish.clear();
-    }
 
     // ---- tables ---------------------------------------------------------------------------------------------
     static void build_powtab(HF base, uint32_t log_size, std::vector<HF>& lo, std::vector<HF>& hi, uint32_t& l1) {
@@ -541,11 +492,11 @@ struct zkb_ctx {
             fs.total = off;
             d_fs.ensure(fs.total);
             d_flags.ensure(256);
-            if (h_out_cap < fs.host_bytes + ZKB_CAP_BYTES) {   // + landing area of a sharded proof's commitment cap
+            if (h_out_cap < fs.host_bytes) {
                 if (h_out) { cudaFreeHost(h_out); h_out = nullptr; h_out_cap = 0; }
                 g_alloc_epoch++;
-                CK(cudaHostAlloc((void**)&h_out, fs.host_bytes + ZKB_CAP_BYTES, cudaHostAllocDefault));
-                h_out_cap = fs.host_bytes + ZKB_CAP_BYTES;
+                CK(cudaHostAlloc((void**)&h_out, fs.host_bytes, cudaHostAllocDefault));
+                h_out_cap = fs.host_bytes;
             }
             // transcript: coin seed = hash(Context ++ public inputs), computed here because the host holds the AIR; all else zero
             DevTs h0;
@@ -676,7 +627,8 @@ struct zkb_ctx {
         NK(g_nccl.CommInitRank(&comm, world, id, rank));
         mg_rank = rank; mg_world = world; log_g = log2u((uint64_t)world);
     }
-    void trace_commit_mg(const uint8_t* const* host_cols_local, const fe* d_src, uint8_t root_out[32]) {
+    // leaves the root at d_cap + 8 words
+    void trace_commit_mg(const uint8_t* const* host_cols_local, const fe* d_src) {
         if (stage != ST_BEGUN) throw StateError("zkb_mg_prove: call zkb_begin first");
         if (!comm) throw StateError("zkb_mg_init has not been called on this context");
         const uint64_t n = air.n, N = air.lde_size();
@@ -746,65 +698,6 @@ struct zkb_ctx {
         t_end(TS_MERKLE);
         // (the `interpolate` slot of zkb_stage_times carries the NVLink all-to-all time of a sharded proof)
         stage = ST_TRACE;
-        if (!root_out) {   // one-shot sharded proof: the channel reads the root on the device; the host copy of the cap (openings) rides along
-            CK(cudaMemcpyAsync(h_out + fs.host_bytes, d_cap.p, 2 * (size_t)G * 32, cudaMemcpyDeviceToHost, stream));
-            return;
-        }
-        mg_cap.assign(2 * (size_t)G, Digest32{});
-        d2h(mg_cap.data(), d_cap.p, 2 * (size_t)G * 32);
-        const Digest32 root = mg_cap[1];
-        parts.commitments.push_back(root);
-        memcpy(ts.trace_root, root.b, 32);
-        memcpy(root_out, root.b, 32);
-    }
-    // TraceLde::query for a sharded trace: every rank gathers the queried rows / authentication nodes it owns, the
-    // contributions are all-gathered and the owner's copy of each entry is kept.
-    void query_trace_mg(const std::vector<uint32_t>& pos, std::vector<uint8_t>& rows, std::vector<uint8_t>& paths) {
-        const uint32_t np = (uint32_t)pos.size(), w = air.w, G = (uint32_t)mg_world;
-        const uint64_t N = air.lde_size(), Nl = N / G;
-        for (uint32_t p : pos) if (p >= N) throw InvalidArg("query position out of range");
-        std::vector<std::vector<uint64_t>> plan = plan_batch_proof(log_N, pos);
-        std::vector<uint64_t> flat;
-        for (auto& v : plan) flat.insert(flat.end(), v.begin(), v.end());
-        // owner and local heap index of every authentication node
-        std::vector<int> owner(flat.size());
-        std::vector<uint64_t> local(flat.size(), 0);
-        for (size_t t = 0; t < flat.size(); t++) {
-            const uint64_t h = flat[t];
-            const uint32_t d = 63 - (uint32_t)__builtin_clzll(h);
-            if (d <= log_g) { owner[t] = -1; continue; }  // replicated cap
-            const uint64_t off = h - ((uint64_t)1 << d);
-            owner[t] = (int)(off >> (d - log_g));
-            if (owner[t] == mg_rank) local[t] = ((uint64_t)1 << (d - log_g)) + (off & (((uint64_t)1 << (d - log_g)) - 1));
-        }
-        const size_t row_bytes = (size_t)np * w * 16, dig_bytes = flat.size() * 32, mine = ((row_bytes + dig_bytes + 15) / 16) * 16;
-        size_t o_pos = 0, o_idx = 1024, o_out = o_idx + ((flat.size() * 8 + 15) / 16) * 16 + 16, total = o_out + mine;
-        uint8_t* base = q_scratch(d_gather, q_goff, total);
-        uint8_t* gathered = q_scratch(d_mg_b, q_moff, mine * G);
-        h2d_small(base + o_pos, pos.data(), np * 4);
-        if (!flat.empty()) h2d_small(base + o_idx, local.data(), flat.size() * 8);
-        k_gather_lde_rows<<<(np * w + 127) / 128, 128, 0, stream>>>(lde_rows_mat(), (const uint32_t*)(base + o_pos), np, (fe*)(base + o_out));
-        check_launch();
-        if (!flat.empty()) {
-            k_gather_digests<<<(unsigned)((flat.size() * 2 + 127) / 128), 128, 0, stream>>>(d_tree.as<uint32_t>(), (const uint64_t*)(base + o_idx),
-                                                                                        (uint32_t)flat.size(), (uint32_t*)(base + o_out + row_bytes));
-            check_launch();
-        }
-        NK(g_nccl.AllGather(base + o_out, gathered, mine, ncclUint8, comm, stream));
-        const uint32_t depth = log_N;
-        q_read(gathered, mine * G, [this, pos, plan, flat, owner, np, w, Nl, row_bytes, dig_bytes, mine, depth, &rows, &paths](const uint8_t* all) {
-            rows.resize(row_bytes);
-            for (uint32_t q = 0; q < np; q++) {
-                const size_t own = pos[q] / Nl;
-                memcpy(&rows[(size_t)q * w * 16], all + own * mine + (size_t)q * w * 16, (size_t)w * 16);
-            }
-            std::vector<uint8_t> dig(dig_bytes);
-            for (size_t t = 0; t < flat.size(); t++) {
-                if (owner[t] < 0) memcpy(&dig[t * 32], mg_cap[flat[t]].b, 32);
-                else memcpy(&dig[t * 32], all + (size_t)owner[t] * mine + row_bytes + t * 32, 32);
-            }
-            paths = batch_proof_bytes(depth, plan, dig.data());
-        });
     }
 
     // ---- Fiat-Shamir steps.  `digest` = device address of the commitment the coin is reseeded with (one-shot proofs: the whole
@@ -1117,18 +1010,16 @@ struct zkb_ctx {
             if (nt > 1) col_sum(sm + o_hp, nt, c, frame + 2 * (size_t)w);
         }
         if (mg_active) {
-            // per-rank [cur wl][next wl] blocks -> the global frame, put back on the device for k_fs_ood
+            // per-rank [cur wl][next wl] blocks -> the global frame [cur w][next w]: two strided copies on the device
             NK(g_nccl.AllGather(sm + o_loc, sm + o_ga, 2 * (size_t)wl * 16, ncclUint8, comm, stream));
-            std::vector<HF> all(2 * (size_t)w), glob(2 * (size_t)w);
-            d2h(all.data(), sm + o_ga, all.size() * 16);
-            for (int r = 0; r < mg_world; r++)
-                for (uint32_t jl = 0; jl < wl; jl++) { glob[r * wl + jl] = all[(size_t)r * 2 * wl + jl]; glob[w + r * wl + jl] = all[(size_t)r * 2 * wl + wl + jl]; }
-            h2d_small(frame, glob.data(), glob.size() * 16);
+            for (uint32_t h = 0; h < 2; h++)
+                CK(cudaMemcpy2DAsync(frame + (size_t)h * w, (size_t)wl * 16, sm + o_ga + (size_t)h * wl, 2 * (size_t)wl * 16, (size_t)wl * 16, (size_t)mg_world,
+                                     cudaMemcpyDeviceToDevice, stream));
         }
         t_end(TS_OOD);
         stage = ST_OOD;
     }
-    void ood_fetch() {   // host copy of the frame (staged API, sharded proofs)
+    void ood_fetch() {   // host copy of the frame (staged API)
         const uint32_t w = air.w;
         std::vector<HF> host(2 * (size_t)w + c);
         d2h(host.data(), fs_fe(fs.o_ood), host.size() * 16);
@@ -1299,64 +1190,50 @@ struct zkb_ctx {
         }
     }
 
-    // K11
+    // K11 (TraceLde::query, ConstraintCommitment::query, FriProver::build_proof): rows and full authentication paths of
+    // commitments [first, first + n) at the J.q positions J.pos, into J.rows_out / J.paths_out, in one launch
+    void open_commitments(OpenJobs& J, uint32_t first, uint32_t n) {
+        J.first = first;
+        J.mat[0] = mg_active ? lde_rows_mat() : lde_mat(); J.mat[1] = comp_mat();
+        J.cap = d_cap.as<uint32_t>(); J.lsub = log_N - (mg_active ? log_g : 0); J.rank = mg_active ? (uint32_t)mg_rank : 0;
+        uint32_t items = 0;
+        for (uint32_t t = first; t < first + n; t++) {
+            const FsTree& tr = fs.trees[t];
+            J.depth[t] = tr.depth; J.width[t] = tr.width;
+            if (t == 0) J.heap[t] = d_tree.as<uint32_t>();
+            else if (t == 1) J.heap[t] = d_comp_tree.as<uint32_t>();
+            else {
+                const uint32_t l = t - 2;
+                J.fri_evals[l] = l == 0 ? d_deep.as<fe>() : d_fri_evals[l].as<fe>();
+                J.fri_rows[l] = fri_domain(l) / 16;
+                J.heap[t] = d_fri_tree[l].as<uint32_t>();
+            }
+            items = std::max(items, J.q * tr.width + J.q * tr.depth * 2);
+        }
+        k_open_all<<<dim3((items + 127) / 128, n), 128, 0, stream>>>(J);
+        check_launch();
+    }
+    // staged zkb_query: one commitment at the caller's positions
     void query(uint32_t which, const std::vector<uint32_t>& pos, std::vector<uint8_t>& rows, std::vector<uint8_t>& paths) {
+        if (mg_active) throw StateError("zkb_query: not available for a column-sharded proof");
         const uint32_t np = (uint32_t)pos.size();
         if (np == 0 || np > 255) throw InvalidArg("bad number of query positions");
-        if (which == 0 && mg_active) { query_trace_mg(pos, rows, paths); return; }
-        uint32_t width, depth; const uint32_t* heap;
-        uint64_t domain;
-        if (which == 0) { width = air.w; domain = air.lde_size(); heap = d_tree.as<uint32_t>(); }
-        else if (which == 1) { width = c; domain = air.lde_size(); heap = d_comp_tree.as<uint32_t>(); }
-        else {
-            uint32_t l = which - 2;
-            if (l >= fri_layers) throw InvalidArg("no such FRI layer");
-            width = 16; domain = fri_domain(l) / 16; heap = d_fri_tree[l].as<uint32_t>();
-        }
+        if (which >= fs.trees.size()) throw InvalidArg("no such FRI layer");
+        const FsTree& tr = fs.trees[which];
+        const uint64_t domain = which < 2 ? air.lde_size() : fri_domain(which - 2) / 16;
         for (uint32_t p : pos) if (p >= domain) throw InvalidArg("query position out of range");
-        depth = log2u(domain);
-        std::vector<std::vector<uint64_t>> plan = plan_batch_proof(depth, pos);
-        std::vector<uint64_t> flat;
-        for (auto& v : plan) flat.insert(flat.end(), v.begin(), v.end());
-        // device scratch: [positions np u32][idx flat u64][rows np*width fe][digests flat*32]
-        size_t o_pos = 0, o_idx = 1024, o_rows = o_idx + ((flat.size() * 8 + 15) / 16) * 16 + 16, o_dig = o_rows + (size_t)np * width * 16,
-               total = o_dig + flat.size() * 32 + 32;
-        uint8_t* base = q_scratch(d_gather, q_goff, total);
-        h2d_small(base + o_pos, pos.data(), np * 4);
-        if (!flat.empty()) h2d_small(base + o_idx, flat.data(), flat.size() * 8);
-        const uint32_t th = np * width;
-        if (which == 0) k_gather_lde_rows<<<(th + 127) / 128, 128, 0, stream>>>(lde_mat(), (const uint32_t*)(base + o_pos), np, (fe*)(base + o_rows));
-        else if (which == 1) k_gather_lde_rows<<<(th + 127) / 128, 128, 0, stream>>>(comp_mat(), (const uint32_t*)(base + o_pos), np, (fe*)(base + o_rows));
-        else {
-            uint32_t l = which - 2;
-            const fe* e = l == 0 ? d_deep.as<fe>() : d_fri_evals[l].as<fe>();
-            k_gather_fri_rows<<<(th + 127) / 128, 128, 0, stream>>>(e, domain, (const uint32_t*)(base + o_pos), np, (fe*)(base + o_rows));
-        }
-        check_launch();
-        if (!flat.empty()) {
-            k_gather_digests<<<(unsigned)((flat.size() * 2 + 127) / 128), 128, 0, stream>>>(heap, (const uint64_t*)(base + o_idx), (uint32_t)flat.size(),
-                                                                                        (uint32_t*)(base + o_dig));
-            check_launch();
-        }
-        const size_t rows_bytes = (size_t)np * width * 16;
-        // rows and digests are adjacent
-        q_read(base + o_rows, rows_bytes + flat.size() * 32, [this, plan, depth, rows_bytes, &rows, &paths](const uint8_t* host) {
-            rows.assign(host, host + rows_bytes);
-            paths = batch_proof_bytes(depth, plan, host + rows_bytes);
-        });
-        if (which == 1 && mg_coset()) {
-            // coset-sharded composition LDE: a queried row lives on the rank that owns its coset (the tree is replicated)
-            const size_t rb = ((rows_bytes + 15) / 16) * 16;
-            uint8_t* gathered = q_scratch(d_mg_b, q_moff, rb * mg_world);
-            NK(g_nccl.AllGather(base + o_rows, gathered, rb, ncclUint8, comm, stream));
-            const uint32_t blow = (uint32_t)air.blowup, lkc = mg_log_kc();
-            q_read(gathered, rb * mg_world, [pos, np, width, rb, blow, lkc, &rows](const uint8_t* all) {   // runs after the reader above
-                for (uint32_t q = 0; q < np; q++) {
-                    const size_t own = (pos[q] & (blow - 1)) >> lkc;
-                    memcpy(&rows[(size_t)q * width * 16], all + own * rb + (size_t)q * width * 16, (size_t)width * 16);
-                }
-            });
-        }
+        // device scratch: [positions np u32][rows np*width fe][full paths np*depth digests]
+        const size_t o_rows = 1024, rb = (size_t)np * tr.width * 16, pb = (size_t)np * tr.depth * 32;
+        d_gather.ensure(o_rows + rb + pb);
+        uint8_t* base = d_gather.as<uint8_t>();
+        h2d_small(base, pos.data(), np * 4);
+        OpenJobs J{};
+        J.q = np; J.pos = (const uint32_t*)base;
+        J.rows_out[which] = (fe*)(base + o_rows); J.paths_out[which] = (uint32_t*)(base + o_rows + rb);
+        open_commitments(J, which, 1);
+        std::vector<uint8_t> host(rb + pb);
+        d2h(host.data(), base + o_rows, host.size());
+        pick_openings(host.data(), host.data() + rb, tr.width, tr.depth, pos, pos, (uint32_t)(domain - 1), rows, paths);
     }
 
     // ==========================================================================================================
@@ -1365,7 +1242,8 @@ struct zkb_ctx {
     // (transcript, OOD frame, remainder, and for every commitment the rows and full authentication paths at the raw query
     // positions, from which the host picks what BatchMerkleProof needs after sorting / deduplicating the positions).
     // sharded = true: `cols` / `d_trace_in` hold only this rank's w/G columns and the proof is produced cooperatively by all
-    // ranks of the NCCL communicator, the channel replicated on every rank's device (every rank returns the same bytes).
+    // ranks of the NCCL communicator, the channel replicated on every rank's device (every rank returns the same bytes); the
+    // openings are completed by one all-reduce before the download, so a sharded proof also waits on the device once.
     std::vector<uint8_t> prove(const zkb_air_desc* desc, const uint8_t* const* cols, const fe* d_trace_in, uint64_t force_nonce,
                                bool sharded = false) {
         static const bool host_prof = getenv("ZKB_HOST_PROFILE") != nullptr;   // diagnostics: host phases of a proof on stderr
@@ -1374,13 +1252,12 @@ struct zkb_ctx {
         begin(desc);
         const auto hp1 = std::chrono::steady_clock::now();
         t_begin(TS_TOTAL);
-        if (sharded) return prove_sharded(cols, d_trace_in, force_nonce);
         if (!d_trace_in && !cols) throw InvalidArg("null trace columns");
         // Small proofs are launch-bound (tens of 3-8 us kernels): from the second proof of a shape on, the whole enqueue sequence
         // is captured into a CUDA graph and replayed with one launch.  What varies between proofs of a shape — coin seed,
         // assertion values, AIR parameters (uploaded by begin()) and the trace — sits at fixed device addresses.
-        const bool small = graphs_on && !force_nonce && ((air.lde_size() * air.w) >> 22) == 0;
-        if (!small) enqueue_proof(cols, d_trace_in, force_nonce);
+        const bool small = graphs_on && !sharded && !force_nonce && ((air.lde_size() * air.w) >> 22) == 0;
+        if (!small) enqueue_proof(cols, d_trace_in, force_nonce, sharded);
         else {
             const fe* src = d_trace_in ? d_trace_in : upload_cols(cols, air.w, air.n, d_trace);
             std::string key((const char*)desc, offsetof(zkb_air_desc, pub_elems));
@@ -1446,10 +1323,11 @@ struct zkb_ctx {
 
     // Everything between "the trace is available" and "the last byte of the proof is on its way to the host": no host
     // synchronisation and no per-proof upload — the sequence depends on the shape only, which is what makes it capturable.
-    void enqueue_proof(const uint8_t* const* cols, const fe* d_trace_in, uint64_t force_nonce) {
-        if (d_trace_in) trace_commit_dev(nullptr, d_trace_in);
+    void enqueue_proof(const uint8_t* const* cols, const fe* d_trace_in, uint64_t force_nonce, bool sharded = false) {
+        if (sharded) trace_commit_mg(cols, d_trace_in);
+        else if (d_trace_in) trace_commit_dev(nullptr, d_trace_in);
         else trace_commit_dev(cols, nullptr);
-        fs_after_trace_root(d_tree.as<uint32_t>() + 8, nullptr);       // channel.commit_trace; get_constraint_composition_coeffs
+        fs_after_trace_root((sharded ? d_cap : d_tree).as<uint32_t>() + 8, nullptr);   // channel.commit_trace; get_constraint_composition_coeffs
         constraints_eval_dev();
         constraints_commit_dev();
         fs_after_constraint_root(d_comp_tree.as<uint32_t>() + 8, nullptr);   // channel.commit_constraints; get_ood_point
@@ -1457,29 +1335,17 @@ struct zkb_ctx {
         fs_after_ood(true, nullptr);                                   // send_ood_*; get_deep_composition_coeffs
         deep_compose_dev();
         enqueue_fri_to_positions(force_nonce);
-        const uint32_t q = air.num_queries;
-        {   // TraceLde::query, ConstraintCommitment::query, FriProver::build_proof at the raw positions: one launch
+        {   // every commitment at the raw positions
             OpenJobs J{};
             uint8_t* base = d_fs.as<uint8_t>();
-            J.n_trees = (uint32_t)fs.trees.size(); J.q = q; J.pos = dts()->positions;
-            J.mat[0] = lde_mat(); J.mat[1] = comp_mat();
-            uint32_t items = 0;
-            for (size_t t = 0; t < fs.trees.size(); t++) {
-                const FsTree& tr = fs.trees[t];
-                J.depth[t] = tr.depth; J.width[t] = tr.width;
-                J.rows_out[t] = (fe*)(base + tr.o_rows); J.paths_out[t] = (uint32_t*)(base + tr.o_paths);
-                if (t == 0) J.heap[t] = d_tree.as<uint32_t>();
-                else if (t == 1) J.heap[t] = d_comp_tree.as<uint32_t>();
-                else {
-                    const uint32_t l = (uint32_t)t - 2;
-                    J.fri_evals[l] = l == 0 ? d_deep.as<fe>() : d_fri_evals[l].as<fe>();
-                    J.fri_rows[l] = fri_domain(l) / 16;
-                    J.heap[t] = d_fri_tree[l].as<uint32_t>();
-                }
-                items = std::max(items, q * tr.width + q * tr.depth * 2);
+            J.q = air.num_queries; J.pos = dts()->positions;
+            for (size_t t = 0; t < fs.trees.size(); t++) { J.rows_out[t] = (fe*)(base + fs.trees[t].o_rows); J.paths_out[t] = (uint32_t*)(base + fs.trees[t].o_paths); }
+            open_commitments(J, 0, (uint32_t)fs.trees.size());
+            // sharded: trace rows and paths, and coset-sharded composition rows, are the owner's value or zero on each rank
+            if (mg_active) {
+                const size_t o = fs.trees[0].o_rows;
+                NK(g_nccl.AllReduce(base + o, base + o, fs.trees[1].o_paths - o, ncclUint8, ncclMax, comm, stream));
             }
-            k_open_all<<<dim3((items + 127) / 128, J.n_trees), 128, 0, stream>>>(J);
-            check_launch();
         }
         t_end(TS_QUERY);
         CK(cudaMemcpyAsync(h_out, d_fs.p, fs.host_bytes, cudaMemcpyDeviceToHost, stream));
@@ -1548,36 +1414,38 @@ struct zkb_ctx {
         for (size_t i = 0; i < positions.size() && i < 256; i++) ts.positions[i] = positions[i];
         return raw;
     }
+    // One commitment from the rows `hrows` and full paths `hpaths` gathered at the positions `raw`: the rows of `pos` (each found
+    // among the raw positions reduced by `mask`) and the batch proof of `pos`
+    static void pick_openings(const uint8_t* hrows, const uint8_t* hpaths, uint32_t width, uint32_t depth, const std::vector<uint32_t>& raw,
+                              const std::vector<uint32_t>& pos, uint32_t mask, std::vector<uint8_t>& rows, std::vector<uint8_t>& paths) {
+        const size_t rb = (size_t)width * 16;
+        std::vector<std::pair<uint32_t, uint32_t>> first(raw.size());   // (reduced position, a raw index that carries it), sorted
+        for (uint32_t i = 0; i < raw.size(); i++) first[i] = {raw[i] & mask, i};
+        std::sort(first.begin(), first.end());
+        auto raw_index_in = [&](uint64_t lo, uint64_t hi_excl) -> uint32_t {   // a raw index whose reduced position is in [lo, hi)
+            auto it = std::lower_bound(first.begin(), first.end(), std::make_pair((uint32_t)lo, 0u));
+            if (it == first.end() || it->first >= hi_excl) throw std::runtime_error("internal error: opening not gathered");
+            return it->second;
+        };
+        rows.resize(pos.size() * rb);
+        for (size_t i = 0; i < pos.size(); i++) memcpy(&rows[i * rb], hrows + (size_t)raw_index_in(pos[i], (uint64_t)pos[i] + 1) * rb, rb);
+        // node `hi` of the heap sits `lv` levels above the leaves and is the sibling of an ancestor of some queried leaf: that
+        // leaf lies under hi ^ 1, and its gathered path holds `hi` at position lv
+        std::vector<std::vector<uint64_t>> plan = plan_batch_proof(depth, pos);
+        std::vector<uint8_t> gathered;
+        for (auto& v : plan)
+            for (uint64_t hi : v) {
+                const uint32_t lv = depth - (63u - (uint32_t)__builtin_clzll(hi));
+                const uint64_t anc = hi ^ 1ull, lo = (anc << lv) - ((uint64_t)1 << depth);
+                const uint8_t* d = hpaths + ((size_t)raw_index_in(lo, lo + ((uint64_t)1 << lv)) * depth + lv) * 32;
+                gathered.insert(gathered.end(), d, d + 32);
+            }
+        paths = batch_proof_bytes(depth, plan, gathered.data());
+    }
     std::vector<uint8_t> assemble_proof() {
         const std::vector<uint32_t> raw = assemble_transcript();
-        const uint32_t q = air.num_queries;
-        // one commitment: rows of `pos` (each found among the raw positions reduced by `mask`) + batch proof
         auto open = [&](const FsTree& tr, const std::vector<uint32_t>& pos, uint32_t mask, std::vector<uint8_t>& rows, std::vector<uint8_t>& paths) {
-            const uint8_t* hrows = h_out + tr.o_rows;
-            const uint8_t* hpaths = h_out + tr.o_paths;
-            const size_t rb = (size_t)tr.width * 16;
-            std::vector<std::pair<uint32_t, uint32_t>> first(q);   // (reduced position, a raw index that carries it), sorted
-            for (uint32_t i = 0; i < q; i++) first[i] = {raw[i] & mask, i};
-            std::sort(first.begin(), first.end());
-            auto raw_index_in = [&](uint64_t lo, uint64_t hi_excl) -> uint32_t {   // a raw index whose reduced position is in [lo, hi)
-                auto it = std::lower_bound(first.begin(), first.end(), std::make_pair((uint32_t)lo, 0u));
-                if (it == first.end() || it->first >= hi_excl) throw std::runtime_error("internal error: opening not gathered");
-                return it->second;
-            };
-            rows.resize(pos.size() * rb);
-            for (size_t i = 0; i < pos.size(); i++) memcpy(&rows[i * rb], hrows + (size_t)raw_index_in(pos[i], (uint64_t)pos[i] + 1) * rb, rb);
-            // node `hi` of the heap sits `lv` levels above the leaves and is the sibling of an ancestor of some queried leaf: that
-            // leaf lies under hi ^ 1, and its gathered path holds `hi` at position lv
-            std::vector<std::vector<uint64_t>> plan = plan_batch_proof(tr.depth, pos);
-            std::vector<uint8_t> gathered;
-            for (auto& v : plan)
-                for (uint64_t hi : v) {
-                    const uint32_t lv = tr.depth - (63u - (uint32_t)__builtin_clzll(hi));
-                    const uint64_t anc = hi ^ 1ull, lo = (anc << lv) - ((uint64_t)1 << tr.depth);
-                    const uint8_t* d = hpaths + ((size_t)raw_index_in(lo, lo + ((uint64_t)1 << lv)) * tr.depth + lv) * 32;
-                    gathered.insert(gathered.end(), d, d + 32);
-                }
-            paths = batch_proof_bytes(tr.depth, plan, gathered.data());
+            pick_openings(h_out + tr.o_rows, h_out + tr.o_paths, tr.width, tr.depth, raw, pos, mask, rows, paths);
         };
         open(fs.trees[0], positions, (uint32_t)(air.lde_size() - 1), parts.trace_rows, parts.trace_paths);
         open(fs.trees[1], positions, (uint32_t)(air.lde_size() - 1), parts.comp_rows, parts.comp_paths);
@@ -1589,99 +1457,6 @@ struct zkb_ctx {
             dom /= 16;
             open(fs.trees[2 + l], fpos, (uint32_t)(dom - 1), parts.fri_rows[l], parts.fri_paths[l]);
         }
-        return serialize_proof(air, parts);
-    }
-
-    // column-sharded proof with the channel on the host (every rank replays it identically between the collectives): the round-1
-    // flow, kept behind ZKB_MG_HOST_COIN=1 for A/B measurements
-    void prove_sharded_host_coin(const uint8_t* const* cols, const fe* d_trace_in, uint64_t force_nonce) {
-        uint8_t root[32];
-        trace_commit_mg(cols, d_trace_in, root);
-        coin.reseed(root);                                   // channel.commit_trace
-        HF alpha = coin.draw();                              // get_constraint_composition_coeffs
-        alpha.to_bytes(ts.constraint_alpha);
-        constraints_eval(alpha, nullptr);
-        constraints_commit(root);
-        coin.reseed(root);                                   // channel.commit_constraints
-        HF zz = coin.draw();                                 // get_ood_point
-        zz.to_bytes(ts.z);
-        ood_eval(zz);
-        parts.ood_trace_interleaved.resize(2 * (size_t)air.w);  // [T_0(z), T_0(zg), T_1(z), ...]  [A.5]
-        for (uint32_t j = 0; j < air.w; j++) { parts.ood_trace_interleaved[2 * j] = ood_cur[j]; parts.ood_trace_interleaved[2 * j + 1] = ood_next[j]; }
-        parts.ood_h = ood_h;
-        uint8_t h[32];
-        HostCoin::hash_elems(parts.ood_trace_interleaved, h); coin.reseed(h);  // send_ood_trace_states
-        HostCoin::hash_elems(parts.ood_h, h); coin.reseed(h);                  // send_ood_constraint_evaluations
-        HF da = coin.draw();                                 // get_deep_composition_coeffs
-        da.to_bytes(ts.deep_alpha);
-        deep_compose(da);
-        t_begin(TS_FRI);
-        for (uint32_t l = 0; l < fri_layers; l++) {          // FriProver::build_layers
-            fri_commit_layer(root);
-            coin.reseed(root);
-            fri_fold(coin.draw());
-        }
-        Digest32 rc;
-        fri_remainder(&rc);
-        coin.reseed(rc.b);
-        t_end(TS_FRI);
-        t_begin(TS_GRIND);
-        uint64_t nonce = force_nonce ? force_nonce : grind(coin.seed, air.grinding);  // grind_query_seed
-        t_end(TS_GRIND);
-        parts.nonce = nonce; ts.pow_nonce = nonce;
-        t_begin(TS_QUERY);
-        positions = coin.draw_integers(air.num_queries, air.lde_size(), nonce);        // get_query_positions
-        std::sort(positions.begin(), positions.end());
-        positions.erase(std::unique(positions.begin(), positions.end()), positions.end());
-        parts.n_unique = (uint32_t)positions.size();
-        ts.n_positions = parts.n_unique;
-        for (size_t i = 0; i < positions.size() && i < 256; i++) ts.positions[i] = positions[i];
-    }
-    // Column-sharded proof.  The channel is replicated on the device of every rank (csrc/coin.cuh: all ranks see the same
-    // commitments, OOD frame and remainder, so they draw the same challenges), as in the single-GPU proof: no host round trip
-    // until the query positions are known; then the openings of all commitments are gathered from their owners in one batch.
-    // ZKB_MG_HOST_COIN=1 keeps the channel on the host, one synchronisation per commitment (the round-1 path; A/B and the staged API).
-    std::vector<uint8_t> prove_sharded(const uint8_t* const* cols, const fe* d_trace_in, uint64_t force_nonce) {
-        static const bool host_coin = getenv("ZKB_MG_HOST_COIN") != nullptr;
-        if (host_coin) prove_sharded_host_coin(cols, d_trace_in, force_nonce);
-        else {
-            trace_commit_mg(cols, d_trace_in, nullptr);
-            fs_after_trace_root(d_cap.as<uint32_t>() + 8, nullptr);        // channel.commit_trace; get_constraint_composition_coeffs
-            constraints_eval_dev();
-            constraints_commit_dev();
-            fs_after_constraint_root(d_comp_tree.as<uint32_t>() + 8, nullptr);   // channel.commit_constraints; get_ood_point
-            ood_eval_dev();
-            fs_after_ood(true, nullptr);                                   // send_ood_*; get_deep_composition_coeffs
-            deep_compose_dev();
-            enqueue_fri_to_positions(force_nonce);
-            // transcript, OOD frame, remainder (not the opening areas behind them, which a sharded proof does not fill)
-            const size_t head = fs.trees.empty() ? fs.host_bytes : std::min(fs.host_bytes, fs.trees[0].o_rows);
-            CK(cudaMemcpyAsync(h_out, d_fs.p, head, cudaMemcpyDeviceToHost, stream));
-            CK(cudaStreamSynchronize(stream));   // spin: the openings are enqueued the moment the positions are known
-            const size_t G = (size_t)mg_world;
-            mg_cap.assign(2 * G, Digest32{});
-            memcpy(mg_cap.data(), h_out + fs.host_bytes, 2 * G * 32);
-            assemble_transcript();
-        }
-        {   // FriProver::build_proof, TraceLde::query, ConstraintCommitment::query
-            std::vector<std::vector<uint32_t>> fpos(fri_layers);
-            uint64_t dom = air.lde_size();
-            parts.fri_rows.resize(fri_layers); parts.fri_paths.resize(fri_layers);
-            for (uint32_t l = 0; l < fri_layers; l++) {
-                fpos[l] = fold_positions(l ? fpos[l - 1] : positions, dom, 16);
-                dom /= 16;
-            }
-            q_begin_batch();   // seven commitments, two all-gathers, one synchronisation
-            try {
-                for (uint32_t l = 0; l < fri_layers; l++) query(2 + l, fpos[l], parts.fri_rows[l], parts.fri_paths[l]);
-                query(0, positions, parts.trace_rows, parts.trace_paths);
-                query(1, positions, parts.comp_rows, parts.comp_paths);
-            } catch (...) { q_defer = false; q_finish.clear(); throw; }
-            q_end_batch();
-        }
-        t_end(TS_QUERY);
-        t_end(TS_TOTAL);
-        stage = ST_QUERY;
         return serialize_proof(air, parts);
     }
 };
