@@ -4,7 +4,13 @@
     python tools/sass_hist.py zk_stark_project_b200/libzkb200.so k_ntt_pass k_hash_lde_rows ... > profiles/rN_sass_hist.txt
 
 For every kernel whose mangled name contains one of the patterns it prints the opcode histogram, the split into FMA-pipe
-(IMAD*) / ALU-pipe / memory classes and — when the kernel has one dominant backward branch — the same for its hottest loop."""
+(IMAD*) / ALU-pipe / memory classes and — when the kernel has one dominant backward branch — the same for its hottest loop.
+
+    python tools/sass_hist.py --regions BINARY KERNEL label=LO-HI[*N][+LO-HI[*N]..] ...
+
+counts the instructions a thread executes per kernel invocation, region by region: each region is a list of SASS address ranges
+[LO, HI) (hex, as printed by cuobjdump -sass) on the path the thread takes, each weighted by how often it runs (loop trips).
+The ranges are read off the disassembly of one build for one launch shape and have to be re-read after any change of the kernel."""
 import collections
 import re
 import subprocess
@@ -72,7 +78,28 @@ def report(name, body):
         print(f"   largest loop: {len(lops)} instructions: " + "; ".join(f"{v} {k}" for k, v in classes(lops).most_common()))
 
 
+def regions(binary, kernel, specs):
+    body = next((b for n, b in kernels(binary) if n == kernel), None)
+    if body is None:
+        sys.exit(f"no kernel {kernel} in {binary}")
+    total = 0
+    print(f"== {kernel}: instructions per thread and invocation, by region")
+    for spec in specs:
+        label, ranges = spec.split("=", 1)
+        n = 0
+        for r in ranges.split("+"):
+            span, _, mult = r.partition("*")
+            lo, hi = (int(x, 16) for x in span.split("-"))
+            n += sum(1 for a, i in body if lo <= a < hi and not i.startswith("NOP")) * (int(mult) if mult else 1)
+        total += n
+        print(f"   {n:6d}  {label}  ({ranges})")
+    print(f"   {total:6d}  total")
+
+
 if __name__ == "__main__":
+    if sys.argv[1] == "--regions":
+        regions(sys.argv[2], sys.argv[3], sys.argv[4:])
+        sys.exit(0)
     binary, pats = sys.argv[1], sys.argv[2:]
     for name, body in kernels(binary):
         if any(p in name for p in pats):

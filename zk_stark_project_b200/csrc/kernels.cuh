@@ -113,6 +113,8 @@ struct NttPass {
     PowTab roots;                  // w_{2^log_tab}^e
     const fe* pow3;                // pow3[l] = 3^(n >> l), l = 0..log_n
     const fe* tw_tab;              // optional: precomputed tile twiddles [(k << a) + t_low][S - 1] (k_build_twiddles); null = generate
+    uint32_t tw_four;              // tw_tab holds every twiddle as its four pre-shifted copies (fe4, four fe per entry)
+    uint32_t tile0;                // (t_low, u0) index of blockIdx.z == 0: launches of more than 65535 of them are split
 };
 
 __device__ __forceinline__ uint32_t bitrev(uint32_t v, uint32_t bits) { return bits == 0 ? 0u : (__brev(v) >> (32 - bits)); }
@@ -175,7 +177,8 @@ __device__ __forceinline__ fe ntt_twiddle(const NttPass& p, uint32_t k, uint32_t
     if (p.coset) t = fe_mul(t, fe_ldg(p.pow3 + l));
     return t;
 }
-// all tile twiddles of a pass, for cosets [0, n_cosets): table[((k << a) + t_low) * (S - 1) + q]
+// all tile twiddles of a pass, for cosets [0, n_cosets): table[((k << a) + t_low) * (S - 1) + q], as four pre-shifted copies
+// (fe4) when p.tw_four, so that the tiles of k_ntt_pass<true> only copy them
 __global__ void k_build_twiddles(const NttPass p, fe* __restrict__ table) {
     const uint32_t S = 1u << (p.b - p.a);
     const uint64_t total = ((uint64_t)p.n_cosets << p.a) * (S - 1u);
@@ -183,7 +186,15 @@ __global__ void k_build_twiddles(const NttPass p, fe* __restrict__ table) {
     if (id >= total) return;
     const uint32_t q = (uint32_t)(id % (S - 1u));
     const uint32_t tile = (uint32_t)(id / (S - 1u));
-    fe_store(table + id, ntt_twiddle(p, tile >> p.a, tile & ((1u << p.a) - 1u), q));
+    const fe w = ntt_twiddle(p, tile >> p.a, tile & ((1u << p.a) - 1u), q);
+    if (p.tw_four) {
+        const fe4 t = fe4_from(w);
+#pragma unroll
+        for (int i = 0; i < 4; i++) fe_store(table + 4 * id + i, t.w[i]);
+    } else fe_store(table + id, w);
+}
+__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src) : "memory");
 }
 
 // the same for ONE column with plain (single-copy) twiddles: narrow tiles (1-2 columns) reuse a twiddle too rarely for the
@@ -251,6 +262,16 @@ __device__ __forceinline__ void ntt_round(fe* sm, const fe4* tw, uint32_t rs, ui
 template <int NC>
 __device__ __forceinline__ void ntt_rounds(fe* sm, const fe4* tw, uint32_t rs, uint32_t log_cj, uint32_t logS) {
     // rounds of up to three layers held in registers
+    if (NC == 2 && log_cj == 4 && logS == 8) {
+        // 256 x 16 tiles (every pass of the 2^16-row transforms of >= 9 columns): with the strides and layer offsets known at
+        // compile time the 16 element addresses of a unit are immediate offsets from one register
+        uint32_t lam0 = 0;
+        asm("" : "+r"(lam0));   // kept opaque: constant twiddle addresses would be hoisted (112 registers) and spilled
+        ntt_round<3, NC>(sm, tw, 17, 4, 8, lam0); __syncthreads();
+        ntt_round<3, NC>(sm, tw, 17, 4, 8, 3); __syncthreads();
+        ntt_round<2, NC>(sm, tw, 17, 4, 8, 6); __syncthreads();
+        return;
+    }
     for (uint32_t lam0 = 0; lam0 < logS;) {
         const uint32_t left = logS - lam0;
         if (left >= 3 && left != 4) { ntt_round<3, NC>(sm, tw, rs, log_cj, logS, lam0); lam0 += 3; }
@@ -273,44 +294,53 @@ __global__ void __launch_bounds__(256, PRE ? 2 : 3) k_ntt_pass(const NttPass p) 
     fe4* tw = reinterpret_cast<fe4*>(sm + (size_t)S * rs);
     fe* tw1 = sm + (size_t)S * rs;
 
-    // tile coordinates: column tile fastest, then coset (so one input tile is reused out of L2), then (t_low, u0)
-    const uint32_t n_ct = (p.ncols + cj - 1) >> log_cj;
-    uint32_t id = blockIdx.x;
-    const uint32_t ct = id % n_ct; id /= n_ct;
-    const uint32_t kk = id % p.n_cosets; id /= p.n_cosets;
+    // tile coordinates (x = column tile, y = coset, z = (t_low, u0)): blocks are dispatched x fastest, so the cosets of one input
+    // tile run back to back and reuse it out of L2
+    const uint32_t ct = blockIdx.x, kk = blockIdx.y, id = p.tile0 + blockIdx.z;
     const uint32_t t_low = id & ((1u << p.a) - 1u);
     const uint32_t u0 = id >> p.a;
     const uint32_t k = p.coset0 + kk;
-    const fe* in = p.in + (size_t)kk * p.in_coset_stride;
-    fe* out = p.out + (size_t)kk * p.out_coset_stride;
-    // twiddles: tw[2^(lam-1) - 1 + th] = s_l * w_{2^l}^{t_low} * w_{2^lam}^{th},  l = a + lam; the three shifted copies are
-    // derived here (three shift-folds per twiddle, once per tile)
-    if (p.tw_tab) {
-        const fe* t = p.tw_tab + ((size_t)(k << p.a) + t_low) * (S - 1u);
-        for (uint32_t q = threadIdx.x; q + 1 < S; q += blockDim.x) { if (PRE) tw[q] = fe4_from(fe_ldg(t + q)); else tw1[q] = fe_ldg(t + q); }
+    // twiddles: tw[2^(lam-1) - 1 + th] = s_l * w_{2^l}^{t_low} * w_{2^lam}^{th},  l = a + lam.  A four-copy table is copied as it
+    // is (cp.async, overlapped with the tile load); otherwise the three shifted copies are derived here, once per tile
+    if (PRE && p.tw_four) {
+        const uint4* t = reinterpret_cast<const uint4*>(p.tw_tab) + ((size_t)(k << p.a) + t_low) * (4u * (S - 1u));
+        uint4* d = reinterpret_cast<uint4*>(tw);
+#pragma unroll 1
+        for (uint32_t q = threadIdx.x; q < 4u * (S - 1u); q += blockDim.x) cp_async16(d + q, t + q);
+        asm volatile("cp.async.commit_group;" ::: "memory");
     } else {
+        const fe* t = p.tw_tab ? p.tw_tab + ((size_t)(k << p.a) + t_low) * (S - 1u) : nullptr;
         for (uint32_t q = threadIdx.x; q + 1 < S; q += blockDim.x) {
-            const fe w = ntt_twiddle(p, k, t_low, q);
+            const fe w = t ? fe_ldg(t + q) : ntt_twiddle(p, k, t_low, q);
             if (PRE) tw[q] = fe4_from(w); else tw1[q] = w;
         }
     }
     // load: row v of the tile is input row (u0 + (n/2^b) v) * 2^a + t_low; store bit-reversed.
-    // blockDim (256) is a multiple of cj, so a thread keeps its column and walks rows with a constant pointer stride.
+    // blockDim (a power of two >= cj) is a multiple of cj, so a thread keeps its column and walks rows v_t, v_t + dv, .. with a
+    // constant pointer stride; counting them with shifts keeps integer divisions out of the loops.
     const uint32_t c_base = ct << log_cj;
-    const uint32_t jj_t = threadIdx.x & (cj - 1u), v_t = threadIdx.x >> log_cj, dv = blockDim.x >> log_cj;
+    const uint32_t log_bd = 31 - __clz(blockDim.x), log_dv = log_bd - log_cj;
+    const uint32_t jj_t = threadIdx.x & (cj - 1u), v_t = threadIdx.x >> log_cj, dv = 1u << log_dv;
+    const uint32_t nrow = v_t < S ? ((S - 1u - v_t) >> log_dv) + 1u : 0u;   // rows of this thread
     const bool col_ok = c_base + jj_t < p.ncols;
     {
         const size_t vstride = ((size_t)p.w_in << (p.log_n - p.b)) << p.a;
-        const fe* src = in + (((size_t)u0 << p.a) + t_low) * p.w_in + p.col0_in + c_base + jj_t + (size_t)v_t * vstride;
+        const fe* src = p.in + (size_t)kk * p.in_coset_stride + (((size_t)u0 << p.a) + t_low) * p.w_in + p.col0_in + c_base + jj_t +
+                        (size_t)v_t * vstride;
         const size_t dstride = (size_t)dv * vstride;
-        fe* smc = sm + jj_t;
-        const uint32_t brs = (32u - logS) & 31u;  // logS == 0: the only row is v = 0 and brev(0) >> 0 == 0
+        char* smc = reinterpret_cast<char*>(sm + jj_t);
+        const uint32_t brs = (32u - logS) & 31u;  // logS == 0: the only row is v = 0 and brev(0) == 0
+        const uint32_t rs16 = rs * 16u;
+        uint32_t vs = v_t << brs;                 // brev(vs) = brev(v) >> brs: row v's bit-reversed position
+        const uint32_t dvs = dv << brs;
         if (col_ok) {
-            for (uint32_t v = v_t; v < S; v += dv, src += dstride) smc[(__brev(v) >> brs) * rs] = fe_load(src);
+#pragma unroll 4
+            for (uint32_t i = 0; i < nrow; i++, vs += dvs, src += dstride) *reinterpret_cast<fe*>(smc + __brev(vs) * rs16) = fe_load(src);
         } else {  // columns past the end of a ragged last tile are zero-filled
-            for (uint32_t v = v_t; v < S; v += dv) smc[(__brev(v) >> brs) * rs] = fe_zero();
+            for (uint32_t i = 0; i < nrow; i++, vs += dvs) *reinterpret_cast<fe*>(smc + __brev(vs) * rs16) = fe_zero();
         }
     }
+    if (PRE) asm volatile("cp.async.wait_all;" ::: "memory");
     __syncthreads();
     // butterflies
     if (PRE) { if (cj >= 16) ntt_rounds<2>(sm, tw, rs, log_cj, logS); else ntt_rounds<1>(sm, tw, rs, log_cj, logS); }   // narrow tiles: one column per thread
@@ -318,28 +348,39 @@ __global__ void __launch_bounds__(256, PRE ? 2 : 3) k_ntt_pass(const NttPass p) 
     // store
     if (p.out_panel) {
         // panel = k*2^a + t_low, slot = t_high; consecutive threads write consecutive slots of one column.  A thread keeps its
-        // slot(s) and walks columns: with S >= 256 every thread covers slots tid, tid + 256, .. of each column; smaller tiles put
-        // 256 / S columns side by side
+        // slot(s) and walks columns: with S >= blockDim every thread covers slots tid, tid + blockDim, .. of each column; smaller
+        // tiles put blockDim / S columns side by side
         const size_t panel = ((size_t)(k - p.panel_k0) << p.a) + t_low;
         const uint32_t lp = logS - p.log_shard;                       // slots per stored chunk
         const size_t np = (size_t)1 << (p.log_kc + p.a);              // panels = stored cosets * 2^a
         const size_t chunk_stride = (np * p.w_out) << lp;             // elements between slot chunks (multi-GPU send view)
-        const uint32_t th0 = threadIdx.x & (S - 1u), jj0 = logS >= 8 ? 0u : (threadIdx.x >> logS), djj = logS >= 8 ? 1u : (blockDim.x >> logS);
+        const bool wide = S >= blockDim.x;
+        const uint32_t th0 = wide ? threadIdx.x : (threadIdx.x & (S - 1u)), dth = wide ? blockDim.x : S;
+        const uint32_t jj0 = wide ? 0u : (threadIdx.x >> logS), log_djj = wide ? 0u : log_bd - logS, djj = 1u << log_djj;
+        const uint32_t jend = min(cj, p.ncols - c_base);
+        const uint32_t ncol = jj0 < jend ? ((jend - 1u - jj0) >> log_djj) + 1u : 0u;
+        const size_t cstep = (size_t)djj << lp;                      // elements between the thread's columns
         fe* colp = p.out + ((panel * p.w_out + p.col0_out + c_base + jj0) << lp);
-        for (uint32_t jj = jj0; jj < cj && c_base + jj < p.ncols; jj += djj, colp += (size_t)djj << lp) {
-            for (uint32_t th = (logS >= 8 ? threadIdx.x : th0); th < S; th += blockDim.x)
-                fe_store(colp + (size_t)(th >> lp) * chunk_stride + (th & ((1u << lp) - 1u)), sm[th * rs + jj]);
+#pragma unroll 1
+        for (uint32_t th = th0; th < S; th += dth) {
+            fe* d = colp + (size_t)(th >> lp) * chunk_stride + (th & ((1u << lp) - 1u));
+            const fe* s = sm + th * rs + jj0;
+#pragma unroll 4
+            for (uint32_t j = 0; j < ncol; j++, d += cstep, s += djj) fe_store(d, *s);
         }
     } else {
         const size_t tstride = (size_t)p.w_out << p.a;
-        fe* dst = out + (((size_t)u0 << p.b) + t_low) * p.w_out + p.col0_out + c_base + jj_t + (size_t)v_t * tstride;
+        fe* dst = p.out + (size_t)kk * p.out_coset_stride + (((size_t)u0 << p.b) + t_low) * p.w_out + p.col0_out + c_base + jj_t +
+                  (size_t)v_t * tstride;
         const size_t dstride = (size_t)dv * tstride;
-        const fe* smc = sm + jj_t;
+        const fe* s = sm + v_t * rs + jj_t;
+        const uint32_t sstep = dv * rs;
         if (col_ok) {
-            for (uint32_t th = v_t; th < S; th += dv, dst += dstride) {
-                fe x = smc[th * rs];
-                if (p.do_scale) x = fe_mul(x, p.scale);
-                fe_store(dst, x);
+            if (p.do_scale) {
+                for (uint32_t i = 0; i < nrow; i++, dst += dstride, s += sstep) fe_store(dst, fe_mul(*s, p.scale));
+            } else {
+#pragma unroll 4
+                for (uint32_t i = 0; i < nrow; i++, dst += dstride, s += sstep) fe_store(dst, *s);
             }
         }
     }

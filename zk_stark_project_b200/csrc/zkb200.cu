@@ -315,51 +315,76 @@ struct zkb_ctx {
         for (uint32_t q = 0; q < passes; q++) { uint32_t take = (log_len - done + (passes - q) - 1) / (passes - q); done += take; b.push_back(done); }
         return b;
     }
-    // Tile twiddles depend only on (transform size, layer range, coset, t_low): tables of up to 64 MiB (192 MiB for narrow tiles) are built once per shape
-    // (k_build_twiddles) and re-read from L2 by every column tile, column group and proof instead of being regenerated
-    // (two multiplications per twiddle) by each of the thousands of tiles that share them.
-    std::map<std::tuple<uint32_t, uint32_t, uint32_t, uint32_t, uint32_t, uint32_t>, DevBuf> tw_cache;
+    // Tile twiddles depend only on (transform size, layer range, coset, t_low): tables are built once per shape (k_build_twiddles)
+    // and re-read from L2 by every column tile, column group and proof instead of being regenerated (two multiplications per
+    // twiddle) by each of the thousands of tiles that share them.  Wide tiles (k_ntt_pass<true>) take a table of four pre-shifted
+    // copies (64 B per twiddle) when it fits in 64 MiB — the tiles then only copy it — else a plain one (16 B per twiddle, shifted
+    // by every tile) within the same cap; narrow tiles (1-2 columns) have as many twiddles as elements, so their plain tables may
+    // take 192 MiB.  Sets p.tw_tab (null: the tiles generate their twiddles) and p.tw_four.
+    std::map<std::tuple<uint32_t, uint32_t, uint32_t, uint32_t, uint32_t, uint32_t, uint32_t>, DevBuf> tw_cache;
     size_t tw_cache_bytes = 0;
-    const fe* twiddle_table(const NttPass& p, uint32_t all_cosets) {
+    void twiddle_table(NttPass& p, uint32_t all_cosets) {
         const uint32_t S = 1u << (p.b - p.a);
-        const uint64_t entries = ((uint64_t)all_cosets << p.a) * (S - 1u), bytes = entries * 16;
-        // narrow tiles (1-2 columns) have as many twiddles as elements: generating them (two multiplications each) would cost
-        // 40 % on top of the butterflies, so their tables may be larger than those of the wide tiles, which amortise a twiddle
-        // over 4-16 columns
-        if (S < 2 || bytes > ((uint64_t)(pre_twiddles(p.cj) ? 64 : 192) << 20)) return nullptr;
-        const auto key = std::make_tuple(p.log_n, p.a, p.b, p.coset, p.inverse, p.coset ? p.log_lde : 0u);
-        auto it = tw_cache.find(key);
-        if (it != tw_cache.end()) return it->second.as<fe>();
-        if (tw_cache_bytes + bytes > ((uint64_t)768 << 20)) {  // a long-lived context that has seen many shapes: start over
-            CK(cudaStreamSynchronize(stream));
-            for (auto& kv : tw_cache) kv.second.release();
-            tw_cache.clear(); tw_cache_bytes = 0;
+        const uint64_t entries = ((uint64_t)all_cosets << p.a) * (S - 1u);
+        const bool pre = pre_twiddles(p.cj);
+        const uint64_t cap = (uint64_t)(pre ? 64 : 192) << 20;
+        p.tw_tab = nullptr; p.tw_four = 0;
+        static const bool log_tables = getenv("ZKB_HOST_PROFILE") != nullptr;   // diagnostics: which passes get which table
+        if (S < 2 || entries * 16 > cap) {
+            if (log_tables && S >= 2)
+                fprintf(stderr, "[zkb twiddles] log_n %u layers [%u, %u) coset %u inverse %u cj %u: no table (%.2f MiB plain), generated\n", p.log_n,
+                        p.a, p.b, p.coset, p.inverse, p.cj, entries * 16 / 1048576.0);
+            return;
         }
-        DevBuf& b = tw_cache[key];
-        b.ensure(bytes);
-        tw_cache_bytes += bytes;
-        NttPass q = p;
-        q.n_cosets = all_cosets; q.coset0 = 0; q.tw_tab = nullptr;
-        k_build_twiddles<<<(unsigned)((entries + 255) / 256), 256, 0, stream>>>(q, b.as<fe>());
-        check_launch();
-        return b.as<fe>();
+        const uint32_t four = pre && entries * 64 <= cap ? 1u : 0u;
+        const uint64_t bytes = entries * (four ? 64 : 16);
+        const auto key = std::make_tuple(p.log_n, p.a, p.b, p.coset, p.inverse, p.coset ? p.log_lde : 0u, four);
+        auto it = tw_cache.find(key);
+        if (it == tw_cache.end()) {
+            if (tw_cache_bytes + bytes > ((uint64_t)768 << 20)) {  // a long-lived context that has seen many shapes: start over
+                if (log_tables) fprintf(stderr, "[zkb twiddles] cache of %.2f MiB over budget: cleared\n", tw_cache_bytes / 1048576.0);
+                CK(cudaStreamSynchronize(stream));
+                for (auto& kv : tw_cache) kv.second.release();
+                tw_cache.clear(); tw_cache_bytes = 0;
+            }
+            DevBuf& b = tw_cache[key];
+            b.ensure(bytes);
+            tw_cache_bytes += bytes;
+            if (log_tables)
+                fprintf(stderr, "[zkb twiddles] log_n %u layers [%u, %u) coset %u inverse %u cj %u: %s table %.2f MiB, cache %.2f MiB\n", p.log_n, p.a,
+                        p.b, p.coset, p.inverse, p.cj, four ? "four-copy" : "plain", bytes / 1048576.0, tw_cache_bytes / 1048576.0);
+            NttPass q = p;
+            q.n_cosets = all_cosets; q.coset0 = 0; q.tw_four = four;
+            k_build_twiddles<<<(unsigned)((entries + 255) / 256), 256, 0, stream>>>(q, b.as<fe>());
+            check_launch();
+            it = tw_cache.find(key);
+        }
+        p.tw_tab = it->second.as<fe>(); p.tw_four = four;
     }
-    void launch_pass(NttPass& p) {
+    void launch_pass(NttPass p) {
         const uint32_t S = 1u << (p.b - p.a);
         const uint32_t rs = p.cj + (p.cj > 1 ? 1 : 0);
         const bool pre = pre_twiddles(p.cj);
         const size_t smem = ((size_t)S * rs + (pre ? 4 : 1) * (size_t)S) * 16;   // tile + twiddles (four copies each for wide tiles)
-        const uint64_t tiles = (uint64_t)((p.ncols + p.cj - 1) / p.cj) * p.n_cosets * ((uint64_t)1 << (p.log_n - (p.b - p.a)));
-        if (tiles > 0x7fffffffull) throw InvalidArg("transform too large for one launch");
+        // grid: x = column tile, y = coset, z = (t_low, u0) tile; z is limited to 65535 per launch
+        const uint32_t n_ct = (p.ncols + p.cj - 1) / p.cj;
+        const uint64_t tiles = (uint64_t)1 << (p.log_n - (p.b - p.a));
+        if (p.n_cosets > 65535) throw InvalidArg("transform too large for one launch");
+        uint32_t threads = 256;
         if (pre) {
             // one two-column radix-8 unit per thread and round: S * cj / 16 threads keep every thread busy (128-row tiles of the
             // three-pass transforms get 128-thread blocks, four per SM); never fewer than the panel store needs (min(S, 256))
             const uint32_t units = p.cj >= 16 ? S * p.cj / 16 : S * p.cj / 8;   // radix-8 units per round (two columns each for 16-wide tiles)
-            uint32_t threads = std::max<uint32_t>(units, std::min<uint32_t>(S, 256));
+            threads = std::max<uint32_t>(units, std::min<uint32_t>(S, 256));
             threads = std::min<uint32_t>(256, std::max<uint32_t>(32, threads));
-            k_ntt_pass<true><<<(unsigned)tiles, threads, smem, stream>>>(p);
-        } else k_ntt_pass<false><<<(unsigned)tiles, 256, smem, stream>>>(p);
-        check_launch();
+        }
+        for (uint64_t z0 = 0; z0 < tiles; z0 += 65535) {
+            p.tile0 = (uint32_t)z0;
+            const dim3 grid(n_ct, p.n_cosets, (unsigned)std::min<uint64_t>(65535, tiles - z0));
+            if (pre) k_ntt_pass<true><<<grid, threads, smem, stream>>>(p);
+            else k_ntt_pass<false><<<grid, threads, smem, stream>>>(p);
+            check_launch();
+        }
     }
     // generic multi-pass transform of `ncols` columns of length 2^log_len.
     //  in : row-major [len][w_in] (column window col0_in..)         bufs: scratch buffers for intermediate passes
@@ -409,7 +434,7 @@ struct zkb_ctx {
                 p.coset = x.coset_lde ? 1 : 0; p.inverse = x.inverse ? 1 : 0;
                 p.log_tab = log_tab; p.log_lde = x.coset_lde ? x.log_lde : 0;
                 p.roots = roots; p.pow3 = d_pow3.as<fe>();
-                p.tw_tab = twiddle_table(p, all_cosets);
+                twiddle_table(p, all_cosets);
                 if (last) {
                     p.out = x.out; p.w_out = x.w_out; p.col0_out = x.col0_out;
                     p.out_panel = x.coset_lde ? 1 : 0;
