@@ -108,6 +108,25 @@ __host__ __device__ __forceinline__ void b3_parent(const uint32_t l[8], const ui
     b3_iv(out);
     b3_compress(out, m, 0, 64, B3_PARENT | (root ? B3_ROOT : 0u));
 }
+// hash(a || b) of two digests: 64 bytes = one ROOT chunk (Blake3_256::merge, the Merkle tree's inner nodes)
+__host__ __device__ __forceinline__ void b3_merge(const uint32_t a[8], const uint32_t b[8], uint32_t out[8]) {
+    uint32_t m[16];
+#pragma unroll
+    for (int i = 0; i < 8; i++) { m[i] = a[i]; m[8 + i] = b[i]; }
+    b3_iv(out);
+    b3_compress(out, m, 0, 64, B3_CHUNK_START | B3_CHUNK_END | B3_ROOT);
+}
+// hash(seed || v_le64): 40 bytes = one ROOT chunk (Blake3_256::merge_with_int)
+__host__ __device__ __forceinline__ void b3_with_int(const uint32_t seed[8], uint64_t v, uint32_t out[8]) {
+    uint32_t m[16];
+#pragma unroll
+    for (int i = 0; i < 8; i++) m[i] = seed[i];
+    m[8] = (uint32_t)v; m[9] = (uint32_t)(v >> 32);
+#pragma unroll
+    for (int i = 10; i < 16; i++) m[i] = 0;
+    b3_iv(out);
+    b3_compress(out, m, 0, 40, B3_CHUNK_START | B3_CHUNK_END | B3_ROOT);
+}
 
 #ifdef __CUDACC__
 // BLAKE3 of `count` field elements (16 B each) read from base[j * stride]; this is

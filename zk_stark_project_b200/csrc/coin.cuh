@@ -27,30 +27,11 @@ struct DevTs {
 };
 
 // ---- BLAKE3 pieces -------------------------------------------------------------------------------------------------------
-// merge(a, b) = hash(a || b), 64 bytes = one ROOT chunk
-__device__ __forceinline__ void fs_merge(const uint32_t a[8], const uint32_t b[8], uint32_t out[8]) {
-    uint32_t m[16];
-#pragma unroll
-    for (int i = 0; i < 8; i++) { m[i] = a[i]; m[8 + i] = b[i]; }
-    b3_iv(out);
-    b3_compress(out, m, 0, 64, B3_CHUNK_START | B3_CHUNK_END | B3_ROOT);
-}
-// merge_with_int(seed, v) = hash(seed || v_le64), 40 bytes
-__device__ __forceinline__ void fs_with_int(const uint32_t seed[8], uint64_t v, uint32_t out[8]) {
-    uint32_t m[16];
-#pragma unroll
-    for (int i = 0; i < 8; i++) m[i] = seed[i];
-    m[8] = (uint32_t)v; m[9] = (uint32_t)(v >> 32);
-#pragma unroll
-    for (int i = 10; i < 16; i++) m[i] = 0;
-    b3_iv(out);
-    b3_compress(out, m, 0, 40, B3_CHUNK_START | B3_CHUNK_END | B3_ROOT);
-}
 // RandomCoin::draw: first 16 bytes of next() as a little-endian u128, rejected while >= p.  One thread.
 __device__ __forceinline__ fe fs_draw(const uint32_t seed[8], uint32_t* failed) {
     for (uint64_t counter = 1; counter <= 1000; counter++) {
         uint32_t d[8];
-        fs_with_int(seed, counter, d);
+        b3_with_int(seed, counter, d);
         // v < p  <=>  not (limbs 3,2 all ones and (limb1, limb0) >= (0xFFFFD300, 1))
         const bool ge = d[3] == 0xFFFFFFFFu && d[2] == 0xFFFFFFFFu && (d[1] > 0xFFFFD300u || (d[1] == 0xFFFFD300u && d[0] >= 1u));
         if (!ge) { fe r; r.x[0] = d[0]; r.x[1] = d[1]; r.x[2] = d[2]; r.x[3] = d[3]; return r; }
@@ -60,7 +41,7 @@ __device__ __forceinline__ fe fs_draw(const uint32_t seed[8], uint32_t* failed) 
 }
 __device__ __forceinline__ void fs_reseed(uint32_t seed[8], const uint32_t digest[8]) {
     uint32_t t[8];
-    fs_merge(seed, digest, t);
+    b3_merge(seed, digest, t);
 #pragma unroll
     for (int i = 0; i < 8; i++) seed[i] = t[i];
 }
@@ -312,7 +293,7 @@ __global__ void __launch_bounds__(256) k_fs_grind(DevTs* ts, uint32_t bits, unsi
         if (!done && (x > limit || x > *best)) done = true;
         if (!done) {
             uint32_t d[8];
-            fs_with_int(seed, x, d);
+            b3_with_int(seed, x, d);
             const uint64_t head = ((uint64_t)d[1] << 32) | d[0];
             if ((head & mask) == 0) { atomicMin(&ts->nonce, (unsigned long long)x); done = true; }
         }
@@ -328,7 +309,7 @@ __global__ void __launch_bounds__(ZKB_FS_THREADS) k_fs_positions(DevTs* ts, uint
         uint32_t seed[8], t[8];
 #pragma unroll
         for (int i = 0; i < 8; i++) seed[i] = ts->seed[i];
-        fs_with_int(seed, ts->nonce, t);
+        b3_with_int(seed, ts->nonce, t);
 #pragma unroll
         for (int i = 0; i < 8; i++) { s_seed[i] = t[i]; ts->seed[i] = t[i]; }
     }
@@ -338,7 +319,7 @@ __global__ void __launch_bounds__(ZKB_FS_THREADS) k_fs_positions(DevTs* ts, uint
     for (int i = 0; i < 8; i++) seed[i] = s_seed[i];
     for (uint32_t q = threadIdx.x; q < num_queries; q += blockDim.x) {
         uint32_t d[8];
-        fs_with_int(seed, (uint64_t)q + 1, d);
+        b3_with_int(seed, (uint64_t)q + 1, d);
         ts->positions[q] = d[0] & domain_mask;
     }
 }

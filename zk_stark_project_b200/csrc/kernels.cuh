@@ -52,6 +52,20 @@ __device__ __forceinline__ size_t lde_row_base(const LdeMat& m, uint32_t k, uint
     const uint32_t chunk = m.view == 0 ? (slot >> m.log_p) : 0u;
     return (((size_t)chunk * np + panel) * m.bw << m.log_p) + (slot & ((1u << m.log_p) - 1u));
 }
+// The rows a rank stores, enumerated (panel, slot): consecutive row numbers are consecutive slots of one panel.  Row `gid` is
+// (coset k, trace-domain index i); its Merkle leaf is r = i*beta + k - leaf0, or, compact (coset-sharded matrices),
+// r = i * (stored cosets) + local coset.
+struct LdeLeaf { uint32_t k, i; uint64_t r; };
+__device__ __forceinline__ LdeLeaf lde_leaf(const LdeMat& m, uint64_t gid, uint64_t leaf0, uint32_t compact) {
+    const uint32_t lpf = lde_full_log_p(m), lt = m.log_n - lpf;
+    const uint32_t lslots = m.view == 0 ? lpf : m.log_p;
+    const uint32_t s = (uint32_t)gid & ((1u << lslots) - 1u);
+    const uint32_t panel = (uint32_t)(gid >> lslots);
+    const uint32_t slot = m.view == 0 ? s : ((m.q_self << m.log_p) + s);
+    const uint32_t k = m.k0 + (panel >> lt), t_low = panel & ((1u << lt) - 1u);
+    const uint32_t i = t_low + (slot << lt);
+    return {k, i, compact ? (((uint64_t)i << m.log_kc) + (k - m.k0)) : (((uint64_t)i << m.log_beta) + k - leaf0)};
+}
 __device__ __forceinline__ size_t lde_col_off(const LdeMat& m, uint32_t j) {
     const uint32_t blk = (j * m.bw_magic) >> 16;
     return (size_t)blk * m.blk_stride + ((size_t)(j - blk * m.bw) << m.log_p);
@@ -119,12 +133,17 @@ struct NttPass {
 
 __device__ __forceinline__ uint32_t bitrev(uint32_t v, uint32_t bits) { return bits == 0 ? 0u : (__brev(v) >> (32 - bits)); }
 
+// twiddle multiply of a butterfly: plain twiddles (fe) or four pre-shifted copies (fe4, f128.cuh)
+__device__ __forceinline__ fe tw_mul(const fe& x, const fe& w) { return fe_mul(x, w); }
+__device__ __forceinline__ fe tw_mul(const fe& x, const fe4& w) { return fe_mul_pre4(x, w); }
+
 // RHO consecutive DIT layers (lam0, lam0 + RHO] of NC columns, done in registers: the 2^RHO elements of a unit sit at
 // positions base + d * 2^lam0.  Layer lam uses tw[2^(lam-1) - 1 + (p0 mod 2^(lam-1))] for the pair (p0, p0 + 2^(lam-1)).
-// Twiddles are held as four pre-shifted copies (fe4, f128.cuh): one 64-byte load serves NC * 2^(RHO-1-s) butterflies of layer s.
+// With four-copy twiddles (TW = fe4) one 64-byte load serves NC * 2^(RHO-1-s) butterflies of layer s; narrow tiles (1-2
+// columns) reuse a twiddle too rarely for the three shift-folds of fe4_from to pay and take plain ones (TW = fe, NC = 1).
 // The NC columns of a thread are `cstride` apart so that the threads of a quarter-warp touch one contiguous 128-byte run.
-template <int RHO, int NC>
-__device__ __forceinline__ void ntt_unit(fe* __restrict__ col, const uint32_t rs, const uint32_t cstride, const fe4* __restrict__ tw,
+template <int RHO, int NC, class TW>
+__device__ __forceinline__ void ntt_unit(fe* __restrict__ col, const uint32_t rs, const uint32_t cstride, const TW* __restrict__ tw,
                                          const uint32_t base, const uint32_t lam0) {
     constexpr int R = 1 << RHO;
     fe x[NC][R];
@@ -137,17 +156,17 @@ __device__ __forceinline__ void ntt_unit(fe* __restrict__ col, const uint32_t rs
     const uint32_t base_low = base & ((1u << lam0) - 1u);
 #pragma unroll
     for (int s = 0; s < RHO; s++) {
-        const fe4* twl = tw + ((1u << (lam0 + s)) - 1u) + base_low;
+        const TW* twl = tw + ((1u << (lam0 + s)) - 1u) + base_low;
 #pragma unroll
         for (int t = 0; t < (1 << s); t++) {
-            const fe4 w = twl[(uint32_t)t << lam0];
+            const TW w = twl[(uint32_t)t << lam0];
 #pragma unroll
             for (int g = 0; g < (R >> (s + 1)); g++) {
                 const int d0 = g * (2 << s) + t, d1 = d0 + (1 << s);
 #pragma unroll
                 for (int c = 0; c < NC; c++) {
                     const fe u = x[c][d0];
-                    const fe v = fe_mul_pre4(x[c][d1], w);
+                    const fe v = tw_mul(x[c][d1], w);
                     x[c][d0] = fe_add(u, v);
                     x[c][d1] = fe_sub(u, v);
                 }
@@ -197,58 +216,8 @@ __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src)
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src) : "memory");
 }
 
-// the same for ONE column with plain (single-copy) twiddles: narrow tiles (1-2 columns) reuse a twiddle too rarely for the
-// three shift-folds of fe4_from to pay
-template <int RHO>
-__device__ __forceinline__ void ntt_unit_plain(fe* __restrict__ col, const uint32_t rs, const fe* __restrict__ tw, const uint32_t base, const uint32_t lam0) {
-    constexpr int R = 1 << RHO;
-    fe x[R];
-    const uint32_t step = rs << lam0;
-    fe* p = col + base * rs;
-#pragma unroll
-    for (int d = 0; d < R; d++) x[d] = p[d * step];
-    const uint32_t base_low = base & ((1u << lam0) - 1u);
-#pragma unroll
-    for (int s = 0; s < RHO; s++) {
-        const fe* twl = tw + ((1u << (lam0 + s)) - 1u) + base_low;
-#pragma unroll
-        for (int t = 0; t < (1 << s); t++) {
-            const fe w = twl[(uint32_t)t << lam0];
-#pragma unroll
-            for (int g = 0; g < (R >> (s + 1)); g++) {
-                const int d0 = g * (2 << s) + t, d1 = d0 + (1 << s);
-                const fe u = x[d0];
-                const fe v = fe_mul(x[d1], w);
-                x[d0] = fe_add(u, v);
-                x[d1] = fe_sub(u, v);
-            }
-        }
-    }
-#pragma unroll
-    for (int d = 0; d < R; d++) p[d * step] = x[d];
-}
-template <int RHO>
-__device__ __forceinline__ void ntt_round_plain(fe* sm, const fe* tw, uint32_t rs, uint32_t log_cj, uint32_t logS, uint32_t lam0) {
-    const uint32_t cj_mask = (1u << log_cj) - 1u;
-    const uint32_t units = (1u << (logS - RHO)) << log_cj;
-    for (uint32_t idx = threadIdx.x; idx < units; idx += blockDim.x) {
-        const uint32_t jj = idx & cj_mask, u = idx >> log_cj;
-        const uint32_t base = (u & ((1u << lam0) - 1u)) + ((u >> lam0) << (lam0 + RHO));
-        ntt_unit_plain<RHO>(sm + jj, rs, tw, base, lam0);
-    }
-}
-__device__ __forceinline__ void ntt_rounds_plain(fe* sm, const fe* tw, uint32_t rs, uint32_t log_cj, uint32_t logS) {
-    for (uint32_t lam0 = 0; lam0 < logS;) {
-        const uint32_t left = logS - lam0;
-        if (left >= 3 && left != 4) { ntt_round_plain<3>(sm, tw, rs, log_cj, logS, lam0); lam0 += 3; }
-        else if (left >= 2) { ntt_round_plain<2>(sm, tw, rs, log_cj, logS, lam0); lam0 += 2; }
-        else { ntt_round_plain<1>(sm, tw, rs, log_cj, logS, lam0); lam0 += 1; }
-        __syncthreads();
-    }
-}
-
-template <int RHO, int NC>
-__device__ __forceinline__ void ntt_round(fe* sm, const fe4* tw, uint32_t rs, uint32_t log_cj, uint32_t logS, uint32_t lam0) {
+template <int RHO, int NC, class TW>
+__device__ __forceinline__ void ntt_round(fe* sm, const TW* tw, uint32_t rs, uint32_t log_cj, uint32_t logS, uint32_t lam0) {
     // a thread owns columns jj and (NC == 2) jj + cj/2 of one unit
     const uint32_t log_cw = log_cj - (NC == 2 ? 1u : 0u);
     const uint32_t cw_mask = (1u << log_cw) - 1u;
@@ -259,8 +228,8 @@ __device__ __forceinline__ void ntt_round(fe* sm, const fe4* tw, uint32_t rs, ui
         ntt_unit<RHO, NC>(sm + jj, rs, 1u << log_cw, tw, base, lam0);
     }
 }
-template <int NC>
-__device__ __forceinline__ void ntt_rounds(fe* sm, const fe4* tw, uint32_t rs, uint32_t log_cj, uint32_t logS) {
+template <int NC, class TW>
+__device__ __forceinline__ void ntt_rounds(fe* sm, const TW* tw, uint32_t rs, uint32_t log_cj, uint32_t logS) {
     // rounds of up to three layers held in registers
     if (NC == 2 && log_cj == 4 && logS == 8) {
         // 256 x 16 tiles (every pass of the 2^16-row transforms of >= 9 columns): with the strides and layer offsets known at
@@ -344,7 +313,7 @@ __global__ void __launch_bounds__(256, PRE ? 2 : 3) k_ntt_pass(const NttPass p) 
     __syncthreads();
     // butterflies
     if (PRE) { if (cj >= 16) ntt_rounds<2>(sm, tw, rs, log_cj, logS); else ntt_rounds<1>(sm, tw, rs, log_cj, logS); }   // narrow tiles: one column per thread
-    else ntt_rounds_plain(sm, tw1, rs, log_cj, logS);
+    else ntt_rounds<1>(sm, tw1, rs, log_cj, logS);
     // store
     if (p.out_panel) {
         // panel = k*2^a + t_low, slot = t_high; consecutive threads write consecutive slots of one column.  A thread keeps its
@@ -407,17 +376,10 @@ __global__ void __launch_bounds__(128) k_hash_lde_rows(const LdeMat m, uint32_t*
     const uint32_t lpf = lde_full_log_p(m), lt = m.log_n - lpf;
     const uint32_t log_rows = m.log_kc + lt + (m.view == 0 ? lpf : m.log_p);   // rows stored on this rank
     if (gid >> log_rows) return;
-    const uint32_t lslots = m.view == 0 ? lpf : m.log_p;
-    const uint32_t s = (uint32_t)gid & ((1u << lslots) - 1u);
-    const uint32_t panel = (uint32_t)(gid >> lslots);
-    const uint32_t slot = m.view == 0 ? s : ((m.q_self << m.log_p) + s);
-    const uint32_t k = m.k0 + (panel >> lt), t_low = panel & ((1u << lt) - 1u);
-    const uint32_t i = t_low + (slot << lt);
-    // leaf index: global r = i*beta + k; compact (coset-sharded matrices): i * (stored cosets) + local coset
-    const uint64_t r = compact ? (((uint64_t)i << m.log_kc) + (k - m.k0)) : (((uint64_t)i << m.log_beta) + k - leaf0);
+    const LdeLeaf L = lde_leaf(m, gid, leaf0, compact);
     uint32_t d[8];
-    b3_hash_elems(m.data + lde_row_base(m, k, i), (size_t)1 << m.log_p, m.w, d, m.bw, m.bw_magic, m.blk_stride);
-    uint4* o = reinterpret_cast<uint4*>(leaves + r * 8);
+    b3_hash_elems(m.data + lde_row_base(m, L.k, L.i), (size_t)1 << m.log_p, m.w, d, m.bw, m.bw_magic, m.blk_stride);
+    uint4* o = reinterpret_cast<uint4*>(leaves + L.r * 8);
     o[0] = make_uint4(d[0], d[1], d[2], d[3]);
     o[1] = make_uint4(d[4], d[5], d[6], d[7]);
 }
@@ -430,17 +392,10 @@ __global__ void __launch_bounds__(128) k_hash_lde_rows_split(const LdeMat m, uin
     const uint32_t lpf = lde_full_log_p(m), lt = m.log_n - lpf;
     const uint32_t log_rows = m.log_kc + lt + (m.view == 0 ? lpf : m.log_p);
     const bool live = ((t >> 2) >> log_rows) == 0;      // whole warps take part in the shuffles; dead rows hash row 0 and drop it
-    const uint64_t gid = live ? (t >> 2) : 0;
-    const uint32_t lslots = m.view == 0 ? lpf : m.log_p;
-    const uint32_t s = (uint32_t)gid & ((1u << lslots) - 1u);
-    const uint32_t panel = (uint32_t)(gid >> lslots);
-    const uint32_t slot = m.view == 0 ? s : ((m.q_self << m.log_p) + s);
-    const uint32_t k = m.k0 + (panel >> lt), t_low = panel & ((1u << lt) - 1u);
-    const uint32_t i = t_low + (slot << lt);
-    const uint64_t r = compact ? (((uint64_t)i << m.log_kc) + (k - m.k0)) : (((uint64_t)i << m.log_beta) + k - leaf0);
+    const LdeLeaf L = lde_leaf(m, live ? (t >> 2) : 0, leaf0, compact);
     const uint32_t nchunks = (m.w + 63u) / 64u;         // 2..4 (the caller sends single-chunk rows to k_hash_lde_rows)
     uint32_t cv[8], nb[8];
-    if (c < nchunks) b3_chunk_cv_elems(m.data + lde_row_base(m, k, i), (size_t)1 << m.log_p, m.w, c, cv, m.bw, m.bw_magic, m.blk_stride);
+    if (c < nchunks) b3_chunk_cv_elems(m.data + lde_row_base(m, L.k, L.i), (size_t)1 << m.log_p, m.w, c, cv, m.bw, m.bw_magic, m.blk_stride);
     else {
 #pragma unroll
         for (int q = 0; q < 8; q++) cv[q] = 0;
@@ -465,7 +420,7 @@ __global__ void __launch_bounds__(128) k_hash_lde_rows_split(const LdeMat m, uin
         }
     }
     if (live && c == 0) {
-        uint4* o = reinterpret_cast<uint4*>(leaves + r * 8);
+        uint4* o = reinterpret_cast<uint4*>(leaves + L.r * 8);
         o[0] = make_uint4(cv[0], cv[1], cv[2], cv[3]);
         o[1] = make_uint4(cv[4], cv[5], cv[6], cv[7]);
     }
@@ -502,12 +457,10 @@ __global__ void __launch_bounds__(256) k_merkle_level(const uint32_t* __restrict
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
     const uint4* s = reinterpret_cast<const uint4*>(src + i * 16);
-    uint32_t m[16], cv[8];
-    uint4 a = s[0], b = s[1], c = s[2], d = s[3];
-    m[0] = a.x; m[1] = a.y; m[2] = a.z; m[3] = a.w; m[4] = b.x; m[5] = b.y; m[6] = b.z; m[7] = b.w;
-    m[8] = c.x; m[9] = c.y; m[10] = c.z; m[11] = c.w; m[12] = d.x; m[13] = d.y; m[14] = d.z; m[15] = d.w;
-    b3_iv(cv);
-    b3_compress(cv, m, 0, 64, B3_CHUNK_START | B3_CHUNK_END | B3_ROOT);
+    const uint4 a = s[0], b = s[1], c = s[2], d = s[3];
+    const uint32_t l[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w}, r[8] = {c.x, c.y, c.z, c.w, d.x, d.y, d.z, d.w};
+    uint32_t cv[8];
+    b3_merge(l, r, cv);
     uint4* o = reinterpret_cast<uint4*>(dst + i * 8);
     o[0] = make_uint4(cv[0], cv[1], cv[2], cv[3]);
     o[1] = make_uint4(cv[4], cv[5], cv[6], cv[7]);
@@ -516,17 +469,14 @@ __global__ void __launch_bounds__(256) k_merkle_level(const uint32_t* __restrict
 // top of a Merkle heap in one launch: levels top, top/2, ..., 1 (top <= 512 nodes) by a single block; every level is
 // read back from global memory after a block barrier (the data is a few KB and stays in L1/L2)
 __global__ void __launch_bounds__(512) k_merkle_top(uint32_t* __restrict__ heap, uint32_t top) {
-    const uint32_t one_flags = B3_CHUNK_START | B3_CHUNK_END | B3_ROOT;
     for (uint32_t lvl = top; lvl >= 1; lvl >>= 1) {
         const uint32_t i = threadIdx.x;
         if (i < lvl) {
             const uint4* s = reinterpret_cast<const uint4*>(heap + (size_t)(2 * (lvl + i)) * 8);
-            uint32_t m[16], cv[8];
-            uint4 a = s[0], b = s[1], c = s[2], d = s[3];
-            m[0] = a.x; m[1] = a.y; m[2] = a.z; m[3] = a.w; m[4] = b.x; m[5] = b.y; m[6] = b.z; m[7] = b.w;
-            m[8] = c.x; m[9] = c.y; m[10] = c.z; m[11] = c.w; m[12] = d.x; m[13] = d.y; m[14] = d.z; m[15] = d.w;
-            b3_iv(cv);
-            b3_compress(cv, m, 0, 64, one_flags);
+            const uint4 a = s[0], b = s[1], c = s[2], d = s[3];
+            const uint32_t l[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w}, r[8] = {c.x, c.y, c.z, c.w, d.x, d.y, d.z, d.w};
+            uint32_t cv[8];
+            b3_merge(l, r, cv);
             uint4* o = reinterpret_cast<uint4*>(heap + (size_t)(lvl + i) * 8);
             o[0] = make_uint4(cv[0], cv[1], cv[2], cv[3]);
             o[1] = make_uint4(cv[4], cv[5], cv[6], cv[7]);
@@ -929,27 +879,6 @@ __global__ void __launch_bounds__(128) k_fri_fold16(const FriFoldParams p) {
 #pragma unroll
     for (int kq = 14; kq >= 0; kq--) acc = fe_add(fe_mul(acc, t), v[kq]);
     fe_store(p.out + i, fe_mul(acc, p.inv16));
-}
-
-// ------------------------------------------------------------------------------------------------
-// K10: ProverChannel::grind_query_seed (grinding factor from src/main.rs:101): smallest nonce >= base whose
-// Blake3(seed || nonce_le64) has >= bits trailing zeros in its first little-endian u64
-__global__ void __launch_bounds__(256) k_grind(const uint32_t* __restrict__ seed, uint64_t base, uint64_t count, uint32_t bits,
-                                               unsigned long long* __restrict__ found) {
-    const uint64_t gid = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (gid >= count) return;
-    const uint64_t nonce = base + gid;
-    uint32_t m[16], cv[8];
-#pragma unroll
-    for (int i = 0; i < 8; i++) m[i] = __ldg(seed + i);
-    m[8] = (uint32_t)nonce; m[9] = (uint32_t)(nonce >> 32);
-#pragma unroll
-    for (int i = 10; i < 16; i++) m[i] = 0;
-    b3_iv(cv);
-    b3_compress(cv, m, 0, 40, B3_CHUNK_START | B3_CHUNK_END | B3_ROOT);
-    const uint64_t head = ((uint64_t)cv[1] << 32) | cv[0];
-    const uint64_t mask = bits >= 64 ? ~0ull : (((uint64_t)1 << bits) - 1ull);
-    if ((head & mask) == 0) atomicMin(found, (unsigned long long)nonce);
 }
 
 // ------------------------------------------------------------------------------------------------

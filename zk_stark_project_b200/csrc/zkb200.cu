@@ -61,6 +61,37 @@ struct DevBuf {
     template <class T> T* as() const { return reinterpret_cast<T*>(p); }
 };
 
+// Device tables kept per shape (twiddles, evaluator inputs, divisors), so that captured graphs of several shapes stay valid
+// side by side.  A long-lived context that has seen many shapes would hold them all: an entry that does not fit the budget
+// next to the others releases every entry first (after the stream is done with them) and the cache starts over.
+template <class Key>
+struct ShapeCache {
+    std::map<Key, DevBuf> map;
+    size_t bytes = 0;
+    const size_t budget;
+    explicit ShapeCache(size_t budget_bytes) : budget(budget_bytes) {}
+    DevBuf* find(const Key& k) {
+        auto it = map.find(k);
+        return it == map.end() ? nullptr : &it->second;
+    }
+    bool full(size_t size) const { return bytes + size > budget && !map.empty(); }
+    DevBuf& insert(const Key& k, size_t size, cudaStream_t stream) {
+        if (full(size)) {
+            CK(cudaStreamSynchronize(stream));
+            release();
+        }
+        DevBuf& b = map[k];
+        try { b.ensure(size); } catch (...) { map.erase(k); throw; }   // no entry without memory behind it
+        bytes += size;
+        return b;
+    }
+    void release() {
+        for (auto& kv : map) kv.second.release();
+        map.clear();
+        bytes = 0;
+    }
+};
+
 static inline fe to_fe(const HF& h) {
     fe r;
     r.x[0] = (uint32_t)h.v; r.x[1] = (uint32_t)(h.v >> 32); r.x[2] = (uint32_t)(h.v >> 64); r.x[3] = (uint32_t)(h.v >> 96);
@@ -135,11 +166,9 @@ struct zkb_ctx {
     struct FsTree { size_t o_rows, o_paths; uint32_t width, depth; };
     struct FsLayout { size_t o_ood = 0, o_rem = 0, host_bytes = 0, o_coef = 0, o_gamma = 0, o_scr = 0, total = 0; uint32_t rem_cap = 0; std::vector<FsTree> trees; } fs;
     DevBuf d_fs, d_in, d_rem_coef;      // d_in: per-proof inputs [assertion values na][AIR params]
-    // shape-only evaluator inputs (periodic column, assertion columns / indices) and divisor tables (k_build_divisors), kept per
-    // distinct shape so that captured graphs of several shapes stay valid side by side
-    std::map<std::string, DevBuf> pack_cache;
-    std::map<std::vector<uint64_t>, DevBuf> div_cache;
-    size_t pack_cache_bytes = 0, div_cache_bytes = 0;
+    // shape-only evaluator inputs (periodic column, assertion columns / indices) and divisor tables (k_build_divisors)
+    ShapeCache<std::string> pack_cache{(size_t)64 << 20};
+    ShapeCache<std::vector<uint64_t>> div_cache{(size_t)2 << 30};
     // ---- CUDA graphs for small proofs: the whole enqueue sequence of a shape, replayed with one launch ---------------------
     struct GraphEntry { cudaGraphExec_t exec = nullptr; uint64_t epoch = 0; uint32_t seen = 0; uint64_t launches = 0; };
     std::map<std::string, GraphEntry> graphs;
@@ -218,9 +247,9 @@ struct zkb_ctx {
         if (comm) { g_nccl.CommDestroy(comm); comm = nullptr; }
         for (auto& b : d_fri_evals) b.release();
         for (auto& b : d_fri_tree) b.release();
-        for (auto& kv : tw_cache) kv.second.release();
-        for (auto& kv : pack_cache) kv.second.release();
-        for (auto& kv : div_cache) kv.second.release();
+        tw_cache.release();
+        pack_cache.release();
+        div_cache.release();
         for (auto& kv : graphs) if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
         if (ev_ok) { for (auto& pr : tev) for (auto& x : pr) cudaEventDestroy(x); for (auto& x : ev_group) cudaEventDestroy(x); cudaStreamDestroy(copy_stream); cudaStreamDestroy(xchg_stream); }
         if (h_stage) cudaFreeHost(h_stage);
@@ -321,8 +350,7 @@ struct zkb_ctx {
     // copies (64 B per twiddle) when it fits in 64 MiB — the tiles then only copy it — else a plain one (16 B per twiddle, shifted
     // by every tile) within the same cap; narrow tiles (1-2 columns) have as many twiddles as elements, so their plain tables may
     // take 192 MiB.  Sets p.tw_tab (null: the tiles generate their twiddles) and p.tw_four.
-    std::map<std::tuple<uint32_t, uint32_t, uint32_t, uint32_t, uint32_t, uint32_t, uint32_t>, DevBuf> tw_cache;
-    size_t tw_cache_bytes = 0;
+    ShapeCache<std::tuple<uint32_t, uint32_t, uint32_t, uint32_t, uint32_t, uint32_t, uint32_t>> tw_cache{(size_t)768 << 20};
     void twiddle_table(NttPass& p, uint32_t all_cosets) {
         const uint32_t S = 1u << (p.b - p.a);
         const uint64_t entries = ((uint64_t)all_cosets << p.a) * (S - 1u);
@@ -339,27 +367,19 @@ struct zkb_ctx {
         const uint32_t four = pre && entries * 64 <= cap ? 1u : 0u;
         const uint64_t bytes = entries * (four ? 64 : 16);
         const auto key = std::make_tuple(p.log_n, p.a, p.b, p.coset, p.inverse, p.coset ? p.log_lde : 0u, four);
-        auto it = tw_cache.find(key);
-        if (it == tw_cache.end()) {
-            if (tw_cache_bytes + bytes > ((uint64_t)768 << 20)) {  // a long-lived context that has seen many shapes: start over
-                if (log_tables) fprintf(stderr, "[zkb twiddles] cache of %.2f MiB over budget: cleared\n", tw_cache_bytes / 1048576.0);
-                CK(cudaStreamSynchronize(stream));
-                for (auto& kv : tw_cache) kv.second.release();
-                tw_cache.clear(); tw_cache_bytes = 0;
-            }
-            DevBuf& b = tw_cache[key];
-            b.ensure(bytes);
-            tw_cache_bytes += bytes;
+        DevBuf* tab = tw_cache.find(key);
+        if (!tab) {
+            if (log_tables && tw_cache.full(bytes)) fprintf(stderr, "[zkb twiddles] cache of %.2f MiB over budget: cleared\n", tw_cache.bytes / 1048576.0);
+            tab = &tw_cache.insert(key, bytes, stream);
             if (log_tables)
                 fprintf(stderr, "[zkb twiddles] log_n %u layers [%u, %u) coset %u inverse %u cj %u: %s table %.2f MiB, cache %.2f MiB\n", p.log_n, p.a,
-                        p.b, p.coset, p.inverse, p.cj, four ? "four-copy" : "plain", bytes / 1048576.0, tw_cache_bytes / 1048576.0);
+                        p.b, p.coset, p.inverse, p.cj, four ? "four-copy" : "plain", bytes / 1048576.0, tw_cache.bytes / 1048576.0);
             NttPass q = p;
             q.n_cosets = all_cosets; q.coset0 = 0; q.tw_four = four;
-            k_build_twiddles<<<(unsigned)((entries + 255) / 256), 256, 0, stream>>>(q, b.as<fe>());
+            k_build_twiddles<<<(unsigned)((entries + 255) / 256), 256, 0, stream>>>(q, tab->as<fe>());
             check_launch();
-            it = tw_cache.find(key);
         }
-        p.tw_tab = it->second.as<fe>(); p.tw_four = four;
+        p.tw_tab = tab->as<fe>(); p.tw_four = four;
     }
     void launch_pass(NttPass p) {
         const uint32_t S = 1u << (p.b - p.a);
@@ -540,6 +560,15 @@ struct zkb_ctx {
         stage = ST_BEGUN;
     }
 
+    // staged API: a commitment's root, downloaded from `d_root`, joins the proof and the transcript slot `ts_root`
+    void take_root(const uint32_t* d_root, uint8_t ts_root[32], uint8_t* root_out) {
+        Digest32 root;
+        d2h(root.b, d_root, 32);
+        parts.commitments.push_back(root);
+        memcpy(ts_root, root.b, 32);
+        if (root_out) memcpy(root_out, root.b, 32);
+    }
+
     // K1-K4.  The trace is committed column group by column group (16 columns): [H2D] -> transpose -> inverse NTT ->
     // coset LDE.  Column groups are independent until the rows are hashed, so the host-to-device copy of group g+1
     // (copy stream) overlaps the transforms of group g, and a group's polynomials (n*16 elements) stay L2-resident
@@ -549,11 +578,7 @@ struct zkb_ctx {
     // that every launch still fills > 25 waves of resident blocks.
     void trace_commit(const uint8_t* const* host_cols, const fe* d_src, uint8_t root_out[32]) {
         trace_commit_dev(host_cols, d_src);
-        Digest32 root;
-        d2h(root.b, d_tree.as<uint32_t>() + 8, 32);
-        parts.commitments.push_back(root);
-        memcpy(ts.trace_root, root.b, 32);
-        if (root_out) memcpy(root_out, root.b, 32);
+        take_root(d_tree.as<uint32_t>() + 8, ts.trace_root, root_out);
     }
     // leaves the root at d_tree + 8 words
     void trace_commit_dev(const uint8_t* const* host_cols, const fe* d_src) {
@@ -576,12 +601,8 @@ struct zkb_ctx {
             CK(cudaStreamWaitEvent(copy_stream, ev_group[16], 0));
             if (ngroups > 16) throw InvalidArg("too many column groups");
             for (uint32_t g = 0; g < ngroups; g++) {
-                const uint32_t c0 = groups[g].first, wc = groups[g].second;
-                bool contiguous = true;
-                for (uint32_t j = 1; j < wc; j++) if (host_cols[c0 + j] != host_cols[c0] + (size_t)j * n * 16) contiguous = false;
-                uint8_t* dst = d_trace.as<uint8_t>() + (size_t)c0 * n * 16;
-                if (contiguous) CK(cudaMemcpyAsync(dst, host_cols[c0], (size_t)wc * n * 16, cudaMemcpyHostToDevice, copy_stream));
-                else for (uint32_t j = 0; j < wc; j++) CK(cudaMemcpyAsync(dst + (size_t)j * n * 16, host_cols[c0 + j], n * 16, cudaMemcpyHostToDevice, copy_stream));
+                const uint32_t c0 = groups[g].first;
+                copy_cols(host_cols + c0, groups[g].second, n, d_trace.as<uint8_t>() + (size_t)c0 * n * 16, copy_stream);
                 CK(cudaEventRecord(ev_group[g], copy_stream));
             }
             d_src = d_trace.as<fe>();
@@ -625,13 +646,19 @@ struct zkb_ctx {
         if (!cols) throw InvalidArg("null trace columns");
         trace_commit(cols, nullptr, root_out);
     }
+    // host columns cols[0 .. w) of n elements into the column-major `dst`: one copy when they are contiguous in host memory
+    static void copy_cols(const uint8_t* const* cols, uint32_t w, uint64_t n, uint8_t* dst, cudaStream_t st) {
+        const size_t cb = (size_t)n * 16;
+        bool contiguous = true;
+        for (uint32_t j = 1; j < w; j++) if (cols[j] != cols[0] + j * cb) contiguous = false;
+        if (contiguous) CK(cudaMemcpyAsync(dst, cols[0], w * cb, cudaMemcpyHostToDevice, st));
+        else for (uint32_t j = 0; j < w; j++) CK(cudaMemcpyAsync(dst + j * cb, cols[j], cb, cudaMemcpyHostToDevice, st));
+    }
     const fe* upload_cols(const uint8_t* const* cols, uint32_t w, uint64_t n, DevBuf& dst) {
         if (!cols) throw InvalidArg("null trace columns");
+        for (uint32_t j = 0; j < w; j++) if (!cols[j]) throw InvalidArg("null trace column");
         dst.ensure((size_t)w * n * 16);
-        bool contiguous = true;
-        for (uint32_t j = 0; j < w; j++) { if (!cols[j]) throw InvalidArg("null trace column"); if (cols[j] != cols[0] + (size_t)j * n * 16) contiguous = false; }
-        if (contiguous) h2d(dst.p, cols[0], (size_t)w * n * 16);
-        else for (uint32_t j = 0; j < w; j++) h2d((uint8_t*)dst.p + (size_t)j * n * 16, cols[j], n * 16);
+        copy_cols(cols, w, n, dst.as<uint8_t>(), stream);
         return dst.as<fe>();
     }
 
@@ -773,7 +800,8 @@ struct zkb_ctx {
         // divisor table of the shape (k_build_divisors): cached until the trace length, the ce blowup or the assertion steps change
         std::vector<uint64_t> dkey{n, ce};
         dkey.insert(dkey.end(), gsteps.begin(), gsteps.end());
-        const bool build_div = div_cache.find(dkey) == div_cache.end();
+        DevBuf* divbuf = div_cache.find(dkey);
+        const bool build_div = !divbuf;
         // 1/(x^n - 1) on the cosets used by the ce domain: x^n = 3^n * w_beta^k, k = kc * beta/ce   (input of the table build only)
         std::vector<HF> zinv(ce);
         if (build_div) {
@@ -800,23 +828,12 @@ struct zkb_ctx {
         if (nl) { memcpy(&pack[off_col], acol.data(), (size_t)nl * 4); memcpy(&pack[off_sel], asel.data(), (size_t)nl * 4); }
         // shape-only data: uploaded once per distinct content and kept (a captured graph of that shape keeps reading it), never
         // per proof and never inside a graph capture
-        DevBuf* packbuf;
-        {
-            const std::string pk((const char*)pack.data(), pack.size());
-            auto it = pack_cache.find(pk);
-            if (it == pack_cache.end()) {
-                if (capturing) throw StateError("evaluator tables changed during a graph capture");
-                if (pack_cache_bytes + total > ((size_t)64 << 20)) {
-                    CK(cudaStreamSynchronize(stream));
-                    for (auto& kv : pack_cache) kv.second.release();
-                    pack_cache.clear(); pack_cache_bytes = 0;
-                }
-                DevBuf& b = pack_cache[pk];
-                b.ensure(total);
-                pack_cache_bytes += total;
-                h2d_small(b.p, pack.data(), total);
-                packbuf = &b;
-            } else packbuf = &it->second;
+        const std::string pk((const char*)pack.data(), pack.size());
+        DevBuf* packbuf = pack_cache.find(pk);
+        if (!packbuf) {
+            if (capturing) throw StateError("evaluator tables changed during a graph capture");
+            packbuf = &pack_cache.insert(pk, total, stream);
+            h2d_small(packbuf->p, pack.data(), total);
         }
         uint8_t* base = packbuf->as<uint8_t>();
         const fe* coef = fs_fe(fs.o_coef);
@@ -825,34 +842,23 @@ struct zkb_ctx {
         p.a_col = (const uint32_t*)(base + off_col); p.a_sel = (const uint32_t*)(base + off_sel);
         p.per_mask = per.empty() ? 0 : (uint32_t)per.size() - 1;
         p.out = out;
-        {
-            auto it = div_cache.find(dkey);
-            if (it == div_cache.end()) {
-                if (capturing) throw StateError("divisor table changed during a graph capture");
-                const size_t bytes = (size_t)(ng + 1) * n * ce * 16;
-                if (div_cache_bytes + bytes > ((size_t)2 << 30) && !div_cache.empty()) {   // long-lived context, many shapes: start over
-                    CK(cudaStreamSynchronize(stream));
-                    for (auto& kv : div_cache) kv.second.release();
-                    div_cache.clear(); div_cache_bytes = 0;
-                }
-                DevBuf& tab = div_cache[dkey];
-                tab.ensure(bytes);
-                div_cache_bytes += bytes;
-                d_aux.ensure(ce * 16);
-                h2d_small(d_aux.p, zinv.data(), ce * 16);
-                DivParams dp{};
-                dp.log_cen = log_n + log_ce; dp.log_ce = log_ce; dp.n_groups = ng;
-                for (uint32_t gi = 0; gi < ng; gi++) dp.g_point[gi] = to_fe(g.pow((u128)gsteps[gi]));
-                dp.g_last = to_fe(g.pow((u128)(n - 1)));
-                dp.zinv = d_aux.as<fe>();
-                dp.roots = roots; dp.log_tab = log_tab;
-                dp.out = tab.as<fe>();
-                const uint64_t threads = (n * ce) / ZKB_DIV_RPT;
-                k_build_divisors<<<(unsigned)((threads + 127) / 128), 128, 0, stream>>>(dp);
-                check_launch();
-                p.div = tab.as<fe>();
-            } else p.div = it->second.as<fe>();
+        if (build_div) {
+            if (capturing) throw StateError("divisor table changed during a graph capture");
+            divbuf = &div_cache.insert(dkey, (size_t)(ng + 1) * n * ce * 16, stream);
+            d_aux.ensure(ce * 16);
+            h2d_small(d_aux.p, zinv.data(), ce * 16);
+            DivParams dp{};
+            dp.log_cen = log_n + log_ce; dp.log_ce = log_ce; dp.n_groups = ng;
+            for (uint32_t gi = 0; gi < ng; gi++) dp.g_point[gi] = to_fe(g.pow((u128)gsteps[gi]));
+            dp.g_last = to_fe(g.pow((u128)(n - 1)));
+            dp.zinv = d_aux.as<fe>();
+            dp.roots = roots; dp.log_tab = log_tab;
+            dp.out = divbuf->as<fe>();
+            const uint64_t threads = (n * ce) / ZKB_DIV_RPT;
+            k_build_divisors<<<(unsigned)((threads + 127) / 128), 128, 0, stream>>>(dp);
+            check_launch();
         }
+        p.div = divbuf->as<fe>();
         // Boundary numerators.  Per-point sums cost nl multiplications at each of the ce*n points; combining the asserted
         // columns in coefficient space (nl per coefficient row) and extending the ng combined polynomials once costs
         // nl*n + ng * ce*n * (log2(n)/2 + ~6).  MiMC on one GPU (128 assertions, ce = 8) is 2.7x cheaper that way; the training
@@ -978,15 +984,11 @@ struct zkb_ctx {
     }
     void constraints_commit(uint8_t root_out[32]) {
         constraints_commit_dev();
-        Digest32 root;
         uint32_t bad_degree = 0;
         CK(cudaMemcpyAsync(&bad_degree, d_flags.p, 4, cudaMemcpyDeviceToHost, stream));
-        d2h(root.b, d_comp_tree.as<uint32_t>() + 8, 32);
+        take_root(d_comp_tree.as<uint32_t>() + 8, ts.constraint_root, root_out);
         // as the oracle (and a release build of Winterfell) the proof is still produced; it will not verify
         if (bad_degree) ts.comp_degree_ok = 0;
-        parts.commitments.push_back(root);
-        memcpy(ts.constraint_root, root.b, 32);
-        if (root_out) memcpy(root_out, root.b, 32);
     }
 
     // K7.  Trace polynomials are held per rank for its own columns (all of them on one GPU); a column-sharded proof
@@ -1134,11 +1136,7 @@ struct zkb_ctx {
     }
     void fri_commit_layer(uint8_t root_out[32]) {
         fri_commit_layer_dev();
-        Digest32 root;
-        d2h(root.b, d_fri_tree[fri_layer].as<uint32_t>() + 8, 32);
-        parts.commitments.push_back(root);
-        memcpy(ts.fri_roots[fri_layer], root.b, 32);
-        if (root_out) memcpy(root_out, root.b, 32);
+        take_root(d_fri_tree[fri_layer].as<uint32_t>() + 8, ts.fri_roots[fri_layer], root_out);
     }
     // the folding challenge is dts()->fri_alpha[fri_layer]
     void fri_fold_dev() {
@@ -1181,38 +1179,32 @@ struct zkb_ctx {
         check_launch();
         stage = ST_FRI_DONE;
     }
-    void fri_remainder(Digest32* commitment) {
+    void fri_remainder(uint8_t commitment_out[32]) {
         fri_remainder_dev(false);
         const uint32_t rs = (uint32_t)(fri_domain(fri_layer) / air.blowup);
         parts.remainder.assign(rs, HF());
         CK(cudaMemcpyAsync(parts.remainder.data(), fs_fe(fs.o_rem), (size_t)rs * 16, cudaMemcpyDeviceToHost, stream));
-        Digest32 d;
-        d2h(d.b, dts()->rem_commit, 32);
-        parts.commitments.push_back(d);
-        memcpy(ts.remainder_commitment, d.b, 32);
-        if (commitment) *commitment = d;
+        take_root(dts()->rem_commit, ts.remainder_commitment, commitment_out);
     }
 
-    // K10
+    // K10: the smallest nonce >= 1 for `t->seed` into t->nonce, which must hold ~0; it stays ~0 when there is none up to 2^44
+    void enqueue_grind(DevTs* t, uint32_t bits) {
+        k_fs_grind<<<(unsigned)sm_count * 8, 256, 0, stream>>>(t, bits, 1ull << 44);
+        check_launch();
+    }
+    // staged zkb_grind: a scratch transcript, so that the proof's own (d_fs) stays untouched
     uint64_t grind(const uint8_t seed[32], uint32_t bits) {
         if (bits > 32) throw InvalidArg("grinding factor must be <= 32");
-        d_gather.ensure(4096);
-        uint32_t* d_seed = d_gather.as<uint32_t>();
-        unsigned long long* d_found = reinterpret_cast<unsigned long long*>(d_gather.as<uint8_t>() + 64);
-        h2d_small(d_seed, seed, 32);
-        unsigned long long init = ~0ull;
-        h2d_small(d_found, &init, 8);
-        uint64_t base = 1;
-        const uint64_t window = (uint64_t)1 << 22;
-        for (;;) {
-            k_grind<<<(unsigned)(window / 256), 256, 0, stream>>>(d_seed, base, window, bits, d_found);
-            check_launch();
-            unsigned long long f;
-            d2h(&f, d_found, 8);
-            if (f != ~0ull) return f;
-            base += window;
-            if (base > ((uint64_t)1 << 44)) throw std::runtime_error("proof-of-work nonce not found");
-        }
+        d_gather.ensure(sizeof(DevTs));
+        DevTs* t = d_gather.as<DevTs>();
+        const unsigned long long none = ~0ull;
+        h2d_small(t->seed, seed, 32);
+        h2d_small(&t->nonce, &none, 8);
+        enqueue_grind(t, bits);
+        unsigned long long nonce;
+        d2h(&nonce, &t->nonce, 8);
+        if (nonce == ~0ull) throw std::runtime_error("proof-of-work nonce not found");
+        return nonce;
     }
 
     // K11 (TraceLde::query, ConstraintCommitment::query, FriProver::build_proof): rows and full authentication paths of
@@ -1389,10 +1381,7 @@ struct zkb_ctx {
         t_end(TS_FRI);
         t_begin(TS_GRIND);
         if (force_nonce) { const unsigned long long v = force_nonce; h2d_small(&dts()->nonce, &v, 8); }
-        else {                                                         // grind_query_seed
-            k_fs_grind<<<(unsigned)sm_count * 8, 256, 0, stream>>>(dts(), air.grinding, 1ull << 44);
-            check_launch();
-        }
+        else enqueue_grind(dts(), air.grinding);                       // grind_query_seed
         t_end(TS_GRIND);
         t_begin(TS_QUERY);
         k_fs_positions<<<1, ZKB_FS_THREADS, 0, stream>>>(dts(), air.num_queries, (uint32_t)(air.lde_size() - 1));   // get_query_positions
@@ -1507,6 +1496,15 @@ static uint8_t* dup_bytes(const std::vector<uint8_t>& v) {
     return p;
 }
 
+// the proving entry points: Prover::prove, then the proof bytes (malloc'ed, released with zkb_free) and the transcript out
+static void prove_out(zkb_ctx* ctx, const zkb_air_desc* air, const uint8_t* const* cols, const void* d_trace, uint64_t force_nonce, bool sharded,
+                      uint8_t** proof_out, uint64_t* proof_len, zkb_transcript* transcript) {
+    std::vector<uint8_t> b = ctx->prove(air, cols, (const fe*)d_trace, force_nonce, sharded);
+    if (transcript) *transcript = ctx->ts;
+    if (proof_len) *proof_len = b.size();
+    if (proof_out) *proof_out = dup_bytes(b);
+}
+
 extern "C" {
 
 int32_t zkb_ctx_create(int32_t device, void* stream, zkb_ctx** out) {
@@ -1553,20 +1551,14 @@ int32_t zkb_prove(zkb_ctx* ctx, const zkb_air_desc* air, const uint8_t* const* c
                   uint64_t* proof_len, zkb_transcript* transcript) {
     return guarded(ctx, [&] {
         if (!cols) throw InvalidArg("null trace columns");
-        std::vector<uint8_t> b = ctx->prove(air, cols, nullptr, force_nonce);
-        if (transcript) *transcript = ctx->ts;
-        if (proof_len) *proof_len = b.size();
-        if (proof_out) *proof_out = dup_bytes(b);
+        prove_out(ctx, air, cols, nullptr, force_nonce, false, proof_out, proof_len, transcript);
     });
 }
 int32_t zkb_prove_device(zkb_ctx* ctx, const zkb_air_desc* air, const void* d_trace, uint64_t force_nonce, uint8_t** proof_out,
                          uint64_t* proof_len, zkb_transcript* transcript) {
     return guarded(ctx, [&] {
         if (!d_trace) throw InvalidArg("null device trace");
-        std::vector<uint8_t> b = ctx->prove(air, nullptr, (const fe*)d_trace, force_nonce);
-        if (transcript) *transcript = ctx->ts;
-        if (proof_len) *proof_len = b.size();
-        if (proof_out) *proof_out = dup_bytes(b);
+        prove_out(ctx, air, nullptr, d_trace, force_nonce, false, proof_out, proof_len, transcript);
     });
 }
 
@@ -1660,11 +1652,9 @@ int32_t zkb_fri_fold(zkb_ctx* ctx, const uint8_t a[16]) {
 }
 int32_t zkb_fri_remainder(zkb_ctx* ctx, uint8_t* coeffs_out, uint64_t* n_out, uint8_t commitment_out[32]) {
     return guarded(ctx, [&] {
-        Digest32 d;
-        ctx->fri_remainder(&d);
+        ctx->fri_remainder(commitment_out);
         if (coeffs_out) memcpy(coeffs_out, ctx->parts.remainder.data(), ctx->parts.remainder.size() * 16);
         if (n_out) *n_out = ctx->parts.remainder.size();
-        if (commitment_out) memcpy(commitment_out, d.b, 32);
     });
 }
 int32_t zkb_grind(zkb_ctx* ctx, const uint8_t seed[32], uint32_t bits, uint64_t* nonce_out) {
@@ -1706,20 +1696,14 @@ int32_t zkb_mg_prove(zkb_ctx* ctx, const zkb_air_desc* air, const uint8_t* const
                      uint64_t* proof_len, zkb_transcript* transcript) {
     return guarded(ctx, [&] {
         if (!local_cols) throw InvalidArg("null trace columns");
-        std::vector<uint8_t> b = ctx->prove(air, local_cols, nullptr, force_nonce, true);
-        if (transcript) *transcript = ctx->ts;
-        if (proof_len) *proof_len = b.size();
-        if (proof_out) *proof_out = dup_bytes(b);
+        prove_out(ctx, air, local_cols, nullptr, force_nonce, true, proof_out, proof_len, transcript);
     });
 }
 int32_t zkb_mg_prove_device(zkb_ctx* ctx, const zkb_air_desc* air, const void* d_local_trace, uint64_t force_nonce, uint8_t** proof_out,
                             uint64_t* proof_len, zkb_transcript* transcript) {
     return guarded(ctx, [&] {
         if (!d_local_trace) throw InvalidArg("null device trace");
-        std::vector<uint8_t> b = ctx->prove(air, nullptr, (const fe*)d_local_trace, force_nonce, true);
-        if (transcript) *transcript = ctx->ts;
-        if (proof_len) *proof_len = b.size();
-        if (proof_out) *proof_out = dup_bytes(b);
+        prove_out(ctx, air, nullptr, d_local_trace, force_nonce, true, proof_out, proof_len, transcript);
     });
 }
 
