@@ -44,7 +44,8 @@ typedef enum {
 
 /*
  * Everything `Prover::prove` derives from (Air, ProofOptions, PublicInputs):
- *   options       winterfell::ProofOptions::new argument order, src/main.rs:98-107
+ *   options       winterfell::ProofOptions::new argument order, src/main.rs:98-107; folding (the FRI folding factor) is one of
+ *                 2, 4, 8, 16, as ProofOptions::new accepts; any other value is ZKB_ERR_INVALID
  *   pub_elems     PublicInputs::to_elements(): src/training/air.rs:70-94, src/aggregation/air.rs:57-81
  *   assertions    Air::get_assertions(): src/training/air.rs:130-151, src/aggregation/air.rs:121-147
  *   params        aggregation: the scaling factor k (src/aggregation/air.rs:108);
@@ -65,7 +66,9 @@ typedef struct {
     uint64_t n_params;
 } zkb_air_desc;
 
-/* Fiat-Shamir transcript of one proof, exported for stage-by-stage parity checks */
+/* Fiat-Shamir transcript of one proof, exported for stage-by-stage parity checks.
+ * n_fri_layers is the proof's true number of FRI layers; fri_roots / fri_alphas hold the first min(n_fri_layers, 16) of them
+ * (a small folding factor can need more than 16 layers, up to 29 at folding 2).  The proof bytes carry every layer. */
 typedef struct {
     uint8_t trace_root[32], constraint_root[32], remainder_commitment[32];
     uint8_t constraint_alpha[16], z[16], deep_alpha[16];

@@ -149,6 +149,8 @@ impl AirDescriptor {
             params,
         }
     }
+    /// The options pass through unchanged: the library proves every FRI folding factor `ProofOptions::new` accepts
+    /// (2, 4, 8 and 16) and returns `ZKB_ERR_INVALID` for options it does not support.
     fn as_ffi(&self) -> ffi::zkb_air_desc {
         let o = &self.options;
         ffi::zkb_air_desc {

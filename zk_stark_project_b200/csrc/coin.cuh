@@ -13,14 +13,17 @@
 namespace zkb {
 
 #define ZKB_FS_THREADS 256
+// FRI layers a proof may have: folding by 2 down to a remainder of at least the blowup (>= 2) from the largest LDE domain
+// (2^30) takes 29
+#define ZKB_MAX_FRI_LAYERS 32
 
 // Transcript of the proof in flight, in device memory; the host receives it with the final download.
 struct DevTs {
     uint32_t seed[8];                 // coin state (the counter restarts at every reseed, so it is not kept)
     uint32_t trace_root[8], constraint_root[8], rem_commit[8];
-    uint32_t fri_roots[16][8];
+    uint32_t fri_roots[ZKB_MAX_FRI_LAYERS][8];
     fe alpha, z, zg, zR, zgR, deep_alpha, az, abz, azg;   // zR = z^64, zgR = (z g)^64
-    fe fri_alpha[16];
+    fe fri_alpha[ZKB_MAX_FRI_LAYERS];
     unsigned long long nonce;
     uint32_t bad_degree, coin_failed;
     uint32_t positions[256];          // raw query draws: unsorted, duplicates kept (the host sorts and dedups)

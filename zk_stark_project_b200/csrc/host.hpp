@@ -40,6 +40,8 @@ struct AirSpec {
         return c < 1 ? 1 : (uint32_t)c;
     }
     uint64_t lde_size() const { return n * blowup; }
+    // every FRI size (layer domain, rows per layer, leaf width, position folding) derives from this
+    uint32_t log_folding() const { return log2u(folding); }
     uint32_t num_fri_layers() const {                                                          // [A.10]
         uint64_t d = lde_size(), max_rem = (uint64_t)(rem_max_degree + 1) * blowup;
         uint32_t r = 0;
@@ -58,7 +60,8 @@ struct AirSpec {
         if (a.w < 1 || a.w > 255) throw InvalidArg("trace width must be in 1..=255");
         if (!is_pow2(a.blowup) || a.blowup < 2 || a.blowup > 128) throw InvalidArg("blowup factor must be a power of two in 2..=128");
         if (a.blowup < a.ce_blowup()) throw InvalidArg("blowup factor too small for the constraint degree");
-        if (a.folding != 16) throw InvalidArg("only FRI folding factor 16 is supported (src/main.rs:103)");
+        if (a.folding != 2 && a.folding != 4 && a.folding != 8 && a.folding != 16)
+            throw InvalidArg("FRI folding factor must be one of 2, 4, 8, 16");
         if (a.num_queries < 1 || a.num_queries > 255) throw InvalidArg("number of queries must be in 1..=255");
         if (a.grinding > 32) throw InvalidArg("grinding factor must be <= 32");
         if (a.rem_max_degree > 255 || ((a.rem_max_degree + 1) & a.rem_max_degree)) throw InvalidArg("bad FRI remainder max degree");

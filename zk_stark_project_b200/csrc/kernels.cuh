@@ -836,49 +836,53 @@ __global__ void __launch_bounds__(128) k_deep_eval(const LdeMat m, const DevTs* 
 }
 
 // ------------------------------------------------------------------------------------------------
-// K9: FRI degree-respecting projection with folding factor 16 (winter-fri folding::apply_drp;
-// folding factor from src/main.rs:103).  next[i] = p_i(alpha), p_i interpolating (x_i w_16^j, e[i + j*rows]),
-// x_i = 3 * w_M^i  — the offset 3 is NOT raised to the 16th power between layers (SURVEY A.10).
+// K9: FRI degree-respecting projection with folding factor F = 2^LOG_F in {2, 4, 8, 16} (winter-fri folding::apply_drp;
+// ProofOptions accepts these four).  next[i] = p_i(alpha), p_i interpolating (x_i w_F^j, e[i + j*rows]), rows = M / F,
+// x_i = 3 * w_M^i  — the offset 3 is NOT raised to the F-th power between layers (SURVEY A.10).
 struct FriFoldParams {
     const fe* in; fe* out;
     uint32_t log_m;            // current domain size M = 2^log_m
     const fe* alpha;           // the layer's folding challenge (device transcript)
-    fe inv3, inv16;
-    fe w16inv[8];              // w_16^{-k}, k = 0..7
+    fe inv3, inv_f;            // 1/3, 1/F
+    fe wf_inv[8];              // w_F^{-k}, k = 0..F/2-1
     PowTab roots; uint32_t log_tab;
 };
-__global__ void __launch_bounds__(128) k_fri_fold16(const FriFoldParams p) {
-    const uint64_t rows = ((uint64_t)1 << p.log_m) >> 4;
+template <int LOG_F>
+__global__ void __launch_bounds__(128) k_fri_fold(const FriFoldParams p) {
+    constexpr int F = 1 << LOG_F;
+    static_assert(LOG_F >= 1 && F / 2 <= (int)(sizeof(p.wf_inv) / sizeof(fe)), "folding factor out of range");
+    const uint64_t rows = ((uint64_t)1 << p.log_m) >> LOG_F;
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= rows) return;
-    fe v[16];
-    // bit-reversed load for an in-register DIT inverse DFT
+    fe v[F];
+    // bit-reversed load for an in-register DIT inverse DFT (__brev folds to a constant per unrolled j; a shift-and-or loop
+    // for the reversal changes the register allocation of the F = 16 instance: 100 registers and 30 more instructions)
 #pragma unroll
-    for (int j = 0; j < 16; j++) {
-        const int br = ((j & 1) << 3) | ((j & 2) << 1) | ((j & 4) >> 1) | ((j & 8) >> 3);
+    for (int j = 0; j < F; j++) {
+        const int br = (int)(__brev((unsigned)j) >> (32 - LOG_F));
         v[br] = fe_load(p.in + i + (uint64_t)j * rows);
     }
 #pragma unroll
-    for (int lam = 1; lam <= 4; lam++) {
+    for (int lam = 1; lam <= LOG_F; lam++) {
         const int half = 1 << (lam - 1);
 #pragma unroll
-        for (int q = 0; q < 8; q++) {
+        for (int q = 0; q < F / 2; q++) {
             const int th = q & (half - 1);
             const int p0 = ((q >> (lam - 1)) << lam) + th;
             fe u = v[p0];
-            fe t = th == 0 ? v[p0 + half] : fe_mul(v[p0 + half], p.w16inv[th * (8 >> (lam - 1))]);
+            fe t = th == 0 ? v[p0 + half] : fe_mul(v[p0 + half], p.wf_inv[th * ((F / 2) >> (lam - 1))]);
             v[p0] = fe_add(u, t);
             v[p0 + half] = fe_sub(u, t);
         }
     }
-    // p(alpha) = (1/16) sum_k c_k (alpha / x_i)^k,  1/x_i = (1/3) w_M^{-i}
+    // p(alpha) = (1/F) sum_k c_k (alpha / x_i)^k,  1/x_i = (1/3) w_M^{-i}
     const uint32_t tab_mask = (1u << p.log_tab) - 1u;
     const uint32_t e = (0u - ((uint32_t)i << (p.log_tab - p.log_m))) & tab_mask;
     const fe t = fe_mul(fe_mul(fe_ldg(p.alpha), p.inv3), powtab(p.roots, e));
-    fe acc = v[15];
+    fe acc = v[F - 1];
 #pragma unroll
-    for (int kq = 14; kq >= 0; kq--) acc = fe_add(fe_mul(acc, t), v[kq]);
-    fe_store(p.out + i, fe_mul(acc, p.inv16));
+    for (int kq = F - 2; kq >= 0; kq--) acc = fe_add(fe_mul(acc, t), v[kq]);
+    fe_store(p.out + i, fe_mul(acc, p.inv_f));
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -894,12 +898,12 @@ __global__ void k_gather_lde_rows(const LdeMat m, const uint32_t* __restrict__ p
 }
 // Openings in ONE launch (blockIdx.y + first = commitment): rows at the raw query positions plus the full authentication path
 // of each, because for small proofs every launch is a measurable part of the latency.  Commitments 0, 1: LDE matrices (trace,
-// constraint composition); 2 + l: FRI layer l, rows [e[p + j*rows]]_{j<16} (folding a position is p mod rows).
+// constraint composition); 2 + l: FRI layer l, rows [e[p + j*rows]]_{j<F} (folding a position is p mod rows).
 // Sharded proofs: an entry this rank does not hold is written as zeros, every other entry is the same on all ranks, so a
 // byte-wise max over the ranks assembles the openings.  Trace rows and the path levels below lsub belong to the rank that owns
 // the queried row (r >> lsub); the levels at or above lsub are read from the replicated cap heap.  A composition row is held
 // by the rank that stores its coset.
-#define ZKB_MAX_OPEN 18
+#define ZKB_MAX_OPEN (2 + ZKB_MAX_FRI_LAYERS)
 struct OpenJobs {
     uint32_t first, q;
     const uint32_t* pos;                 // raw positions (device transcript)
@@ -913,6 +917,7 @@ struct OpenJobs {
     const uint32_t* cap;                 // trace commitment: heap of the top depth - lsub levels (one GPU: lsub = depth)
     uint32_t lsub, rank;                 // trace commitment: log2 rows per rank, this rank
 };
+static_assert(sizeof(OpenJobs) <= 4096, "k_open_all takes OpenJobs by value: it must fit the 4 KiB of kernel parameters");
 __global__ void __launch_bounds__(128) k_open_all(const OpenJobs J) {
     const uint32_t t = blockIdx.y + J.first;
     const uint32_t idx = blockIdx.x * blockDim.x + threadIdx.x;

@@ -509,14 +509,14 @@ struct zkb_ctx {
         h_stage_used = 0;
         coin.init(air.coin_seed());
         fri_layers = air.num_fri_layers();
-        if (fri_layers > 16) throw InvalidArg("too many FRI layers");
+        if (fri_layers > ZKB_MAX_FRI_LAYERS) throw InvalidArg("too many FRI layers");
         fri_layer = 0; fri_committed = false;
         positions.clear();
         mg_active = false;
         {   // device transcript + openings layout (everything is determined by the shape)
             auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
             const uint32_t w = air.w, q = air.num_queries;
-            const uint64_t m_last = air.lde_size() >> (4 * fri_layers);
+            const uint64_t m_last = fri_domain(fri_layers);
             fs = FsLayout();
             fs.o_ood = al(sizeof(DevTs));
             fs.o_rem = fs.o_ood + (2 * (size_t)w + c) * 16;
@@ -529,7 +529,7 @@ struct zkb_ctx {
             };
             add_tree(w, log_N);
             add_tree(c, log_N);
-            for (uint32_t l = 0; l < fri_layers; l++) add_tree(16, log2u(fri_domain(l) / 16));
+            for (uint32_t l = 0; l < fri_layers; l++) add_tree(air.folding, log2u(fri_rows(l)));
             fs.host_bytes = off;
             fs.o_coef = off; off += ((size_t)air.num_transition() + air.assertions.size()) * 16;
             fs.o_gamma = off; off += ((size_t)w + c) * 16;
@@ -1122,35 +1122,46 @@ struct zkb_ctx {
 
     // K9
     const fe* fri_cur_evals() const { return fri_layer == 0 ? d_deep.as<fe>() : d_fri_evals[fri_layer].as<fe>(); }
-    uint64_t fri_domain(uint32_t layer) const { return air.lde_size() >> (4 * layer); }
+    uint64_t fri_domain(uint32_t layer) const { return air.lde_size() >> (air.log_folding() * layer); }
+    uint64_t fri_rows(uint32_t layer) const { return fri_domain(layer) >> air.log_folding(); }   // leaves of layer `layer`
     // leaves the layer's root at d_fri_tree[layer] + 8 words
     void fri_commit_layer_dev() {
         if (stage != ST_DEEP || fri_layer >= fri_layers || fri_committed) throw StateError("zkb_fri_commit_layer: out of order");
-        const uint64_t M = fri_domain(fri_layer), rows = M / 16;
+        const uint64_t rows = fri_rows(fri_layer);
         DevBuf& tree = d_fri_tree[fri_layer];
         tree.ensure(2 * rows * 32);
-        k_hash_strided_rows<<<(unsigned)((rows + 127) / 128), 128, 0, stream>>>(fri_cur_evals(), rows, 16, tree.as<uint32_t>() + rows * 8);
+        k_hash_strided_rows<<<(unsigned)((rows + 127) / 128), 128, 0, stream>>>(fri_cur_evals(), rows, air.folding, tree.as<uint32_t>() + rows * 8);
         check_launch();
         build_merkle(tree.as<uint32_t>(), rows);
         fri_committed = true;
     }
+    // the public transcript keeps the first 16 layers' roots and challenges; the proof carries every layer
+    static constexpr uint32_t TS_FRI_SLOTS = sizeof(zkb_transcript::fri_roots) / sizeof(zkb_transcript::fri_roots[0]);
     void fri_commit_layer(uint8_t root_out[32]) {
         fri_commit_layer_dev();
-        take_root(d_fri_tree[fri_layer].as<uint32_t>() + 8, ts.fri_roots[fri_layer], root_out);
+        uint8_t spare[32];
+        take_root(d_fri_tree[fri_layer].as<uint32_t>() + 8, fri_layer < TS_FRI_SLOTS ? ts.fri_roots[fri_layer] : spare, root_out);
     }
     // the folding challenge is dts()->fri_alpha[fri_layer]
     void fri_fold_dev() {
         if (stage != ST_DEEP || !fri_committed) throw StateError("zkb_fri_fold: commit the layer first");
-        const uint64_t M = fri_domain(fri_layer), rows = M / 16;
+        const uint64_t rows = fri_rows(fri_layer);
         DevBuf& nxt = d_fri_evals[fri_layer + 1];
-        nxt.ensure(rows * 16);
+        nxt.ensure(rows * sizeof(fe));
         FriFoldParams p{};
-        p.in = fri_cur_evals(); p.out = nxt.as<fe>(); p.log_m = log2u(M);
-        p.alpha = &dts()->fri_alpha[fri_layer]; p.inv3 = to_fe(HF::from_u64(3).inv()); p.inv16 = to_fe(HF::from_u64(16).inv());
-        HF wi = HF::root_of_unity(4).inv(), x = HF::raw(1);
-        for (int q = 0; q < 8; q++) { p.w16inv[q] = to_fe(x); x = x * wi; }
+        p.in = fri_cur_evals(); p.out = nxt.as<fe>(); p.log_m = log2u(fri_domain(fri_layer));
+        p.alpha = &dts()->fri_alpha[fri_layer]; p.inv3 = to_fe(HF::from_u64(3).inv()); p.inv_f = to_fe(HF::from_u64(air.folding).inv());
+        HF wi = HF::root_of_unity(air.log_folding()).inv(), x = HF::raw(1);
+        for (uint32_t q = 0; q < air.folding / 2; q++) { p.wf_inv[q] = to_fe(x); x = x * wi; }
         p.roots = roots; p.log_tab = log_tab;
-        k_fri_fold16<<<(unsigned)((rows + 127) / 128), 128, 0, stream>>>(p);
+        const dim3 grid((unsigned)((rows + 127) / 128)), block(128);
+        switch (air.log_folding()) {
+            case 1: k_fri_fold<1><<<grid, block, 0, stream>>>(p); break;
+            case 2: k_fri_fold<2><<<grid, block, 0, stream>>>(p); break;
+            case 3: k_fri_fold<3><<<grid, block, 0, stream>>>(p); break;
+            case 4: k_fri_fold<4><<<grid, block, 0, stream>>>(p); break;
+            default: throw InvalidArg("FRI folding factor must be one of 2, 4, 8, 16");
+        }
         check_launch();
         fri_layer++;
         fri_committed = false;
@@ -1158,7 +1169,7 @@ struct zkb_ctx {
     }
     void fri_fold(const HF& alpha) {
         if (stage != ST_DEEP || !fri_committed) throw StateError("zkb_fri_fold: commit the layer first");
-        alpha.to_bytes(ts.fri_alphas[fri_layer]);
+        if (fri_layer < TS_FRI_SLOTS) alpha.to_bytes(ts.fri_alphas[fri_layer]);
         fs_upload(&dts()->fri_alpha[fri_layer], alpha);
         fri_fold_dev();
     }
@@ -1222,7 +1233,7 @@ struct zkb_ctx {
             else {
                 const uint32_t l = t - 2;
                 J.fri_evals[l] = l == 0 ? d_deep.as<fe>() : d_fri_evals[l].as<fe>();
-                J.fri_rows[l] = fri_domain(l) / 16;
+                J.fri_rows[l] = fri_rows(l);
                 J.heap[t] = d_fri_tree[l].as<uint32_t>();
             }
             items = std::max(items, J.q * tr.width + J.q * tr.depth * 2);
@@ -1237,7 +1248,7 @@ struct zkb_ctx {
         if (np == 0 || np > 255) throw InvalidArg("bad number of query positions");
         if (which >= fs.trees.size()) throw InvalidArg("no such FRI layer");
         const FsTree& tr = fs.trees[which];
-        const uint64_t domain = which < 2 ? air.lde_size() : fri_domain(which - 2) / 16;
+        const uint64_t domain = which < 2 ? air.lde_size() : fri_rows(which - 2);
         for (uint32_t p : pos) if (p >= domain) throw InvalidArg("query position out of range");
         // device scratch: [positions np u32][rows np*width fe][full paths np*depth digests]
         const size_t o_rows = 1024, rb = (size_t)np * tr.width * 16, pb = (size_t)np * tr.depth * 32;
@@ -1408,14 +1419,14 @@ struct zkb_ctx {
         parts.commitments.push_back(dg(h->constraint_root));
         for (uint32_t l = 0; l < fri_layers; l++) {
             parts.commitments.push_back(dg(h->fri_roots[l]));
-            memcpy(ts.fri_roots[l], h->fri_roots[l], 32); memcpy(ts.fri_alphas[l], &h->fri_alpha[l], 16);
+            if (l < TS_FRI_SLOTS) { memcpy(ts.fri_roots[l], h->fri_roots[l], 32); memcpy(ts.fri_alphas[l], &h->fri_alpha[l], 16); }
         }
         parts.commitments.push_back(dg(h->rem_commit));
         const HF* frame = reinterpret_cast<const HF*>(h_out + fs.o_ood);
         parts.ood_trace_interleaved.resize(2 * (size_t)w);   // [T_0(z), T_0(zg), T_1(z), ...]  [A.5]
         for (uint32_t j = 0; j < w; j++) { parts.ood_trace_interleaved[2 * j] = frame[j]; parts.ood_trace_interleaved[2 * j + 1] = frame[w + j]; }
         parts.ood_h.assign(frame + 2 * (size_t)w, frame + 2 * (size_t)w + c);
-        const uint32_t rs = (uint32_t)((air.lde_size() >> (4 * fri_layers)) / air.blowup);
+        const uint32_t rs = (uint32_t)(fri_domain(fri_layers) / air.blowup);
         const HF* rem = reinterpret_cast<const HF*>(h_out + fs.o_rem);
         parts.remainder.assign(rem, rem + rs);
         parts.nonce = h->nonce; ts.pow_nonce = h->nonce;
@@ -1467,8 +1478,8 @@ struct zkb_ctx {
         std::vector<uint32_t> fpos = positions;
         uint64_t dom = air.lde_size();
         for (uint32_t l = 0; l < fri_layers; l++) {
-            fpos = fold_positions(fpos, dom, 16);
-            dom /= 16;
+            fpos = fold_positions(fpos, dom, air.folding);
+            dom /= air.folding;
             open(fs.trees[2 + l], fpos, (uint32_t)(dom - 1), parts.fri_rows[l], parts.fri_paths[l]);
         }
         return serialize_proof(air, parts);

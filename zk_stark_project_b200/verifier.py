@@ -166,7 +166,7 @@ def _fold_positions(positions, domain, folding):
 
 
 def _fold_row(row, x, alpha):
-    """p(alpha) for the degree < 16 polynomial through (x * w_16^j, row[j])."""
+    """p(alpha) for the degree < F polynomial through (x * w_F^j, row[j]), F = len(row) (the folding factor)."""
     f = len(row)
     w_inv = inv(root_of_unity(f.bit_length() - 1))
     finv, t = inv(f), alpha * inv(x) % P
