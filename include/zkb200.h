@@ -95,6 +95,8 @@ void zkb_ctx_destroy(zkb_ctx* ctx);
 const char* zkb_last_error(const zkb_ctx* ctx);
 /* number of kernels the context has launched so far (evidence for bench.py's gpu_launches) */
 uint64_t zkb_kernel_launches(const zkb_ctx* ctx);
+/* host-to-device bytes the context has copied so far (copies replayed from a captured CUDA graph are not counted again) */
+uint64_t zkb_h2d_bytes(const zkb_ctx* ctx);
 int32_t zkb_last_stage_times(const zkb_ctx* ctx, zkb_stage_times* out);
 /* pinned host memory for trace columns (fast H2D); plain malloc'ed memory works too, only slower */
 void* zkb_host_alloc(size_t bytes);
@@ -124,6 +126,42 @@ int32_t zkb_prove_device(zkb_ctx* ctx, const zkb_air_desc* air, const void* d_tr
 int32_t zkb_prove_batch(zkb_ctx* const* lanes, uint32_t n_lanes, const zkb_air_desc* const* airs, const uint8_t* const* const* cols,
                         uint32_t count, uint8_t** proofs_out, uint64_t* lens_out);
 void zkb_free(void* p);
+
+/* ---- winterfell::verify (src/main.rs:251-257, 430-436, 478-484) ------------------------------------------------------
+ * One value per distinct check of winter-verifier's `verify`, in the order it runs them.  A proof gets the first check it fails. */
+typedef enum {
+    ZKB_VERIFY_OK = 0,
+    ZKB_VERIFY_MALFORMED = 1,            /* the bytes are not a proof (deserialization; includes non-canonical field elements) */
+    ZKB_VERIFY_TRACE_INFO = 2,           /* trace width / length differ from the AIR */
+    ZKB_VERIFY_OPTIONS = 3,              /* proof options differ from the AIR's (AcceptableOptions::OptionSet) */
+    ZKB_VERIFY_COMMITMENTS = 4,          /* wrong number of commitments or of FRI layers */
+    ZKB_VERIFY_OOD_FRAME = 5,            /* OOD frame of the wrong shape */
+    ZKB_VERIFY_OOD_CONSISTENCY = 6,      /* constraint evaluations at z do not match the OOD frame */
+    ZKB_VERIFY_POW = 7,                  /* query seed proof-of-work */
+    ZKB_VERIFY_UNIQUE_QUERIES = 8,       /* number of unique query positions */
+    ZKB_VERIFY_TRACE_VALUES = 9,         /* size of the queried trace rows */
+    ZKB_VERIFY_TRACE_MERKLE = 10,        /* trace rows against the trace commitment */
+    ZKB_VERIFY_CONSTRAINT_VALUES = 11,   /* size of the queried constraint rows */
+    ZKB_VERIFY_CONSTRAINT_MERKLE = 12,   /* constraint rows against the constraint commitment */
+    ZKB_VERIFY_FRI_VALUES = 13,          /* size of an FRI layer's queried rows */
+    ZKB_VERIFY_FRI_MERKLE = 14,          /* FRI layer rows against the layer commitment */
+    ZKB_VERIFY_FRI_FOLDING = 15,         /* a DEEP value or a folded value differs from the next layer's */
+    ZKB_VERIFY_FRI_TRUNCATION = 16,      /* FRI degree truncation */
+    ZKB_VERIFY_REMAINDER_DEGREE = 17,    /* remainder longer than its degree bound */
+    ZKB_VERIFY_REMAINDER_COMMITMENT = 18,/* remainder against its commitment */
+    ZKB_VERIFY_REMAINDER_FOLDING = 19    /* last folded values against the remainder polynomial */
+} zkb_verdict;
+
+/* winterfell::verify::<Air, Blake3_256, DefaultRandomCoin, MerkleTree>(proof, pub_inputs, AcceptableOptions::OptionSet([air's options]))
+ * for `count` proofs at once (src/main.rs:251-257, 430-436, 478-484).  verdicts_out[i] = ZKB_VERIFY_OK or the first check proof i
+ * fails, in winter-verifier's order.  A rejected proof is a verdict, not a call failure: the call returns 0 once every proof has
+ * a verdict, and a negative zkb_status only for bad arguments (including an air the prover would reject) or a CUDA failure.
+ * transcripts_out: NULL, or count transcripts (what the verifier re-derived: roots, alpha, z, DEEP and FRI alphas, nonce, positions);
+ * a proof rejected before the first draw gets a zeroed transcript.  count = 0 does nothing.
+ * Every proof is parsed and its lengths checked on the host; the checks run on the context's stream with two host
+ * synchronisations per call (after the channel, after the last check), whatever the batch size. */
+int32_t zkb_verify_batch(zkb_ctx* ctx, const zkb_air_desc* const* airs, const uint8_t* const* proofs, const uint64_t* lens,
+                         uint32_t count, int32_t* verdicts_out, zkb_transcript* transcripts_out);
 
 /* ---- staged surface: the three associated types + the stages inside Prover::prove ------------------------
  * Order: begin -> trace_commit -> constraints_eval -> constraints_commit -> ood_eval -> deep_compose

@@ -52,6 +52,28 @@ pub const ZKB_AIR_ID_TRAINING: u32 = 1;
 pub const ZKB_AIR_ID_AGGREGATION: u32 = 2;
 pub const ZKB_AIR_ID_MIMC: u32 = 3;
 
+/// zkb_verdict: one value per check of winter-verifier's `verify`, in the order it runs them
+pub const ZKB_VERIFY_OK: i32 = 0;
+pub const ZKB_VERIFY_MALFORMED: i32 = 1;
+pub const ZKB_VERIFY_TRACE_INFO: i32 = 2;
+pub const ZKB_VERIFY_OPTIONS: i32 = 3;
+pub const ZKB_VERIFY_COMMITMENTS: i32 = 4;
+pub const ZKB_VERIFY_OOD_FRAME: i32 = 5;
+pub const ZKB_VERIFY_OOD_CONSISTENCY: i32 = 6;
+pub const ZKB_VERIFY_POW: i32 = 7;
+pub const ZKB_VERIFY_UNIQUE_QUERIES: i32 = 8;
+pub const ZKB_VERIFY_TRACE_VALUES: i32 = 9;
+pub const ZKB_VERIFY_TRACE_MERKLE: i32 = 10;
+pub const ZKB_VERIFY_CONSTRAINT_VALUES: i32 = 11;
+pub const ZKB_VERIFY_CONSTRAINT_MERKLE: i32 = 12;
+pub const ZKB_VERIFY_FRI_VALUES: i32 = 13;
+pub const ZKB_VERIFY_FRI_MERKLE: i32 = 14;
+pub const ZKB_VERIFY_FRI_FOLDING: i32 = 15;
+pub const ZKB_VERIFY_FRI_TRUNCATION: i32 = 16;
+pub const ZKB_VERIFY_REMAINDER_DEGREE: i32 = 17;
+pub const ZKB_VERIFY_REMAINDER_COMMITMENT: i32 = 18;
+pub const ZKB_VERIFY_REMAINDER_FOLDING: i32 = 19;
+
 extern "C" {
     pub fn zkb_ctx_create(device: i32, stream: *mut c_void, out: *mut *mut zkb_ctx) -> i32;
     pub fn zkb_ctx_create_lane(device: i32, out: *mut *mut zkb_ctx) -> i32;
@@ -66,6 +88,9 @@ extern "C" {
                             proof_out: *mut *mut u8, proof_len: *mut u64, transcript: *mut zkb_transcript) -> i32;
     pub fn zkb_prove_batch(lanes: *const *mut zkb_ctx, n_lanes: u32, airs: *const *const zkb_air_desc, cols: *const *const *const u8,
                            count: u32, proofs_out: *mut *mut u8, lens_out: *mut u64) -> i32;
+    /// winterfell::verify for `count` proofs; verdicts_out[i] = ZKB_VERIFY_OK (0) or the first zkb_verdict proof i fails
+    pub fn zkb_verify_batch(ctx: *mut zkb_ctx, airs: *const *const zkb_air_desc, proofs: *const *const u8, lens: *const u64, count: u32,
+                            verdicts_out: *mut i32, transcripts_out: *mut zkb_transcript) -> i32;
     /// key32: 32 bytes of ChaCha20 key for the blinding masks, or null = OS entropy (what rand::thread_rng() does)
     pub fn zkb_training_trace_device(ctx: *mut zkb_ctx, raw_rows: *const u8, n_raw: u32, half: u32, n: u64, key32: *const u8,
                                      d_out: *mut *mut c_void, first_row_out: *mut u8, last_row_out: *mut u8) -> i32;

@@ -32,7 +32,7 @@ use winterfell::{
     matrix::ColMatrix,
     Air, Assertion, AuxRandElements, CompositionPoly, CompositionPolyTrace, ConstraintCommitment,
     ConstraintCompositionCoefficients, ConstraintEvaluator, EvaluationFrame, PartitionOptions, Proof, ProofOptions, Prover,
-    ProverError, Queries, StarkDomain, Trace, TraceInfo, TraceLde, TracePolyTable, TraceTable,
+    ProverError, Queries, StarkDomain, Trace, TraceInfo, TraceLde, TracePolyTable, TraceTable, VerifierError,
 };
 
 type H = Blake3_256<Felt>;
@@ -75,6 +75,48 @@ impl GpuContext {
         }
     }
 }
+impl GpuContext {
+    /// `winterfell::verify::<Air, Blake3_256, DefaultRandomCoin, MerkleTree>` for every (proof bytes, AIR) pair in one call
+    /// (`src/main.rs:251-257, 430-436, 478-484`), with `AcceptableOptions::OptionSet([air's options])`.  A rejected proof is an
+    /// `Err` entry; a bad argument or a device failure panics like every other call of this crate (see `check`).
+    pub fn verify_batch(&self, batch: &[(&[u8], &GpuAirDesc)]) -> Vec<Result<(), VerifierError>> {
+        let descs: Vec<ffi::zkb_air_desc> = batch.iter().map(|(_, a)| a.0.as_ffi()).collect();
+        let airs: Vec<*const ffi::zkb_air_desc> = descs.iter().map(|d| d as *const _).collect();
+        let proofs: Vec<*const u8> = batch.iter().map(|(p, _)| p.as_ptr()).collect();
+        let lens: Vec<u64> = batch.iter().map(|(p, _)| p.len() as u64).collect();
+        let mut verdicts = vec![0i32; batch.len()];
+        let rc = unsafe {
+            ffi::zkb_verify_batch(self.raw, airs.as_ptr(), proofs.as_ptr(), lens.as_ptr(), batch.len() as u32, verdicts.as_mut_ptr(),
+                                  ptr::null_mut())
+        };
+        self.check(rc, "zkb_verify_batch");
+        verdicts.into_iter().map(verifier_error).collect()
+    }
+}
+/// zkb_verdict -> winter-verifier 0.12's `VerifierError` (VERIFY-FIRST: variant names recalled from upstream, not compiled here)
+fn verifier_error(v: i32) -> Result<(), VerifierError> {
+    use winterfell::{FriVerifierError as F, VerifierError as V};
+    match v {
+        ffi::ZKB_VERIFY_OK => Ok(()),
+        ffi::ZKB_VERIFY_MALFORMED | ffi::ZKB_VERIFY_TRACE_INFO | ffi::ZKB_VERIFY_COMMITMENTS | ffi::ZKB_VERIFY_OOD_FRAME
+        | ffi::ZKB_VERIFY_TRACE_VALUES | ffi::ZKB_VERIFY_CONSTRAINT_VALUES => {
+            Err(V::ProofDeserializationError(format!("zkb_verdict {v}")))
+        }
+        ffi::ZKB_VERIFY_OPTIONS => Err(V::UnacceptableProofOptions),
+        ffi::ZKB_VERIFY_OOD_CONSISTENCY => Err(V::InconsistentOodConstraintEvaluations),
+        ffi::ZKB_VERIFY_POW => Err(V::QuerySeedProofOfWorkVerificationFailed),
+        ffi::ZKB_VERIFY_UNIQUE_QUERIES => Err(V::ProofDeserializationError("number of unique queries".into())),
+        ffi::ZKB_VERIFY_TRACE_MERKLE => Err(V::TraceQueryDoesNotMatchCommitment),
+        ffi::ZKB_VERIFY_CONSTRAINT_MERKLE => Err(V::ConstraintQueryDoesNotMatchCommitment),
+        ffi::ZKB_VERIFY_FRI_VALUES => Err(V::FriVerificationFailed(F::InvalidLayerValues)),
+        ffi::ZKB_VERIFY_FRI_MERKLE => Err(V::FriVerificationFailed(F::LayerCommitmentMismatch)),
+        ffi::ZKB_VERIFY_FRI_FOLDING => Err(V::FriVerificationFailed(F::InvalidLayerFolding(0))),
+        ffi::ZKB_VERIFY_FRI_TRUNCATION => Err(V::FriVerificationFailed(F::DegreeTruncation(0, 0, 0))),
+        ffi::ZKB_VERIFY_REMAINDER_DEGREE => Err(V::FriVerificationFailed(F::RemainderDegreeMismatch(0))),
+        ffi::ZKB_VERIFY_REMAINDER_COMMITMENT => Err(V::FriVerificationFailed(F::RemainderCommitmentMismatch)),
+        _ => Err(V::FriVerificationFailed(F::InvalidRemainderFolding)),
+    }
+}
 impl Drop for GpuContext {
     fn drop(&mut self) {
         unsafe { ffi::zkb_ctx_destroy(self.raw) }
@@ -114,6 +156,16 @@ fn batching_code(m: winterfell::BatchingMethod) -> u32 {
         winterfell::BatchingMethod::Algebraic => 1,
         #[allow(unreachable_patterns)]
         _ => 2,
+    }
+}
+
+/// The AIR a batch-verified proof is checked against: what `winterfell::verify` receives as the AIR type, the public inputs and
+/// `AcceptableOptions::OptionSet([options])`.  Build `air` the way `verify` does, `A::new(trace_info, pub_inputs, options)` with
+/// the options the caller accepts (src/main.rs:98-107 for the reference's proofs).
+pub struct GpuAirDesc(AirDescriptor);
+impl GpuAirDesc {
+    pub fn new<A: Air<BaseField = Felt>>(air: &A, kind: &GpuAir, pub_inputs: &A::PublicInputs) -> Self {
+        Self(AirDescriptor::new(air, kind, &pub_inputs.to_elements()))
     }
 }
 

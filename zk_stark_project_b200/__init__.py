@@ -9,14 +9,14 @@ from .field import P, Felt, f64_to_felt
 from .options import ProofOptions, FieldExtension, BatchingMethod
 from .trace import TraceTable, DeviceTrace
 from .prover import Proof, Prover, ProverError
-from .verifier import verify, VerifierError
+from .verifier import verify, verify_batch, VerifierError
 from .training import TrainingUpdateProver, TrainingUpdateInputs, TrainingUpdateAir
 from .aggregation import GlobalUpdateProver, GlobalUpdateInputs, GlobalUpdateAir
 from .mimc import MimcProver, MimcInputs, MimcAir, mimc_cipher, mimc_hash_matrix, get_round_constants
 
 __all__ = [
     "P", "Felt", "f64_to_felt", "ProofOptions", "FieldExtension", "BatchingMethod", "TraceTable", "DeviceTrace", "Proof", "Prover",
-    "ProverError", "verify", "VerifierError", "TrainingUpdateProver", "TrainingUpdateInputs", "TrainingUpdateAir", "GlobalUpdateProver",
+    "ProverError", "verify", "verify_batch", "VerifierError", "TrainingUpdateProver", "TrainingUpdateInputs", "TrainingUpdateAir", "GlobalUpdateProver",
     "GlobalUpdateInputs", "GlobalUpdateAir", "MimcProver", "MimcInputs", "MimcAir", "mimc_cipher", "mimc_hash_matrix",
     "get_round_constants",
 ]

@@ -6,7 +6,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libzkb200.so")
 SOURCES = ["zkb200.cu"]
-HEADERS = ["f128.cuh", "blake3.cuh", "kernels.cuh", "host.hpp", "hostfield.hpp", "nccl_loader.hpp", "../../include/zkb200.h"]
+HEADERS = ["f128.cuh", "blake3.cuh", "kernels.cuh", "verify.cuh", "host.hpp", "hostfield.hpp", "nccl_loader.hpp", "../../include/zkb200.h"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-shared",
               "-Xcompiler", "-fPIC", "-diag-suppress", "550"]
 

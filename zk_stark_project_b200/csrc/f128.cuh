@@ -329,7 +329,9 @@ __device__ __forceinline__ fe fe_sqr_n(fe x, int k) {
     for (int i = 0; i < k; i++) x = fe_sqr(x);
     return x;
 }
-__device__ __noinline__ fe fe_inv(const fe& a) {
+// The chain is written once: fe_inv_inline is inlined into its caller (the batch verifier's kernels), fe_inv is the prover's
+// out-of-line call.  Calling fe_inv from more kernels would change how the prover's callers are allocated around the call.
+__device__ __forceinline__ fe fe_inv_inline(const fe& a) {
     const fe e2 = fe_mul(fe_sqr(a), a);
     const fe e4 = fe_mul(fe_sqr_n(e2, 2), e2);
     const fe e8 = fe_mul(fe_sqr_n(e4, 4), e4);
@@ -343,5 +345,6 @@ __device__ __noinline__ fe fe_inv(const fe& a) {
     r = fe_mul(fe_sqr_n(r, 9), e8);          // 0 11111111
     return fe_mul(fe_sqr_n(r, 32), e32);     // 32 ones
 }
+__device__ __noinline__ fe fe_inv(const fe& a) { return fe_inv_inline(a); }
 
 }  // namespace zkb

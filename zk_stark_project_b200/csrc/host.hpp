@@ -214,6 +214,161 @@ static inline std::vector<uint8_t> serialize_proof(const AirSpec& a, const Proof
     return w.buf;
 }
 
+// ---- readers: the inverse of serialize_proof / batch_proof_bytes over untrusted bytes ------------------------------------
+// Every read is bounds-checked before it happens (lengths are compared with what is left, never added to a position first).
+struct ByteReader {
+    const uint8_t* p; size_t n, pos = 0;
+    bool ok = true;
+    ByteReader(const uint8_t* p_, size_t n_) : p(p_), n(n_) {}
+    bool need(size_t k) { if (!ok || k > n - pos) ok = false; return ok; }
+    uint64_t le(size_t k) { if (!need(k)) return 0; uint64_t v = 0; memcpy(&v, p + pos, k); pos += k; return v; }
+    uint8_t u8() { return (uint8_t)le(1); }
+    uint16_t u16() { return (uint16_t)le(2); }
+    uint32_t u32() { return (uint32_t)le(4); }
+    uint64_t u64() { return le(8); }
+    size_t skip(uint64_t k) { const size_t at = pos; if (need(k)) pos += (size_t)k; return at; }   // offset of the skipped bytes
+    uint64_t usize() {  // vint64
+        const uint8_t first = u8();
+        if (!ok) return 0;
+        const int length = first == 0 ? 9 : __builtin_ctz(first) + 1;
+        if (length == 9) return u64();
+        uint64_t enc = first;
+        for (int i = 1; i < length; i++) enc |= (uint64_t)u8() << (8 * i);
+        return enc >> length;
+    }
+};
+static inline bool canonical(const uint8_t* e) { u128 v; memcpy(&v, e, 16); return v < HF::modulus(); }
+
+// Where each section of Proof::to_bytes() lies in the input (byte offsets, lengths in bytes), as serialize_proof writes them
+struct Span { size_t off = 0, len = 0; };
+struct ProofLayout {
+    uint32_t w = 0, log_n = 0;
+    uint8_t opt[8] = {};             // num_queries, blowup, grinding, field extension, folding, remainder degree, batching x2
+    uint32_t n_unique = 0;
+    Span commitments, trace_rows, trace_paths, comp_rows, comp_paths, ood_trace, ood_h, remainder;
+    std::vector<Span> fri_rows, fri_paths;
+    uint64_t nonce = 0;
+    size_t n_commitments() const { return commitments.len / 32; }
+};
+// false: not a proof (the sequential verifier's deserialization error).  The OOD frame and the remainder must be canonical
+// here; queried rows are checked where the verifier reads them.
+static inline bool parse_proof(const uint8_t* b, size_t len, ProofLayout& L) {
+    ByteReader r(b, len);
+    L = ProofLayout();
+    L.w = r.u8();
+    if (r.u8() != 0 || r.u8() != 0) return false;
+    L.log_n = r.u8();
+    if (!r.ok || L.log_n < 3 || L.log_n > 32) return false;
+    if (r.u16() != 0 || r.u8() != 16) return false;
+    { const size_t m = r.skip(16); u128 P = HF::modulus(); if (!r.ok || memcmp(b + m, &P, 16)) return false; }
+    for (auto& o : L.opt) o = r.u8();
+    if (r.u8() != 1 || r.u8() != 1) return false;
+    L.n_unique = r.u8();
+    { const uint16_t cl = r.u16(); if (cl % 32) return false; L.commitments = {r.skip(cl), cl}; }
+    auto vec = [&](Span& s) { const uint64_t k = r.usize(); s = {r.skip(k), (size_t)k}; };
+    vec(L.trace_rows); vec(L.trace_paths); vec(L.comp_rows); vec(L.comp_paths);
+    auto elems = [&](Span& s, size_t bytes) {
+        s = {r.skip(bytes), bytes};
+        if (r.ok) for (size_t i = 0; i < bytes; i += 16) if (!canonical(b + s.off + i)) r.ok = false;
+    };
+    { const uint16_t tl = r.u16(); if (!r.ok || tl < 1 || (tl - 1) % 16 || r.u8() != 2) return false; elems(L.ood_trace, tl - 1u); }
+    if (r.u16() != 0) return false;
+    { const uint16_t el = r.u16(); if (el % 16) return false; elems(L.ood_h, el); }
+    const uint8_t nl = r.u8();
+    L.fri_rows.resize(nl); L.fri_paths.resize(nl);
+    for (uint32_t i = 0; i < nl; i++) {
+        const uint32_t a = r.u32(); L.fri_rows[i] = {r.skip(a), a};
+        const uint32_t c = r.u32(); L.fri_paths[i] = {r.skip(c), c};
+    }
+    { const uint16_t rl = r.u16(); if (rl % 16) return false; elems(L.remainder, rl); }
+    if (r.u8() != 1) return false;
+    L.nonce = r.u64();
+    return r.ok && r.pos == len;
+}
+
+// BatchMerkleProof::read_from: depth and, per vector of `nodes`, the offsets of its digests.  false: not a batch proof.
+struct BatchProofLayout { uint32_t depth = 0; std::vector<std::vector<size_t>> nodes; };
+static inline bool parse_batch_proof(const uint8_t* b, size_t len, BatchProofLayout& L) {
+    ByteReader r(b, len);
+    L = BatchProofLayout();
+    L.depth = r.u8();
+    const uint64_t nv = r.usize();
+    if (!r.ok || nv > len) return false;
+    L.nodes.resize((size_t)nv);
+    for (auto& v : L.nodes) {
+        const uint64_t k = r.usize();
+        if (!r.ok || k > 64) return false;
+        for (uint64_t i = 0; i < k; i++) { const size_t at = r.skip(32); if (!r.ok) return false; v.push_back(at); }
+    }
+    return r.ok && r.pos == len;
+}
+
+// BatchMerkleProof::get_root as a plan of merges, for the device: `leaf_ids[i]` is the digest id of the leaf at indexes[i]
+// (any order), node_ids[i] the ids of the digests of nodes[i].  Every merge gets a fresh id from `next_id` and is appended to
+// jobs[level] (level 0 merges leaves).  Returns false, like get_root, when the proof's structure does not fit the indexes
+// (an index out of range, a duplicate, a missing or surplus node vector, a node vector that runs out); *root_id is the id of
+// the computed root otherwise.  get_root's node map is replaced by one array per level: the nodes a level computes are
+// ascending and distinct, and a node's sibling, when it is computed too, is its neighbour in that array.
+struct MergeJob { uint32_t a, b, out; };
+static inline bool plan_batch_root(uint32_t depth, const std::vector<uint32_t>& indexes, const std::vector<uint32_t>& leaf_ids,
+                                   const std::vector<std::vector<uint32_t>>& node_ids, std::vector<std::vector<MergeJob>>& all_jobs,
+                                   uint32_t& all_next_id, uint32_t* root_id) {
+    if (indexes.empty() || depth < 1 || depth > 32) return false;
+    const uint64_t n = (uint64_t)1 << depth;
+    std::vector<std::pair<uint64_t, uint32_t>> leaf(indexes.size());   // (leaf index, digest id), ascending
+    for (size_t i = 0; i < indexes.size(); i++) {
+        if (indexes[i] >= n) return false;
+        leaf[i] = {indexes[i], leaf_ids[i]};
+    }
+    std::sort(leaf.begin(), leaf.end());
+    size_t pairs = 0;   // distinct (index & ~1): one node vector each
+    for (size_t i = 0; i < leaf.size(); i++) {
+        if (i && leaf[i].first == leaf[i - 1].first) return false;
+        if (!i || (leaf[i].first & ~1ull) != (leaf[i - 1].first & ~1ull)) pairs++;
+    }
+    if (pairs != node_ids.size()) return false;
+    std::vector<std::vector<MergeJob>> jobs(depth);   // appended to all_jobs only if the structure fits
+    uint32_t next_id = all_next_id;
+    std::vector<uint64_t> cur, nxt;                   // heap indices of the nodes computed at a level, ascending
+    std::vector<uint32_t> cur_id, nxt_id;
+    std::vector<size_t> ptr;                          // next unread node of each vector
+    for (size_t i = 0, k = 0; i < leaf.size(); k++) {
+        const uint64_t idx = leaf[i].first & ~1ull;
+        uint32_t l, r;
+        if (leaf[i].first == idx) {
+            l = leaf[i].second;
+            if (i + 1 < leaf.size() && leaf[i + 1].first == idx + 1) { r = leaf[i + 1].second; ptr.push_back(0); i += 2; }
+            else { if (node_ids[k].empty()) return false; r = node_ids[k][0]; ptr.push_back(1); i += 1; }
+        } else {
+            if (node_ids[k].empty()) return false;
+            l = node_ids[k][0]; r = leaf[i].second; ptr.push_back(1); i += 1;
+        }
+        jobs[0].push_back({l, r, next_id});
+        cur.push_back((n + idx) >> 1);
+        cur_id.push_back(next_id++);
+    }
+    for (uint32_t d = 1; d < depth; d++) {
+        nxt.clear(); nxt_id.clear();
+        for (size_t k = 0; k < cur.size(); k++) {
+            const uint64_t node = cur[k], sib = node ^ 1;
+            const uint32_t nd = cur_id[k];
+            uint32_t sd;
+            if (k + 1 < cur.size() && cur[k + 1] == sib) { sd = cur_id[k + 1]; k++; }
+            else { if (node_ids[k].size() <= ptr[k]) return false; sd = node_ids[k][ptr[k]++]; }
+            jobs[d].push_back((node & 1) ? MergeJob{sd, nd, next_id} : MergeJob{nd, sd, next_id});
+            nxt.push_back(node >> 1);
+            nxt_id.push_back(next_id++);
+        }
+        cur.swap(nxt); cur_id.swap(nxt_id);
+    }
+    if (cur.empty() || cur[0] != 1) return false;
+    *root_id = cur_id[0];
+    if (all_jobs.size() < depth) all_jobs.resize(depth);
+    for (uint32_t d = 0; d < depth; d++) all_jobs[d].insert(all_jobs[d].end(), jobs[d].begin(), jobs[d].end());
+    all_next_id = next_id;
+    return true;
+}
+
 // winter-fri fold_positions  [A.10]
 static inline std::vector<uint32_t> fold_positions(const std::vector<uint32_t>& pos, uint64_t domain, uint32_t folding) {
     uint64_t target = domain / folding;

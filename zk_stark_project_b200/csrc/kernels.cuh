@@ -847,20 +847,20 @@ struct FriFoldParams {
     fe wf_inv[8];              // w_F^{-k}, k = 0..F/2-1
     PowTab roots; uint32_t log_tab;
 };
-template <int LOG_F>
-__global__ void __launch_bounds__(128) k_fri_fold(const FriFoldParams p) {
+// One row of the projection, shared by the prover (k_fri_fold) and the verifier (k_v_eval): load(j) = the row's element at
+// x_i w_F^j, wf_inv(k) = w_F^{-k} (k < F/2), alpha_over_x() = alpha / x_i, inv_f = 1/F; store(v) receives p(alpha).  The loads,
+// the twiddles, alpha / x_i and the store are callables so that each kernel keeps its own addressing and the prover's
+// instructions are what they were before the split.
+template <int LOG_F, class Load, class WfInv, class AlphaOverX, class Store>
+__device__ __forceinline__ void fri_fold_row(Load load, WfInv wf_inv, AlphaOverX alpha_over_x, const fe& inv_f, Store store) {
     constexpr int F = 1 << LOG_F;
-    static_assert(LOG_F >= 1 && F / 2 <= (int)(sizeof(p.wf_inv) / sizeof(fe)), "folding factor out of range");
-    const uint64_t rows = ((uint64_t)1 << p.log_m) >> LOG_F;
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= rows) return;
     fe v[F];
     // bit-reversed load for an in-register DIT inverse DFT (__brev folds to a constant per unrolled j; a shift-and-or loop
     // for the reversal changes the register allocation of the F = 16 instance: 100 registers and 30 more instructions)
 #pragma unroll
     for (int j = 0; j < F; j++) {
         const int br = (int)(__brev((unsigned)j) >> (32 - LOG_F));
-        v[br] = fe_load(p.in + i + (uint64_t)j * rows);
+        v[br] = load(j);
     }
 #pragma unroll
     for (int lam = 1; lam <= LOG_F; lam++) {
@@ -870,19 +870,32 @@ __global__ void __launch_bounds__(128) k_fri_fold(const FriFoldParams p) {
             const int th = q & (half - 1);
             const int p0 = ((q >> (lam - 1)) << lam) + th;
             fe u = v[p0];
-            fe t = th == 0 ? v[p0 + half] : fe_mul(v[p0 + half], p.wf_inv[th * ((F / 2) >> (lam - 1))]);
+            fe t = th == 0 ? v[p0 + half] : fe_mul(v[p0 + half], wf_inv(th * ((F / 2) >> (lam - 1))));
             v[p0] = fe_add(u, t);
             v[p0 + half] = fe_sub(u, t);
         }
     }
-    // p(alpha) = (1/F) sum_k c_k (alpha / x_i)^k,  1/x_i = (1/3) w_M^{-i}
-    const uint32_t tab_mask = (1u << p.log_tab) - 1u;
-    const uint32_t e = (0u - ((uint32_t)i << (p.log_tab - p.log_m))) & tab_mask;
-    const fe t = fe_mul(fe_mul(fe_ldg(p.alpha), p.inv3), powtab(p.roots, e));
+    // p(alpha) = (1/F) sum_k c_k (alpha / x_i)^k
+    const fe t = alpha_over_x();
     fe acc = v[F - 1];
 #pragma unroll
     for (int kq = F - 2; kq >= 0; kq--) acc = fe_add(fe_mul(acc, t), v[kq]);
-    fe_store(p.out + i, fe_mul(acc, p.inv_f));
+    store(fe_mul(acc, inv_f));
+}
+template <int LOG_F>
+__global__ void __launch_bounds__(128) k_fri_fold(const FriFoldParams p) {
+    constexpr int F = 1 << LOG_F;
+    static_assert(LOG_F >= 1 && F / 2 <= (int)(sizeof(p.wf_inv) / sizeof(fe)), "folding factor out of range");
+    const uint64_t rows = ((uint64_t)1 << p.log_m) >> LOG_F;
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= rows) return;
+    fe* const out = p.out + i;   // formed before the row fold: this keeps the address arithmetic where the unfactored kernel had it
+    fri_fold_row<LOG_F>([&](int j) { return fe_load(p.in + i + (uint64_t)j * rows); }, [&](int k) { return p.wf_inv[k]; }, [&] {
+        // 1/x_i = (1/3) w_M^{-i}
+        const uint32_t tab_mask = (1u << p.log_tab) - 1u;
+        const uint32_t e = (0u - ((uint32_t)i << (p.log_tab - p.log_m))) & tab_mask;
+        return fe_mul(fe_mul(fe_ldg(p.alpha), p.inv3), powtab(p.roots, e));
+    }, p.inv_f, [&](const fe& r) { fe_store(out, r); });
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -16,10 +16,12 @@
 #include <cstdlib>
 #include <functional>
 #include <map>
+#include <mutex>
 #include <thread>
 #include <tuple>
 #include <memory>
 #include "kernels.cuh"
+#include "verify.cuh"
 #include "host.hpp"
 
 namespace zkb {
@@ -109,6 +111,7 @@ struct zkb_ctx {
     cudaStream_t stream = nullptr;
     std::string err;
     uint64_t launches = 0;
+    uint64_t h2d_bytes = 0;   // host-to-device bytes copied by this context's calls (zkb_h2d_bytes)
     int sm_count = 148;
 
     // ---- per-proof state -------------------------------------------------------------------------------------
@@ -182,6 +185,12 @@ struct zkb_ctx {
     const fe* d_params() const { return d_in.as<fe>() + air.assertions.size(); }
     DevBuf d_lde_rows, d_mg_a, d_mg_b;  // recv view of the LDE; all-gather staging
     DevBuf d_cap;                       // sharded trace commitment: heap of the replicated top log G levels, cap[1] = root
+    // ---- batch verification (csrc/verify.cuh): staging of the parsed proofs, the plan, the channel's draws, computed digests ----
+    DevBuf d_vstage, d_vplan, d_vts, d_vdig;
+    uint8_t* h_vstage = nullptr;        // pinned, grown on demand
+    size_t h_vstage_cap = 0;
+    uint8_t* h_vplan = nullptr;
+    size_t h_vplan_cap = 0;
 
     // ==========================================================================================================
     void count() { launches++; }
@@ -242,7 +251,8 @@ struct zkb_ctx {
         cudaStreamSynchronize(stream);
         for (DevBuf* b : {&d_trace, &d_bufA, &d_bufB, &d_tmp1, &d_tmp2, &d_lde, &d_tree, &d_small, &d_comp_evals, &d_comp_lde, &d_comp_tree,
                           &d_ab, &d_ab_lde, &d_deep, &d_roots_lo, &d_roots_hi, &d_inv3_lo, &d_inv3_hi, &d_pow3, &d_aux, &d_gather, &d_user_trace, &d_flags,
-                          &d_lde_rows, &d_mg_a, &d_mg_b, &d_cap, &d_bnd_coef, &d_bnd_lde, &d_fs, &d_in, &d_rem_coef})
+                          &d_lde_rows, &d_mg_a, &d_mg_b, &d_cap, &d_bnd_coef, &d_bnd_lde, &d_fs, &d_in, &d_rem_coef, &d_vstage, &d_vplan,
+                          &d_vts, &d_vdig})
             b->release();
         if (comm) { g_nccl.CommDestroy(comm); comm = nullptr; }
         for (auto& b : d_fri_evals) b.release();
@@ -254,15 +264,18 @@ struct zkb_ctx {
         if (ev_ok) { for (auto& pr : tev) for (auto& x : pr) cudaEventDestroy(x); for (auto& x : ev_group) cudaEventDestroy(x); cudaStreamDestroy(copy_stream); cudaStreamDestroy(xchg_stream); }
         if (h_stage) cudaFreeHost(h_stage);
         if (h_out) cudaFreeHost(h_out);
+        if (h_vstage) cudaFreeHost(h_vstage);
+        if (h_vplan) cudaFreeHost(h_vplan);
         if (ev_done) cudaEventDestroy(ev_done);
         if (owns_stream && stream) { cudaStreamDestroy(stream); stream = nullptr; }
     }
 
-    void h2d(void* dst, const void* src, size_t bytes) { CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, stream)); }
+    void h2d(void* dst, const void* src, size_t bytes) { CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, stream)); h2d_bytes += bytes; }
     // small upload through the pinned staging area: returns immediately, `src` may be released right away.  The area is
     // rewound at the start of every proof (every proof ends with a stream synchronisation).
     void h2d_small(void* dst, const void* src, size_t bytes) {
         if (bytes == 0) return;
+        h2d_bytes += bytes;
         const size_t need = (bytes + 255) & ~(size_t)255;
         if (h_stage_used + need > h_stage_cap) {  // does not fit: plain (staged by the driver) copy, then wait so `src` can go away
             CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, stream));
@@ -603,6 +616,7 @@ struct zkb_ctx {
             for (uint32_t g = 0; g < ngroups; g++) {
                 const uint32_t c0 = groups[g].first;
                 copy_cols(host_cols + c0, groups[g].second, n, d_trace.as<uint8_t>() + (size_t)c0 * n * 16, copy_stream);
+                h2d_bytes += (size_t)groups[g].second * n * 16;
                 CK(cudaEventRecord(ev_group[g], copy_stream));
             }
             d_src = d_trace.as<fe>();
@@ -659,6 +673,7 @@ struct zkb_ctx {
         for (uint32_t j = 0; j < w; j++) if (!cols[j]) throw InvalidArg("null trace column");
         dst.ensure((size_t)w * n * 16);
         copy_cols(cols, w, n, dst.as<uint8_t>(), stream);
+        h2d_bytes += (size_t)w * n * 16;
         return dst.as<fe>();
     }
 
@@ -1484,6 +1499,381 @@ struct zkb_ctx {
         }
         return serialize_proof(air, parts);
     }
+
+    // ==========================================================================================================
+    // winter-verifier `verify` for a batch (csrc/verify.cuh).  Host: parse every proof and check every length, count and depth
+    // against the AIR before anything that depends on it is uploaded; pack the parsed sections into one pinned staging buffer
+    // (one copy up).  Device: the channel and the OOD check.  Host, after the first synchronisation: positions, position folding
+    // and the Merkle merge plans.  Device: leaves, merges level by level, roots, DEEP and FRI checks.  Second synchronisation:
+    // the verdicts.  Host-found failures and device-found failures are ordinals of the same order; the smaller one wins.
+    struct VItem {
+        AirSpec air;
+        ProofLayout L;
+        uint32_t fail = VO_ACCEPT, nl = 0, c = 0;
+        std::vector<BatchProofLayout> bp;                         // 0 trace, 1 constraint, 2 + l FRI layer l
+        std::vector<std::vector<std::vector<uint32_t>>> node_ids; // digest ids of bp[k].nodes
+        uint64_t o_comm = 0, o_ood = 0, o_h = 0, o_rem = 0, o_trows = 0, o_crows = 0;
+        std::vector<uint64_t> o_fri;
+        std::vector<uint32_t> positions;                          // sorted, unique
+    };
+    static void grow_pinned(uint8_t*& p, size_t& cap, size_t need) {
+        if (need <= cap) return;
+        if (p) cudaFreeHost(p);
+        p = nullptr; cap = 0;
+        CK(cudaHostAlloc((void**)&p, need, cudaHostAllocDefault));
+        cap = need;
+    }
+    static int32_t verdict_of(uint32_t ord) {
+        static const int32_t head[VO_FRI0] = {ZKB_VERIFY_MALFORMED, ZKB_VERIFY_TRACE_INFO, ZKB_VERIFY_OPTIONS, ZKB_VERIFY_COMMITMENTS,
+                                              ZKB_VERIFY_OOD_FRAME, ZKB_VERIFY_OOD_CONSISTENCY, ZKB_VERIFY_POW, ZKB_VERIFY_UNIQUE_QUERIES,
+                                              ZKB_VERIFY_TRACE_VALUES, ZKB_VERIFY_CONSTRAINT_VALUES, ZKB_VERIFY_MALFORMED, ZKB_VERIFY_MALFORMED,
+                                              ZKB_VERIFY_MALFORMED, ZKB_VERIFY_TRACE_MERKLE, ZKB_VERIFY_MALFORMED, ZKB_VERIFY_CONSTRAINT_MERKLE};
+        static const int32_t layer[VO_FRI_STEP] = {ZKB_VERIFY_FRI_VALUES, ZKB_VERIFY_MALFORMED, ZKB_VERIFY_MALFORMED, ZKB_VERIFY_FRI_MERKLE,
+                                                   ZKB_VERIFY_FRI_FOLDING, ZKB_VERIFY_FRI_TRUNCATION};
+        static const int32_t rem[3] = {ZKB_VERIFY_REMAINDER_DEGREE, ZKB_VERIFY_REMAINDER_COMMITMENT, ZKB_VERIFY_REMAINDER_FOLDING};
+        if (ord < VO_FRI0) return head[ord];
+        if (ord < VO_REM) return layer[(ord - VO_FRI0) % VO_FRI_STEP];
+        if (ord < VO_ACCEPT) return rem[ord - VO_REM];
+        return ZKB_VERIFY_OK;
+    }
+
+    // fn(i) for every i < n, on up to one host thread per core when n is large enough to pay for starting them; the first
+    // exception thrown is rethrown once every thread has finished
+    template <class F>
+    static void host_parallel(uint32_t n, F&& fn) {
+        const uint32_t T = n < 16 ? 1u : std::min<uint32_t>(n / 8, std::max(1u, std::thread::hardware_concurrency()));
+        if (T <= 1) { for (uint32_t i = 0; i < n; i++) fn(i); return; }
+        std::vector<std::thread> th;
+        std::exception_ptr err;
+        std::mutex m;
+        for (uint32_t t = 0; t < T; t++)
+            th.emplace_back([&, t] {
+                try { for (uint32_t i = t; i < n; i += T) fn(i); }
+                catch (...) { std::lock_guard<std::mutex> g(m); if (!err) err = std::current_exception(); }
+            });
+        for (auto& x : th) x.join();
+        if (err) std::rethrow_exception(err);
+    }
+    // digest ids a proof's plan gives its own leaves and merges, relocated after every proof is planned
+    static constexpr uint32_t LOCAL_ID = 0x80000000u;
+    struct VPlan {
+        std::vector<VLeafJob> leaves;
+        std::vector<std::vector<MergeJob>> merges;
+        std::vector<VRootJob> roots;
+        std::vector<VEvalJob> evals;
+        uint32_t ids = 0;
+    };
+
+    void verify_batch(const zkb_air_desc* const* airs, const uint8_t* const* proofs, const uint64_t* lens, uint32_t count, int32_t* verdicts,
+                      zkb_transcript* tss) {
+        if (count == 0) return;
+        if (!airs || !proofs || !lens || !verdicts) throw InvalidArg("null argument");
+        CK(cudaSetDevice(device));
+        static const bool host_prof = getenv("ZKB_HOST_PROFILE") != nullptr;   // diagnostics: host phases of a call on stderr
+        const auto hp0 = std::chrono::steady_clock::now();
+        std::vector<VItem> it(count);
+        for (uint32_t i = 0; i < count; i++) if (!proofs[i]) throw InvalidArg("null proof");
+        auto al = [](size_t x) { return (x + 15) & ~(size_t)15; };
+        size_t off = al((size_t)count * 4);               // [verdicts][VProof x count][roots of unity][per proof sections][nodes]
+        const size_t o_proofs = off;
+        off = al(off + (size_t)count * sizeof(VProof));
+        const size_t o_roots = off;
+        off += 41 * 16;
+        // ---- parse: everything the sequential verifier checks before its first draw, and every position-independent check ----
+        host_parallel(count, [&](uint32_t i) {
+            VItem& x = it[i];
+            x.air = AirSpec::from_desc(airs[i]);
+            const AirSpec& a = x.air;
+            const uint8_t* b = proofs[i];
+            auto fail = [&](uint32_t ord) { x.fail = std::min(x.fail, ord); };
+            if (!parse_proof(b, (size_t)lens[i], x.L)) { fail(VO_MALFORMED); return; }
+            ProofLayout& L = x.L;
+            const uint8_t want[8] = {(uint8_t)a.num_queries, (uint8_t)a.blowup, (uint8_t)a.grinding, (uint8_t)a.field_ext, (uint8_t)a.folding,
+                                     (uint8_t)a.rem_max_degree, (uint8_t)a.batch_c, (uint8_t)a.batch_d};
+            x.nl = a.num_fri_layers(); x.c = a.num_comp_cols();
+            if (L.w != a.w || L.log_n != log2u(a.n)) { fail(VO_TRACE_INFO); return; }
+            if (memcmp(L.opt, want, 8)) { fail(VO_OPTIONS); return; }
+            if (L.n_commitments() != 2 + x.nl + 1 || L.fri_rows.size() != x.nl) { fail(VO_COMMITMENTS); return; }
+            if (L.ood_trace.len != 2 * (size_t)a.w * 16 || L.ood_h.len != (size_t)x.c * 16) { fail(VO_OOD_SHAPE); return; }
+            // batch Merkle proofs: read where the verifier reads them
+            x.bp.resize(2 + x.nl);
+            for (uint32_t k = 0; k < 2 + x.nl; k++) {
+                const Span& sp = k == 0 ? L.trace_paths : k == 1 ? L.comp_paths : L.fri_paths[k - 2];
+                const uint32_t ord = k == 0 ? VO_TRACE_PATHS_PARSE : k == 1 ? VO_CONSTRAINT_PATHS_PARSE : VO_FRI0 + VO_FRI_STEP * (k - 2) + VO_FRI_PATHS_PARSE;
+                if (!parse_batch_proof(b + sp.off, sp.len, x.bp[k])) { fail(ord); x.bp[k] = BatchProofLayout(); }
+            }
+            {   // degree bookkeeping of FriVerifier::verify
+                uint64_t md = a.n;
+                for (uint32_t l = 0; l < x.nl; l++) {
+                    if (md % a.folding) fail(VO_FRI0 + VO_FRI_STEP * l + VO_FRI_TRUNCATION);
+                    md /= a.folding;
+                }
+                if (L.remainder.len / 16 > md) fail(VO_REM);
+            }
+        });
+        // staging offsets and the digest ids of the proofs' Merkle nodes, in proof order
+        uint32_t n_nodes = 0;
+        for (uint32_t i = 0; i < count; i++) {
+            VItem& x = it[i];
+            if (x.fail <= VO_OOD_SHAPE) continue;
+            const ProofLayout& L = x.L;
+            x.node_ids.resize(x.bp.size());
+            for (size_t k = 0; k < x.bp.size(); k++)
+                for (auto& v : x.bp[k].nodes) {
+                    std::vector<uint32_t> ids(v.size());
+                    for (auto& d : ids) d = n_nodes++;
+                    x.node_ids[k].push_back(std::move(ids));
+                }
+            auto place = [&](size_t len) { const size_t o = off; off = al(off + len); return (uint64_t)o; };
+            x.o_comm = place(L.commitments.len); x.o_ood = place(L.ood_trace.len); x.o_h = place(L.ood_h.len); x.o_rem = place(L.remainder.len);
+            x.o_trows = place(L.trace_rows.len); x.o_crows = place(L.comp_rows.len);
+            for (uint32_t l = 0; l < x.nl; l++) x.o_fri.push_back(place(L.fri_rows[l].len));
+        }
+        // AIR data of the OOD check, then the nodes
+        std::vector<uint64_t> o_air(count, 0);
+        for (uint32_t i = 0; i < count; i++) {
+            if (it[i].fail <= VO_OOD_SHAPE) continue;
+            const AirSpec& a = it[i].air;
+            o_air[i] = off;
+            off = al(off + a.assertions.size() * 16) ; off = al(off + a.params.size() * 16); off = al(off + a.assertions.size() * 16);
+            off = al(off + a.assertions.size() * 4); off = al(off + (a.assertions.size() + 1) * 4);
+        }
+        const size_t o_nodes = off;
+        const size_t total = off + (size_t)n_nodes * 32;
+        grow_pinned(h_vstage, h_vstage_cap, total);
+        uint8_t* H = h_vstage;
+        VProof* hp = reinterpret_cast<VProof*>(H + o_proofs);
+        {
+            HF* r = reinterpret_cast<HF*>(H + o_roots);
+            for (int k = 0; k <= 40; k++) r[k] = HF::root_of_unity(k);
+        }
+        if (n_nodes >= LOCAL_ID) throw InvalidArg("too many Merkle nodes in one batch");
+        host_parallel(count, [&](uint32_t i) {   // every proof writes its own parts of the staging buffer
+            VItem& x = it[i];
+            reinterpret_cast<uint32_t*>(H)[i] = x.fail;
+            VProof& p = hp[i];
+            memset(&p, 0, sizeof(p));
+            if (x.fail <= VO_OOD_SHAPE) return;   // not a proof of this AIR: no device work
+            const AirSpec& a = x.air;
+            const ProofLayout& L = x.L;
+            const uint8_t* b = proofs[i];
+            auto put = [&](uint64_t o, const Span& s) { memcpy(H + o, b + s.off, s.len); };
+            put(x.o_comm, L.commitments); put(x.o_ood, L.ood_trace); put(x.o_h, L.ood_h); put(x.o_rem, L.remainder);
+            put(x.o_trows, L.trace_rows); put(x.o_crows, L.comp_rows);
+            for (uint32_t l = 0; l < x.nl; l++) put(x.o_fri[l], L.fri_rows[l]);
+            for (uint32_t k = 0; k < x.bp.size(); k++) {
+                const Span& sp = k == 0 ? L.trace_paths : k == 1 ? L.comp_paths : L.fri_paths[k - 2];
+                for (size_t v = 0; v < x.bp[k].nodes.size(); v++)
+                    for (size_t q = 0; q < x.bp[k].nodes[v].size(); q++)
+                        memcpy(H + o_nodes + (size_t)x.node_ids[k][v][q] * 32, b + sp.off + x.bp[k].nodes[v][q], 32);
+            }
+            HostCoin coin;
+            coin.init(a.coin_seed());
+            memcpy(p.seed, coin.seed, 32);
+            p.o_comm = x.o_comm; p.o_ood = x.o_ood; p.o_h = x.o_h; p.o_rem = x.o_rem;
+            p.nonce = L.nonce;
+            p.w = a.w; p.c = x.c; p.nt = a.num_transition(); p.na = (uint32_t)a.assertions.size(); p.np = (uint32_t)a.params.size();
+            p.n_layers = x.nl; p.rem_len = (uint32_t)(L.remainder.len / 16); p.q = a.num_queries;
+            p.log_n = log2u(a.n); p.log_N = log2u(a.lde_size()); p.grinding = a.grinding; p.air_id = a.id;
+            p.active = 1; p.ood = x.fail > VO_OOD ? 1 : 0;
+            // sorted assertions, parameters, boundary groups (g^step), columns, group offsets
+            const size_t na = a.assertions.size();
+            std::vector<uint32_t> goff;
+            std::vector<HF> gpts;
+            const HF g = HF::root_of_unity((int)p.log_n);
+            for (size_t k = 0; k < na; k++)
+                if (k == 0 || a.assertions[k].step != a.assertions[k - 1].step) { goff.push_back((uint32_t)k); gpts.push_back(g.pow((u128)a.assertions[k].step)); }
+            goff.push_back((uint32_t)na);
+            p.ng = (uint32_t)gpts.size();
+            uint64_t o = o_air[i];
+            p.o_aval = o; for (size_t k = 0; k < na; k++) memcpy(H + o + 16 * k, &a.assertions[k].value, 16); o = al(o + na * 16);
+            p.o_params = o; memcpy(H + o, a.params.data(), a.params.size() * 16); o = al(o + a.params.size() * 16);
+            p.o_gpts = o; memcpy(H + o, gpts.data(), gpts.size() * 16); o = al(o + na * 16);
+            p.o_acol = o; for (size_t k = 0; k < na; k++) memcpy(H + o + 4 * k, &a.assertions[k].col, 4); o = al(o + na * 4);
+            p.o_goff = o; memcpy(H + o, goff.data(), goff.size() * 4);
+        });
+        const auto hp1 = std::chrono::steady_clock::now();
+        d_vstage.ensure(total);
+        d_vts.ensure((size_t)count * sizeof(DevTs));
+        h2d(d_vstage.p, H, total);
+        VArgs A{};
+        A.base = d_vstage.as<uint8_t>();
+        A.proofs = reinterpret_cast<const VProof*>(A.base + o_proofs);
+        A.ts = d_vts.as<DevTs>();
+        A.verdict = d_vstage.as<uint32_t>();
+        A.roots = reinterpret_cast<const fe*>(A.base + o_roots);
+        A.nodes = reinterpret_cast<const uint32_t*>(A.base + o_nodes);
+        A.n_nodes = n_nodes;
+        for (uint32_t lf = 1; lf <= 4; lf++) {   // folding constants of every factor (the prover's FriFoldParams has them per layer)
+            const HF wi = HF::root_of_unity((int)lf).inv();
+            HF x = HF::raw(1);
+            for (uint32_t k = 0; k < (1u << lf) / 2; k++) { A.fold_wf_inv[lf - 1][k] = to_fe(x); x = x * wi; }
+            A.fold_inv_f[lf - 1] = to_fe(HF::from_u64(1u << lf).inv());
+        }
+        k_v_channel<<<count, ZKB_FS_THREADS, 0, stream>>>(A);
+        check_launch();
+        k_v_ood<<<(unsigned)(((uint64_t)count * 32 + 127) / 128), 128, 0, stream>>>(A, count);
+        check_launch();
+        std::vector<DevTs> hts(count);
+        std::vector<uint32_t> dv(count);
+        CK(cudaMemcpyAsync(hts.data(), d_vts.p, (size_t)count * sizeof(DevTs), cudaMemcpyDeviceToHost, stream));
+        CK(cudaMemcpyAsync(dv.data(), d_vstage.p, (size_t)count * 4, cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));   // synchronisation 1: positions and the channel's verdicts
+        const auto hp2 = std::chrono::steady_clock::now();
+
+        // ---- plan: positions, position folding, Merkle merges, DEEP / FRI evaluations ----
+        std::vector<VPlan> plans(count);
+        host_parallel(count, [&](uint32_t i) {
+            VItem& x = it[i];
+            if (x.fail <= VO_OOD_SHAPE) return;
+            std::vector<VLeafJob>& leaves = plans[i].leaves;
+            std::vector<std::vector<MergeJob>>& merges = plans[i].merges;
+            std::vector<VRootJob>& roots_chk = plans[i].roots;
+            std::vector<VEvalJob>& evals = plans[i].evals;
+            uint32_t next_id = LOCAL_ID;
+            const AirSpec& a = x.air;
+            const ProofLayout& L = x.L;
+            uint32_t f = std::min(x.fail, dv[i]);
+            const uint32_t F = a.folding, w = a.w, c = x.c;
+            const uint32_t log_N = log2u(a.lde_size()), log_F = a.log_folding();
+            x.positions.assign(hts[i].positions, hts[i].positions + a.num_queries);
+            std::sort(x.positions.begin(), x.positions.end());
+            x.positions.erase(std::unique(x.positions.begin(), x.positions.end()), x.positions.end());
+            const std::vector<uint32_t>& pos = x.positions;
+            const size_t nq = pos.size();
+            auto leaf = [&](uint64_t o, uint32_t cnt, uint32_t ord) { leaves.push_back({o, cnt, next_id, i, ord}); return next_id++; };
+            auto tree = [&](uint32_t k, const std::vector<uint32_t>& idx, const std::vector<uint32_t>& ids, uint32_t ord) {
+                uint32_t root = 0;
+                if (!plan_batch_root(x.bp[k].depth, idx, ids, x.node_ids[k], merges, next_id, &root)) f = std::min(f, ord);
+                else roots_chk.push_back({x.o_comm + 32 * (uint64_t)k, root, i, ord, 0});
+            };
+            do {
+                if (f <= VO_UNIQUE) break;
+                if (L.n_unique != nq) { f = VO_UNIQUE; break; }
+                if (L.trace_rows.len != nq * w * 16) { f = VO_TRACE_VALUES; break; }
+                if (L.comp_rows.len != nq * c * 16) { f = VO_CONSTRAINT_VALUES; break; }
+                std::vector<uint32_t> tid, cid;
+                if (f > VO_TRACE_ROWS_PARSE) for (size_t q = 0; q < nq; q++) tid.push_back(leaf(x.o_trows + q * w * 16, w, VO_TRACE_ROWS_PARSE));
+                if (f > VO_CONSTRAINT_ROWS_PARSE) for (size_t q = 0; q < nq; q++) cid.push_back(leaf(x.o_crows + q * c * 16, c, VO_CONSTRAINT_ROWS_PARSE));
+                if (f > VO_TRACE_MERKLE) tree(0, pos, tid, VO_TRACE_MERKLE);
+                if (f > VO_CONSTRAINT_MERKLE) tree(1, pos, cid, VO_CONSTRAINT_MERKLE);
+                auto deep_job = [&](size_t q, uint64_t target, uint32_t ord) {
+                    evals.push_back({x.o_trows + q * w * 16, x.o_crows + q * c * 16, target, i, ~0u, pos[q], log_N, pos[q], log_N, ord, F});
+                };
+                std::vector<uint32_t> cur = pos, prev;
+                uint64_t dom = a.lde_size();
+                for (uint32_t l = 0; l < x.nl; l++) {
+                    const uint32_t base = VO_FRI0 + VO_FRI_STEP * l;
+                    if (f <= base) break;
+                    const std::vector<uint32_t> folded = fold_positions(cur, dom, F);
+                    const uint64_t rows = dom / F;
+                    if (L.fri_rows[l].len != folded.size() * F * 16) { f = base + VO_FRI_VALUES; break; }
+                    std::vector<uint32_t> ids;
+                    if (f > base + VO_FRI_ROWS_PARSE) for (size_t r = 0; r < folded.size(); r++) ids.push_back(leaf(x.o_fri[l] + r * F * 16, F, base + VO_FRI_ROWS_PARSE));
+                    if (f > base + VO_FRI_MERKLE) tree(2 + l, folded, ids, base + VO_FRI_MERKLE);
+                    if (f > base + VO_FRI_FOLDING) {   // get_query_values: position q sits in row (q mod rows), slot (q div rows)
+                        std::vector<std::pair<uint32_t, uint32_t>> row_of(folded.size());   // (folded position, row), ascending
+                        for (size_t r = 0; r < folded.size(); r++) row_of[r] = {folded[r], (uint32_t)r};
+                        std::sort(row_of.begin(), row_of.end());
+                        auto target = [&](uint32_t q) {
+                            const uint32_t fq = (uint32_t)(q % rows);
+                            const uint32_t r = std::lower_bound(row_of.begin(), row_of.end(), std::make_pair(fq, 0u))->second;
+                            return x.o_fri[l] + ((uint64_t)r * F + q / rows) * 16;
+                        };
+                        const uint32_t ord = base + VO_FRI_FOLDING;
+                        if (l == 0) for (size_t q = 0; q < nq; q++) deep_job(q, target(pos[q]), ord);
+                        else for (size_t r = 0; r < prev.size(); r++)
+                            evals.push_back({x.o_fri[l - 1] + r * F * 16, 0, target(prev[r]), i, l - 1, prev[r], log2u(dom * F), 0, 0, ord, F});
+                    }
+                    prev = folded; cur = folded; dom = rows;
+                }
+                if (f > VO_REM + 1) roots_chk.push_back({x.o_comm + 32 * (uint64_t)(2 + x.nl), leaf(x.o_rem, (uint32_t)(L.remainder.len / 16), VO_REM + 1), i, VO_REM + 1, 0});
+                if (f > VO_REM + 2) {   // the last evaluations against the remainder polynomial
+                    if (x.nl == 0) for (size_t q = 0; q < nq; q++) deep_job(q, ~0ull, VO_REM + 2);
+                    else for (size_t r = 0; r < prev.size(); r++)
+                        evals.push_back({x.o_fri[x.nl - 1] + r * F * 16, 0, ~0ull, i, x.nl - 1, prev[r], log2u(dom) + log_F, prev[r], log2u(dom), VO_REM + 2, F});
+                }
+            } while (false);
+            x.fail = f;
+            plans[i].ids = next_id - LOCAL_ID;
+        });
+        // one id space for the batch: each proof's ids follow the nodes and the ids of the proofs before it
+        std::vector<VLeafJob> leaves;
+        std::vector<std::vector<MergeJob>> merges;
+        std::vector<VRootJob> roots_chk;
+        std::vector<VEvalJob> evals;
+        uint32_t next_id = n_nodes;
+        for (uint32_t i = 0; i < count; i++) {
+            VPlan& pl = plans[i];
+            if ((uint64_t)next_id + pl.ids >= LOCAL_ID) throw InvalidArg("too many digests in one batch");
+            const uint32_t base = next_id;
+            auto reloc = [base](uint32_t id) { return id >= LOCAL_ID ? base + (id - LOCAL_ID) : id; };
+            for (VLeafJob j : pl.leaves) { j.out = reloc(j.out); leaves.push_back(j); }
+            if (merges.size() < pl.merges.size()) merges.resize(pl.merges.size());
+            for (size_t d = 0; d < pl.merges.size(); d++)
+                for (const MergeJob& j : pl.merges[d]) merges[d].push_back({reloc(j.a), reloc(j.b), reloc(j.out)});
+            for (VRootJob j : pl.roots) { j.id = reloc(j.id); roots_chk.push_back(j); }
+            evals.insert(evals.end(), pl.evals.begin(), pl.evals.end());
+            next_id += pl.ids;
+        }
+        const auto hp3 = std::chrono::steady_clock::now();
+        // ---- plan upload: [leaves][merges, level by level][roots][evaluations] ----
+        std::vector<size_t> lvl_off(merges.size() + 1, 0);
+        size_t po = al(leaves.size() * sizeof(VLeafJob));
+        for (size_t d = 0; d < merges.size(); d++) { lvl_off[d] = po; po = al(po + merges[d].size() * sizeof(VMergeJob)); }
+        const size_t o_rchk = po; po = al(po + roots_chk.size() * sizeof(VRootJob));
+        const size_t o_eval = po; po = al(po + evals.size() * sizeof(VEvalJob));
+        const size_t plan_bytes = std::max<size_t>(po, 16);
+        grow_pinned(h_vplan, h_vplan_cap, plan_bytes);
+        memcpy(h_vplan, leaves.data(), leaves.size() * sizeof(VLeafJob));
+        for (size_t d = 0; d < merges.size(); d++) {
+            static_assert(sizeof(MergeJob) == sizeof(VMergeJob), "merge job layouts differ");
+            memcpy(h_vplan + lvl_off[d], merges[d].data(), merges[d].size() * sizeof(VMergeJob));
+        }
+        memcpy(h_vplan + o_rchk, roots_chk.data(), roots_chk.size() * sizeof(VRootJob));
+        memcpy(h_vplan + o_eval, evals.data(), evals.size() * sizeof(VEvalJob));
+        d_vplan.ensure(plan_bytes);
+        d_vdig.ensure(std::max<size_t>(32, (size_t)(next_id - n_nodes) * 32));
+        h2d(d_vplan.p, h_vplan, plan_bytes);
+        A.dig = d_vdig.as<uint32_t>();
+        const uint8_t* P = d_vplan.as<uint8_t>();
+        auto grid = [](size_t n) { return (unsigned)((n + 127) / 128); };
+        if (!leaves.empty()) { k_v_leaves<<<grid(leaves.size()), 128, 0, stream>>>(A, (const VLeafJob*)P, (uint32_t)leaves.size()); check_launch(); }
+        for (size_t d = 0; d < merges.size(); d++) {
+            if (merges[d].empty()) continue;
+            k_v_merge<<<grid(merges[d].size()), 128, 0, stream>>>(A, (const VMergeJob*)(P + lvl_off[d]), (uint32_t)merges[d].size());
+            check_launch();
+        }
+        if (!roots_chk.empty()) { k_v_roots<<<grid(roots_chk.size()), 128, 0, stream>>>(A, (const VRootJob*)(P + o_rchk), (uint32_t)roots_chk.size()); check_launch(); }
+        if (!evals.empty()) { k_v_eval<<<grid(evals.size()), 128, 0, stream>>>(A, (const VEvalJob*)(P + o_eval), (uint32_t)evals.size()); check_launch(); }
+        CK(cudaMemcpyAsync(dv.data(), d_vstage.p, (size_t)count * 4, cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));   // synchronisation 2: the verdicts
+        if (host_prof) {
+            const auto hp4 = std::chrono::steady_clock::now();
+            auto us = [](auto a, auto b) { return std::chrono::duration<double, std::micro>(b - a).count(); };
+            fprintf(stderr, "[zkb verify] %u proofs: parse + pack %.1f us, upload + channel + OOD %.1f us, plan %.1f us (%zu leaves, %zu levels, "
+                    "%zu evaluations), upload + checks %.1f us\n", count, us(hp0, hp1), us(hp1, hp2), us(hp2, hp3), leaves.size(), merges.size(),
+                    evals.size(), us(hp3, hp4));
+        }
+        for (uint32_t i = 0; i < count; i++) {
+            VItem& x = it[i];
+            verdicts[i] = verdict_of(std::min(x.fail, dv[i]));
+            if (!tss) continue;
+            zkb_transcript& t = tss[i];
+            memset(&t, 0, sizeof(t));
+            t.comp_degree_ok = 1;
+            if (x.bp.empty()) continue;   // the channel did not run
+            const uint8_t* cm = proofs[i] + x.L.commitments.off;
+            const DevTs& h = hts[i];
+            memcpy(t.trace_root, cm, 32); memcpy(t.constraint_root, cm + 32, 32); memcpy(t.remainder_commitment, cm + 32 * (2 + x.nl), 32);
+            memcpy(t.constraint_alpha, &h.alpha, 16); memcpy(t.z, &h.z, 16); memcpy(t.deep_alpha, &h.deep_alpha, 16);
+            t.n_fri_layers = x.nl;
+            for (uint32_t l = 0; l < x.nl && l < TS_FRI_SLOTS; l++) { memcpy(t.fri_roots[l], cm + 32 * (2 + l), 32); memcpy(t.fri_alphas[l], &h.fri_alpha[l], 16); }
+            t.pow_nonce = x.L.nonce;
+            t.n_positions = (uint32_t)x.positions.size();
+            for (size_t q = 0; q < x.positions.size() && q < 256; q++) t.positions[q] = x.positions[q];
+        }
+    }
 };
 
 // ================================================================================================================
@@ -1547,6 +1937,7 @@ int32_t zkb_ctx_create_lane(int32_t device, zkb_ctx** out) {
 void zkb_ctx_destroy(zkb_ctx* ctx) { if (ctx) { ctx->destroy(); delete ctx; } }
 const char* zkb_last_error(const zkb_ctx* ctx) { return ctx ? ctx->err.c_str() : g_last_error.c_str(); }
 uint64_t zkb_kernel_launches(const zkb_ctx* ctx) { return ctx ? ctx->launches : 0; }
+uint64_t zkb_h2d_bytes(const zkb_ctx* ctx) { return ctx ? ctx->h2d_bytes : 0; }
 int32_t zkb_last_stage_times(const zkb_ctx* ctx, zkb_stage_times* out) {
     if (!ctx || !out) return ZKB_ERR_INVALID;
     zkb_ctx* c = const_cast<zkb_ctx*>(ctx);  // elapsed times are read from the recorded events on first request
@@ -1593,6 +1984,11 @@ int32_t zkb_prove_batch(zkb_ctx* const* lanes, uint32_t n_lanes, const zkb_air_d
     uint32_t first = UINT32_MAX; int32_t out = ZKB_OK;
     for (uint32_t l = 0; l < n_lanes; l++) if (rc[l] != ZKB_OK && failed[l] < first) { first = failed[l]; out = rc[l]; }
     return out;
+}
+
+int32_t zkb_verify_batch(zkb_ctx* ctx, const zkb_air_desc* const* airs, const uint8_t* const* proofs, const uint64_t* lens, uint32_t count,
+                         int32_t* verdicts_out, zkb_transcript* transcripts_out) {
+    return guarded(ctx, [&] { ctx->verify_batch(airs, proofs, lens, count, verdicts_out, transcripts_out); });
 }
 
 int32_t zkb_begin(zkb_ctx* ctx, const zkb_air_desc* air) { return guarded(ctx, [&] { ctx->begin(air); }); }

@@ -58,6 +58,8 @@ def load():
     lib.zkb_last_error.argtypes = [C.c_void_p]
     lib.zkb_kernel_launches.restype = C.c_uint64
     lib.zkb_kernel_launches.argtypes = [C.c_void_p]
+    lib.zkb_h2d_bytes.restype = C.c_uint64
+    lib.zkb_h2d_bytes.argtypes = [C.c_void_p]
     lib.zkb_host_alloc.restype = C.c_void_p
     lib.zkb_host_alloc.argtypes = [C.c_size_t]
     lib.zkb_host_free.argtypes = [C.c_void_p]
@@ -65,7 +67,7 @@ def load():
     lib.zkb_ctx_destroy.argtypes = [C.c_void_p]
     for name in EXPORTS:
         fn = getattr(lib, name)
-        if name not in ("zkb_last_error", "zkb_kernel_launches", "zkb_host_alloc", "zkb_host_free", "zkb_free", "zkb_ctx_destroy"):
+        if name not in ("zkb_last_error", "zkb_kernel_launches", "zkb_h2d_bytes", "zkb_host_alloc", "zkb_host_free", "zkb_free", "zkb_ctx_destroy"):
             fn.restype = C.c_int32
     _lib = lib
     return lib
@@ -73,12 +75,12 @@ def load():
 
 # every symbol include/zkb200.h declares
 EXPORTS = [
-    "zkb_ctx_create", "zkb_ctx_create_lane", "zkb_ctx_destroy", "zkb_last_error", "zkb_kernel_launches", "zkb_last_stage_times", "zkb_host_alloc",
+    "zkb_ctx_create", "zkb_ctx_create_lane", "zkb_ctx_destroy", "zkb_last_error", "zkb_kernel_launches", "zkb_h2d_bytes", "zkb_last_stage_times", "zkb_host_alloc",
     "zkb_host_free", "zkb_prove", "zkb_prove_device", "zkb_free", "zkb_begin", "zkb_trace_commit", "zkb_trace_commit_device",
     "zkb_trace_read_frame", "zkb_trace_read_frames", "zkb_trace_polys_read", "zkb_constraints_eval", "zkb_constraints_commit", "zkb_ood_eval",
     "zkb_deep_compose", "zkb_fri_num_layers", "zkb_fri_commit_layer", "zkb_fri_fold", "zkb_fri_remainder", "zkb_grind",
     "zkb_query", "zkb_mg_unique_id", "zkb_mg_init", "zkb_mg_prove", "zkb_mg_prove_device", "zkb_prove_batch", "zkb_mimc_trace", "zkb_mimc_trace_device", "zkb_training_trace_device", "zkb_download", "zkb_blake3_host", "zkb_mimc_cipher_batch", "zkb_mimc_hash_matrix_batch", "zkb_upload_trace", "zkb_test_field", "zkb_test_hash_elements",
-    "zkb_test_merkle_root", "zkb_test_lde",
+    "zkb_test_merkle_root", "zkb_test_lde", "zkb_verify_batch",
 ]
 
 
@@ -154,6 +156,9 @@ class Context:
     def launches(self):
         return int(self.lib.zkb_kernel_launches(self.handle))
 
+    def h2d_bytes(self):
+        return int(self.lib.zkb_h2d_bytes(self.handle))
+
     def stage_times(self):
         t = StageTimes()
         self.check(self.lib.zkb_last_stage_times(self.handle, C.byref(t)))
@@ -209,6 +214,21 @@ class Context:
         proof = C.string_at(out, ln.value)
         self.lib.zkb_free(out)
         return proof, ts
+
+    # ---- winterfell::verify for a batch ----
+    def verify_batch(self, airs, proofs):
+        """zkb_verify_batch: one zkb_verdict per proof (0 = accepted) and the transcripts the verifier re-derived.
+        airs: AIR descriptions (dicts or AirDesc), proofs: bytes, one per AIR."""
+        count = len(proofs)
+        descs = [self.prepare(a) for a in airs]
+        bufs = [bytes(p) for p in proofs]
+        air_arr = (C.POINTER(AirDesc) * max(count, 1))(*[C.pointer(d) for d in descs])
+        proof_arr = (C.c_char_p * max(count, 1))(*bufs)
+        lens = (C.c_uint64 * max(count, 1))(*[len(b) for b in bufs])
+        verdicts = (C.c_int32 * max(count, 1))()
+        ts = (Transcript * max(count, 1))()
+        self.check(self.lib.zkb_verify_batch(self.handle, air_arr, proof_arr, lens, C.c_uint32(count), verdicts, ts))
+        return [int(verdicts[i]) for i in range(count)], [ts[i] for i in range(count)]
 
     def upload_trace(self, trace_ptr, w, n):
         cols = self._col_ptrs(trace_ptr, w, n)

@@ -348,3 +348,65 @@ def verify(proof, air):
         if acc != e:
             raise VerifierError("invalid FRI remainder folding")
     return True
+
+
+# zkb_verdict (include/zkb200.h) -> the message `verify` raises for the same check
+VERDICT_MESSAGES = {
+    1: "proof deserialization failed",
+    2: "trace info in the proof does not match the AIR",
+    3: "unacceptable proof options",
+    4: "wrong number of commitments / FRI layers",
+    5: "malformed OOD trace frame",
+    6: "inconsistent OOD constraint evaluations",
+    7: "query seed proof-of-work verification failed",
+    8: "number of unique queries does not match the proof",
+    9: "malformed query values",
+    10: "trace query did not match the commitment",
+    11: "malformed query values",
+    12: "constraint query did not match the commitment",
+    13: "malformed FRI layer",
+    14: "FRI layer query did not match the commitment",
+    15: "invalid FRI layer folding",
+    16: "FRI degree truncation",
+    17: "FRI remainder mismatch",
+    18: "FRI remainder mismatch",
+    19: "invalid FRI remainder folding",
+}
+
+
+def verify_batch(proofs, airs, ctx=None):
+    """`winterfell::verify` for many proofs in one GPU call (zkb_verify_batch).  proofs: bytes or Proof objects; airs: one
+    `Air.describe()` dict per proof.  Returns one entry per proof: None when it is accepted, else a VerifierError carrying the
+    message `verify` raises for the first check it fails (its `verdict` attribute is the zkb_verdict value)."""
+    if not isinstance(proofs, (list, tuple)) or not isinstance(airs, (list, tuple)):
+        raise TypeError("proofs and airs must be lists")
+    if len(proofs) != len(airs):
+        raise ValueError(f"{len(proofs)} proofs but {len(airs)} AIR descriptions")
+    from .prover import Proof
+    data = []
+    for p in proofs:
+        b = p.to_bytes() if isinstance(p, Proof) else p
+        if not isinstance(b, (bytes, bytearray, memoryview)):
+            raise TypeError("every proof must be bytes or a Proof")
+        data.append(bytes(b))
+    for a in airs:
+        if not isinstance(a, (dict, _lib.AirDesc)):
+            raise TypeError("every AIR must be an Air.describe() dict")
+    if not data:
+        return []
+    own = ctx is None
+    ctx = _lib.Context(0) if own else ctx
+    try:
+        verdicts, _ = ctx.verify_batch(list(airs), data)
+    finally:
+        if own:
+            ctx.close()   # its stream, device buffers and pinned staging go now, not whenever the collector runs
+    out = []
+    for v in verdicts:
+        if v == 0:
+            out.append(None)
+        else:
+            e = VerifierError(VERDICT_MESSAGES[v])
+            e.verdict = v
+            out.append(e)
+    return out
