@@ -1,13 +1,20 @@
-"""Shared seeded inputs for the parity tests (SURVEY §8d: none of the reference's thread_rng sites are used)."""
+"""Shared seeded inputs and checks for the parity tests (SURVEY §8d: none of the reference's thread_rng sites are used)."""
+import ctypes as C
+import json
+import os
 import random
+import subprocess
+import sys
 
 import numpy as np
 
 import zk_stark_project_b200 as Z
 from zk_stark_project_b200 import field as F
+from zk_stark_project_b200 import lib as L
 from zk_stark_project_b200.training import AC, FE
 
 P = Z.P
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def splitmix(seed):
@@ -26,8 +33,8 @@ def splitmix(seed):
 from zk_stark_project_b200.synthetic import random_felts, synthetic_training_air  # noqa: E402,F401
 
 
-def options(blowup=16, queries=40, grinding=8):
-    return Z.ProofOptions(queries, blowup, grinding, Z.FieldExtension.NONE, 16, 7)
+def options(blowup=16, queries=40, grinding=8, folding=16, rem=7):
+    return Z.ProofOptions(queries, blowup, grinding, Z.FieldExtension.NONE, folding, rem)
 
 
 def model(rng, sigma):
@@ -58,6 +65,200 @@ def aggregation_prover(num_updates, opts, seed=0x5EED0003):
 
 def mimc_prover(width, steps, opts):
     return Z.MimcProver(opts, [j + 1 for j in range(width)], steps)
+
+
+# ---- cases: (AIR description, contiguous [w][n][2] uint64 trace) -------------------------------------------------------------
+
+def training_case(w, n, opts, seed):
+    """Training AIR over a random training-shaped trace (the training prover is data-oblivious, see synthetic.py)."""
+    data = random_felts(w * n, seed).reshape(w, n, 2)
+    return synthetic_training_air(n, opts, data), data
+
+
+def mimc_case(oracle, w, n, opts):
+    """MiMC chains seeded 1..w; traces longer than 1024 rows come from the oracle, which builds them much faster."""
+    p = mimc_prover(w, n, opts)
+    if n <= 1024:
+        return prover_case(p)
+    data = np.frombuffer(oracle.mimc_trace(p.seeds, n, p.rc), dtype=np.uint64).reshape(w, n, 2)
+    return p.describe(Z.TraceTable(data)), data
+
+
+def prover_case(prover):
+    trace = prover.build_trace()
+    return prover.describe(trace), np.ascontiguousarray(trace.data)
+
+
+def prove_both(ctx, oracle, air, data):
+    """Proves `data` on the GPU and with the oracle: the transcripts and then the proof bytes must be equal, and the oracle's
+    verifier and the product's Python verifier must accept the proof.  Returns the proof."""
+    data = np.ascontiguousarray(data)
+    ref, ts_o, _ = oracle.prove(air, data.tobytes())
+    proof, ts = ctx.prove_host(air, data.ctypes.data)
+    diff = transcript_diff(ts_o, ts)
+    assert diff is None, f"transcripts diverge at `{diff}`"
+    assert proof == ref, "proof bytes differ although the transcript matches"
+    oracle.verify(air, proof)
+    assert Z.verify(proof, air)
+    return proof
+
+
+# ---- the layout of Proof::to_bytes() -----------------------------------------------------------------------------------------
+
+def proof_sections(proof):
+    """Proof::to_bytes() cut into its data sections, in order: {name: slice}, length prefixes and constant bytes excluded.
+    The tests' only reader of the proof layout, kept apart from the verifiers it checks."""
+    pos = 0
+    out = {}
+
+    def take(name, k):
+        nonlocal pos
+        out[name] = slice(pos, pos + k)
+        pos += k
+
+    def vint():  # winter-utils vint64
+        nonlocal pos
+        first = proof[pos]
+        length = 9 if first == 0 else (first & -first).bit_length()
+        if length == 9:
+            v = int.from_bytes(proof[pos + 1:pos + 9], "little")
+        else:
+            v = int.from_bytes(proof[pos:pos + length], "little") >> length
+        pos += length
+        return v
+
+    def uint(k):
+        nonlocal pos
+        v = int.from_bytes(proof[pos:pos + k], "little")
+        pos += k
+        return v
+
+    take("context", 4 + 2 + 1 + 16 + 8 + 2 + 1)
+    take("commitments", uint(2))
+    for name in ("trace rows", "trace paths", "constraint rows", "constraint paths"):
+        take(name, vint())
+    tl = uint(2)
+    pos += 1
+    take("ood trace", tl - 1)
+    pos += 2
+    take("ood constraints", uint(2))
+    for layer in range(uint(1)):
+        take(f"fri values {layer}", uint(4))
+        take(f"fri paths {layer}", uint(4))
+    take("remainder", uint(2))
+    pos += 1
+    take("nonce", 8)
+    assert pos == len(proof)
+    return out
+
+
+def commitments(proof):
+    """Trace root, constraint root, one root per FRI layer, remainder commitment."""
+    blob = proof[proof_sections(proof)["commitments"]]
+    return [blob[i:i + 32] for i in range(0, len(blob), 32)]
+
+
+def fri_layers(proof):
+    """(queried values, BatchMerkleProof bytes) of every FRI layer."""
+    s = proof_sections(proof)
+    return [(proof[s[f"fri values {l}"]], proof[s[f"fri paths {l}"]]) for l in range(sum(k.startswith("fri values") for k in s))]
+
+
+# ---- the staged C ABI --------------------------------------------------------------------------------------------------------
+
+class Staged:
+    """One proof driven call by call through the staged surface of a Context (zkb_begin ... zkb_fri_remainder, zkb_query).
+    Each method marshals its call's arguments, raises ZkbError when the call fails and returns what the call writes."""
+
+    def __init__(self, ctx, air):
+        self.lib, self.h, self.check = ctx.lib, ctx.handle, ctx.check
+        self.w, self.n = air["trace_width"], air["trace_len"]
+        self.desc = L.make_desc(air)
+        self.check(self.lib.zkb_begin(self.h, C.byref(self.desc)))
+
+    def trace_commit(self, data):
+        """`data`: contiguous [w][n][2] trace.  Returns the trace root."""
+        cols = (C.c_void_p * self.w)(*[data.ctypes.data + j * self.n * 16 for j in range(self.w)])
+        root = C.create_string_buffer(32)
+        self.check(self.lib.zkb_trace_commit(self.h, cols, root))
+        return root.raw
+
+    def read_frame(self, step):
+        cur, nxt = C.create_string_buffer(16 * self.w), C.create_string_buffer(16 * self.w)
+        self.check(self.lib.zkb_trace_read_frame(self.h, C.c_uint64(step), cur, nxt))
+        return cur.raw, nxt.raw
+
+    def read_frames(self, steps):
+        k = len(steps)
+        cur, nxt = C.create_string_buffer(16 * self.w * k), C.create_string_buffer(16 * self.w * k)
+        self.check(self.lib.zkb_trace_read_frames(self.h, (C.c_uint64 * k)(*steps), C.c_uint32(k), cur, nxt))
+        return cur.raw, nxt.raw
+
+    def trace_polys(self):
+        out = C.create_string_buffer(16 * self.n * self.w)
+        self.check(self.lib.zkb_trace_polys_read(self.h, out))
+        return out.raw
+
+    def constraints_eval(self, alpha, ce=0):
+        """Returns the ce * n constraint evaluations when the constraint blowup `ce` is given, else None."""
+        ev = C.create_string_buffer(16 * self.n * ce) if ce else None
+        self.check(self.lib.zkb_constraints_eval(self.h, alpha, ev))
+        return ev.raw if ce else None
+
+    def constraints_commit(self):
+        root = C.create_string_buffer(32)
+        self.check(self.lib.zkb_constraints_commit(self.h, root))
+        return root.raw
+
+    def ood_eval(self, z):
+        self.check(self.lib.zkb_ood_eval(self.h, z, None, None, None))
+
+    def deep_compose(self, alpha):
+        self.check(self.lib.zkb_deep_compose(self.h, alpha))
+
+    def fri_num_layers(self):
+        nl = C.c_uint32()
+        self.check(self.lib.zkb_fri_num_layers(self.h, C.byref(nl)))
+        return nl.value
+
+    def fri_commit_layer(self):
+        root = C.create_string_buffer(32)
+        self.check(self.lib.zkb_fri_commit_layer(self.h, root))
+        return root.raw
+
+    def fri_fold(self, alpha):
+        self.check(self.lib.zkb_fri_fold(self.h, alpha))
+
+    def fri_remainder(self):
+        """Returns the remainder commitment."""
+        coeffs, count, root = C.create_string_buffer(16 * 256), C.c_uint64(), C.create_string_buffer(32)
+        self.check(self.lib.zkb_fri_remainder(self.h, coeffs, C.byref(count), root))
+        return root.raw
+
+    def query(self, which, positions, row_elems):
+        """Rows of `row_elems` elements and the BatchMerkleProof bytes of commitment `which` (0 trace, 1 constraints, 2 + l FRI
+        layer l) at `positions`."""
+        k = len(positions)
+        rows, po, ln = C.create_string_buffer(16 * row_elems * k), C.c_void_p(), C.c_uint64()
+        self.check(self.lib.zkb_query(self.h, C.c_uint32(which), (C.c_uint32 * k)(*positions), C.c_uint32(k), rows, C.byref(po), C.byref(ln)))
+        paths = C.string_at(po, ln.value)
+        self.lib.zkb_free(po)
+        return rows.raw, paths
+
+
+# ---- column-sharded proofs ---------------------------------------------------------------------------------------------------
+
+def run_sharded(ranks, port, cases, one_gpu):
+    """tests/mg_worker.py on `ranks` ranks under torchrun: each case's column-sharded proof must equal its single-GPU proof.
+    one_gpu: all ranks on the first visible GPU, talking over NCCL's socket transport on the loopback interface."""
+    env = dict(os.environ)
+    if one_gpu:
+        env.update(CUDA_VISIBLE_DEVICES=os.environ.get("CUDA_VISIBLE_DEVICES", "0").split(",")[0], NCCL_SOCKET_IFNAME="lo",
+                   GLOO_SOCKET_IFNAME="lo", NCCL_IB_DISABLE="1")
+    r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(ranks), "--master-addr", "127.0.0.1",
+                        "--master-port", str(port), "tests/mg_worker.py", json.dumps(cases)], cwd=ROOT, env=env, capture_output=True, text=True,
+                       timeout=600)
+    assert r.returncode == 0 and "mg ok" in r.stdout, f"{ranks} ranks: " + r.stdout[-2000:] + r.stderr[-2000:]
 
 
 TS_FIELDS = ["trace_root", "constraint_alpha", "constraint_root", "z", "deep_alpha", "n_fri_layers", "fri_roots", "fri_alphas",

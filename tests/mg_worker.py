@@ -2,6 +2,9 @@
 
   python -m torch.distributed.run --nnodes=1 --nproc-per-node G --master-addr 127.0.0.1 --master-port P tests/mg_worker.py [cases]
 
+cases: a JSON list of [kind, w, n, blowup] or [kind, w, n, blowup, folding] with kind "mimc" or "training"; FRI folding 16 when
+omitted.
+
 torch.distributed (gloo) is only the control plane here (NCCL id broadcast, result gathering); the data-path collectives
 run inside libzkb200.so on its own NCCL communicator."""
 import json
@@ -17,7 +20,7 @@ import torch.distributed as dist  # noqa: E402
 
 import zk_stark_project_b200 as Z  # noqa: E402
 from zk_stark_project_b200 import lib as L  # noqa: E402
-from zk_stark_project_b200 import synthetic as S  # noqa: E402
+from tests import common as T  # noqa: E402
 
 
 def main():
@@ -35,8 +38,9 @@ def main():
     cases = json.loads(sys.argv[1]) if len(sys.argv) > 1 else [["mimc", 64, 4096, 8], ["mimc", 16, 256, 8], ["training", 128, 1024, 16],
                                                                 ["training", 240, 512, 16], ["mimc", 24, 256, 8], ["mimc", 64, 1 << 16, 8]]
     results = []
-    for kind, w, n, blowup in cases:
-        opts = Z.ProofOptions(40, blowup, 16, Z.FieldExtension.NONE, 16, 7)
+    for case in cases:
+        kind, w, n, blowup, folding = (case + [16])[:5]
+        opts = T.options(blowup, 40, 16, folding)
         if kind == "mimc":
             rc = Z.get_round_constants()
             raw = ctx.mimc_trace([j + 1 for j in range(w)], n, rc)
@@ -44,8 +48,7 @@ def main():
             get = lambda c, r: int(data[c, r, 0]) | (int(data[c, r, 1]) << 64)
             air = Z.MimcAir(w, n, Z.MimcInputs([get(j, 0) for j in range(w)], [get(j, n - 1) for j in range(w)]), opts).describe()
         else:
-            data = S.random_felts(w * n, 99).reshape(w, n, 2)
-            air = S.synthetic_training_air(n, opts, data)
+            air, data = T.training_case(w, n, opts, 99)
         prepared = ctx.prepare(air)
         t0 = time.time()
         single, ts1 = ctx.prove_host(prepared, data.ctypes.data)
@@ -57,8 +60,8 @@ def main():
         sharded, ts2 = ctx.mg_prove_host(prepared, mine.ctypes.data, world)
         t3 = time.time()
         ok = sharded == single
-        results.append(dict(case=[kind, w, n, blowup], ok=ok, roots_equal=bytes(ts1.trace_root) == bytes(ts2.trace_root),
-                            z_equal=bytes(ts1.z) == bytes(ts2.z), single_ms=(t1 - t0) * 1e3, sharded_ms=(t3 - t2) * 1e3, proof_len=len(sharded)))
+        results.append(dict(case=case, ok=ok, roots_equal=bytes(ts1.trace_root) == bytes(ts2.trace_root), z_equal=bytes(ts1.z) == bytes(ts2.z),
+                            fri_layers=int(ts2.n_fri_layers), single_ms=(t1 - t0) * 1e3, sharded_ms=(t3 - t2) * 1e3, proof_len=len(sharded)))
     gathered = [None] * world
     dist.all_gather_object(gathered, results)
     if rank == 0:

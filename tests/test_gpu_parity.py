@@ -75,28 +75,10 @@ def test_interpolate_and_lde(gpu_ctx, oracle, n, w, blowup):
     assert lde.raw == o_lde, "LDE differs"
 
 
-def _prove_both(gpu_ctx, oracle, air, trace):
-    proof_o, ts_o, _ = oracle.prove(air, trace.to_bytes())
-    data = np.ascontiguousarray(trace.data)
-    proof_g, ts_g = gpu_ctx.prove_host(air, data.ctypes.data)
-    diff = T.transcript_diff(ts_o, ts_g)
-    assert diff is None, f"transcripts diverge at `{diff}`"
-    assert proof_g == proof_o, "proof bytes differ although the transcript matches"
-    oracle.verify(air, proof_g)
-    assert Z.verify(proof_g, air)  # the product's own (Python) verifier
-    return proof_g
-
-
 @pytest.mark.parametrize("width,steps,blowup", [(1, 64, 8), (4, 64, 8), (64, 256, 8), (3, 1024, 16), (8, 1 << 14, 8),
                                                 (64, 1 << 13, 8)])  # the last one takes the boundary-polynomial path
 def test_mimc_proof_parity(gpu_ctx, oracle, width, steps, blowup):
-    p = T.mimc_prover(width, steps, T.options(blowup=blowup))
-    if steps <= 1024:
-        trace = p.build_trace()
-    else:
-        raw = oracle.mimc_trace(p.seeds, steps, p.rc)
-        trace = Z.TraceTable(np.frombuffer(raw, dtype=np.uint64).reshape(width, steps, 2))
-    _prove_both(gpu_ctx, oracle, p.describe(trace), trace)
+    T.prove_both(gpu_ctx, oracle, *T.mimc_case(oracle, width, steps, T.options(blowup=blowup)))
 
 
 def test_mimc_device_trace(gpu_ctx, oracle):
@@ -107,31 +89,22 @@ def test_mimc_device_trace(gpu_ctx, oracle):
 
 @pytest.mark.parametrize("updates", [1, 6, 16, 30])
 def test_aggregation_proof_parity(gpu_ctx, oracle, updates):
-    p = T.aggregation_prover(updates, T.options())
-    trace = p.build_trace()
-    _prove_both(gpu_ctx, oracle, p.describe(trace), trace)
+    T.prove_both(gpu_ctx, oracle, *T.prover_case(T.aggregation_prover(updates, T.options())))
 
 
 @pytest.mark.parametrize("bs", [1, 2, 5])
 def test_training_proof_parity(gpu_ctx, oracle, bs):
-    p = T.training_prover(bs, T.options())
-    trace = p.build_trace()
-    _prove_both(gpu_ctx, oracle, p.describe(trace), trace)
+    T.prove_both(gpu_ctx, oracle, *T.prover_case(T.training_prover(bs, T.options())))
 
 
 def test_training_reference_options_bs1(gpu_ctx, oracle):
     """The exact ProofOptions of src/main.rs:98-107 (21-bit grinding): smallest-nonce PoW must match the oracle."""
-    p = T.training_prover(1, Z.ProofOptions.reference())
-    trace = p.build_trace()
-    _prove_both(gpu_ctx, oracle, p.describe(trace), trace)
+    T.prove_both(gpu_ctx, oracle, *T.prover_case(T.training_prover(1, Z.ProofOptions.reference())))
 
 
 def test_training_synthetic_8192(gpu_ctx, oracle):
     """bs=50-sized trace (the largest the reference CLI reaches, src/main.rs:77): two-pass NTT, 2^17-row LDE."""
-    n = 8192
-    data = T.random_felts(240 * n, 0x5EED0400).reshape(240, n, 2)
-    air = T.synthetic_training_air(n, T.options(), data)
-    _prove_both(gpu_ctx, oracle, air, Z.TraceTable(data))
+    T.prove_both(gpu_ctx, oracle, *T.training_case(240, 8192, T.options(), 0x5EED0400))
 
 
 def test_python_prover_surface(gpu_ctx, oracle):
@@ -147,12 +120,9 @@ def test_invalid_inputs_rejected(gpu_ctx):
     """tests/integration_tests.rs:201-230 expects a panic on mismatched batch sizes; the C ABI returns ZKB_ERR_INVALID."""
     with pytest.raises(AssertionError):
         Z.TrainingUpdateProver(T.options(), [[0] * 9] * 6, [0] * 6, [[0] * 9] * 6, [0] * 6, [[0] * 9], [[0] * 9], [[0] * 6], 1, 1, 2)
-    p = T.mimc_prover(2, 64, T.options(blowup=8))
-    trace = p.build_trace()
-    air = p.describe(trace)
+    air, data = T.prover_case(T.mimc_prover(2, 64, T.options(blowup=8)))
     bad = dict(air)
     bad["options"] = dict(air["options"], blowup=4)  # below the degree-7 constraint blowup
-    data = np.ascontiguousarray(trace.data)
     with pytest.raises(L.ZkbError) as e:
         gpu_ctx.prove_host(bad, data.ctypes.data)
     assert e.value.status == -1
@@ -163,86 +133,54 @@ def test_invalid_inputs_rejected(gpu_ctx):
 
 def test_staged_api_matches_one_shot(gpu_ctx, oracle):
     """The staged surface (TraceLde / ConstraintEvaluator / ConstraintCommitment + DEEP/FRI stages) reproduces the oracle transcript."""
-    p = T.aggregation_prover(16, T.options())
-    trace = p.build_trace()
-    air = p.describe(trace)
-    _, ts, _ = oracle.prove(air, trace.to_bytes())
-    lib, h = gpu_ctx.lib, gpu_ctx.handle
-    d = L.make_desc(air)
-    data = np.ascontiguousarray(trace.data)
-    w, n = trace.width(), trace.length()
-    cols = (C.c_void_p * w)(*[data.ctypes.data + j * n * 16 for j in range(w)])
-    root = C.create_string_buffer(32)
-    gpu_ctx.check(lib.zkb_begin(h, C.byref(d)))
-    gpu_ctx.check(lib.zkb_trace_commit(h, cols, root))
-    assert root.raw == bytes(ts.trace_root)
+    air, data = T.prover_case(T.aggregation_prover(16, T.options()))
+    _, ts, _ = oracle.prove(air, data.tobytes())
+    w, n = air["trace_width"], air["trace_len"]
+    st = T.Staged(gpu_ctx, air)
+    assert st.trace_commit(data) == bytes(ts.trace_root)
     # TraceLde::read_main_trace_frame_into
-    cur, nxt = C.create_string_buffer(16 * w), C.create_string_buffer(16 * w)
-    gpu_ctx.check(lib.zkb_trace_read_frame(h, C.c_uint64(0), cur, nxt))
-    _, lde, _ = oracle.trace_commit(trace.to_bytes(), n, w, 16, want_lde=True)
-    assert cur.raw == lde[:16 * w] and nxt.raw == lde[16 * 16 * w:17 * 16 * w]
-    gpu_ctx.check(lib.zkb_constraints_eval(h, bytes(ts.constraint_alpha), None))
-    gpu_ctx.check(lib.zkb_constraints_commit(h, root))
-    assert root.raw == bytes(ts.constraint_root)
+    cur, nxt = st.read_frame(0)
+    _, lde, _ = oracle.trace_commit(data.tobytes(), n, w, 16, want_lde=True)
+    assert cur == lde[:16 * w] and nxt == lde[16 * 16 * w:17 * 16 * w]
+    st.constraints_eval(bytes(ts.constraint_alpha))
+    assert st.constraints_commit() == bytes(ts.constraint_root)
     # out-of-order call is refused
-    assert lib.zkb_deep_compose(h, bytes(ts.deep_alpha)) == -3
-    gpu_ctx.check(lib.zkb_ood_eval(h, bytes(ts.z), None, None, None))
-    gpu_ctx.check(lib.zkb_deep_compose(h, bytes(ts.deep_alpha)))
-    nl = C.c_uint32()
-    gpu_ctx.check(lib.zkb_fri_num_layers(h, C.byref(nl)))
-    assert nl.value == ts.n_fri_layers
-    for l in range(nl.value):
-        gpu_ctx.check(lib.zkb_fri_commit_layer(h, root))
-        assert root.raw == bytes(ts.fri_roots[l])
-        gpu_ctx.check(lib.zkb_fri_fold(h, bytes(ts.fri_alphas[l])))
-    rem, cnt = C.create_string_buffer(16 * 64), C.c_uint64()
-    gpu_ctx.check(lib.zkb_fri_remainder(h, rem, C.byref(cnt), root))
-    assert root.raw == bytes(ts.remainder_commitment)
+    with pytest.raises(L.ZkbError) as e:
+        st.deep_compose(bytes(ts.deep_alpha))
+    assert e.value.status == -3
+    st.ood_eval(bytes(ts.z))
+    st.deep_compose(bytes(ts.deep_alpha))
+    nl = st.fri_num_layers()
+    assert nl == ts.n_fri_layers
+    for l in range(nl):
+        assert st.fri_commit_layer() == bytes(ts.fri_roots[l])
+        st.fri_fold(bytes(ts.fri_alphas[l]))
+    assert st.fri_remainder() == bytes(ts.remainder_commitment)
 
 
 def test_column_sharded_proof_two_gpus():
     """SURVEY §8e / BASELINE configs[4]: a proof produced cooperatively by 2 GPUs (column-sharded LDE, NVLink all-to-all,
     row-sharded hashing, all-gather of subtree roots) is byte-identical to the single-GPU proof."""
-    import subprocess
-    import sys
     import torch
     if torch.cuda.device_count() < 2:
         pytest.skip("needs 2 GPUs")
-    root = __import__("os").path.dirname(__import__("os").path.dirname(__import__("os").path.abspath(__file__)))
-    cases = '[["mimc", 64, 1024, 8], ["mimc", 16, 256, 8], ["training", 128, 512, 16], ["training", 240, 256, 16], ["mimc", 6, 128, 8]]'
-    r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
-                        "--master-port", "29611", "tests/mg_worker.py", cases], cwd=root, capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "mg ok" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
+    T.run_sharded(2, 29611, [["mimc", 64, 1024, 8], ["mimc", 16, 256, 8], ["training", 128, 512, 16], ["training", 240, 256, 16],
+                             ["mimc", 6, 128, 8]], one_gpu=False)
 
 
 def test_column_sharded_proof_ranks_share_one_gpu():
     """The sharded path with 2 and 4 ranks on one GPU, the ranks talking over NCCL's socket transport: rows and authentication
     nodes owned by one rank, the cap levels of the trace paths, the all-reduce of the openings, the OOD frame reorder and, with
     more ranks than the blowup, the replicated composition commitment.  The proofs must equal the single-GPU proof."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, CUDA_VISIBLE_DEVICES=os.environ.get("CUDA_VISIBLE_DEVICES", "0").split(",")[0], NCCL_SOCKET_IFNAME="lo",
-               GLOO_SOCKET_IFNAME="lo", NCCL_IB_DISABLE="1")
-    for g, port, cases in ((2, 29613, '[["mimc", 64, 1024, 8], ["training", 128, 512, 16], ["mimc", 6, 128, 8]]'),
-                           (4, 29615, '[["training", 128, 1024, 2], ["mimc", 16, 256, 8]]')):
-        r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(g), "--master-addr", "127.0.0.1",
-                            "--master-port", str(port), "tests/mg_worker.py", cases], cwd=root, env=env, capture_output=True, text=True, timeout=600)
-        assert r.returncode == 0 and "mg ok" in r.stdout, f"{g} ranks: " + r.stdout[-2000:] + r.stderr[-2000:]
-
-
-def _training_shaped(oracle, gpu_ctx, w, n, opts, seed):
-    data = T.random_felts(w * n, seed).reshape(w, n, 2)
-    air = T.synthetic_training_air(n, opts, data)
-    return _prove_both(gpu_ctx, oracle, air, Z.TraceTable(data))
+    T.run_sharded(2, 29613, [["mimc", 64, 1024, 8], ["training", 128, 512, 16], ["mimc", 6, 128, 8]], one_gpu=True)
+    T.run_sharded(4, 29615, [["training", 128, 1024, 2], ["mimc", 16, 256, 8]], one_gpu=True)
 
 
 @pytest.mark.parametrize("w,n,blowup", [(2, 8, 2), (2, 8, 16), (4, 16, 4), (254, 16, 8), (6, 32, 32), (10, 64, 64), (2, 8, 128), (30, 2048, 2)])
 def test_edge_shapes_training_air(gpu_ctx, oracle, w, n, blowup):
     """Minimum trace length (TraceInfo: n >= 8), extreme widths, every blowup factor ProofOptions accepts (2..128),
     domains small enough that FRI has zero layers (N <= 128: the remainder is interpolated straight from the DEEP evaluations)."""
-    _training_shaped(oracle, gpu_ctx, w, n, Z.ProofOptions(27, blowup, 6, Z.FieldExtension.NONE, 16, 7), 31 * w + n)
+    T.prove_both(gpu_ctx, oracle, *T.training_case(w, n, T.options(blowup, 27, 6), 31 * w + n))
 
 
 @pytest.mark.parametrize("queries,grinding,rem", [(1, 0, 7), (255, 3, 7), (40, 10, 0), (40, 4, 3), (40, 4, 15), (12, 32 - 16, 31)])
@@ -252,39 +190,32 @@ def test_option_extremes(gpu_ctx, oracle, queries, grinding, rem):
     # with remainder degree 0 FRI folds all the way to a constant: the trace length must be a power of the folding factor
     # or the verifier reports degree truncation (as Winterfell's does)
     n = 4096 if rem == 0 else 1024
-    _training_shaped(oracle, gpu_ctx, 8, n, opts, 77 + queries)
+    T.prove_both(gpu_ctx, oracle, *T.training_case(8, n, opts, 77 + queries))
 
 
 def test_mimc_width_255_like(gpu_ctx, oracle):
     """Widest MiMC trace that still fits TraceInfo (255 columns: 4 BLAKE3 chunks per leaf with a ragged tail)."""
-    p = T.mimc_prover(255, 64, T.options(blowup=8))
-    trace = p.build_trace()
-    _prove_both(gpu_ctx, oracle, p.describe(trace), trace)
+    T.prove_both(gpu_ctx, oracle, *T.mimc_case(oracle, 255, 64, T.options(blowup=8)))
 
 
 def test_repeated_proofs_reuse_context(gpu_ctx, oracle):
     """A context is reused across proofs of different shapes (buffers grow, tables are rebuilt); results stay exact."""
     for width, steps, blowup in [(4, 4096, 8), (2, 64, 16), (16, 512, 8), (4, 4096, 8)]:
-        p = T.mimc_prover(width, steps, T.options(blowup=blowup))
-        raw = oracle.mimc_trace(p.seeds, steps, p.rc)
-        trace = Z.TraceTable(np.frombuffer(raw, dtype=np.uint64).reshape(width, steps, 2))
-        _prove_both(gpu_ctx, oracle, p.describe(trace), trace)
+        T.prove_both(gpu_ctx, oracle, *T.mimc_case(oracle, width, steps, T.options(blowup=blowup)))
 
 
 def test_pageable_and_scattered_columns(gpu_ctx, oracle):
     """Columns handed over as separate, non-contiguous, pageable host buffers (what a Vec<Vec<Felt>> TraceTable looks like)."""
-    p = T.aggregation_prover(16, T.options())
-    trace = p.build_trace()
-    air = p.describe(trace)
-    w, n = trace.width(), trace.length()
-    cols = [np.array(trace.data[j], copy=True) for j in reversed(range(w))][::-1]  # separately allocated
+    air, data = T.prover_case(T.aggregation_prover(16, T.options()))
+    w = air["trace_width"]
+    cols = [np.array(data[j], copy=True) for j in reversed(range(w))][::-1]  # separately allocated
     ptrs = (C.c_void_p * w)(*[c.ctypes.data for c in cols])
     d = L.make_desc(air)
     out, ln, ts = C.c_void_p(), C.c_uint64(), L.Transcript()
     gpu_ctx.check(gpu_ctx.lib.zkb_prove(gpu_ctx.handle, C.byref(d), ptrs, C.c_uint64(0), C.byref(out), C.byref(ln), C.byref(ts)))
     proof = C.string_at(out, ln.value)
     gpu_ctx.lib.zkb_free(out)
-    ref, _, _ = oracle.prove(air, trace.to_bytes())
+    ref, _, _ = oracle.prove(air, data.tobytes())
     assert proof == ref
 
 
@@ -306,10 +237,8 @@ def test_mimc_helpers_batch(gpu_ctx):
 def test_full_size_training_proof(gpu_ctx, oracle):
     """BASELINE.json configs[1] at full size (2^16 x 240, blowup 16, the reference's exact options: 40 queries, 21-bit grinding):
     the CUDA proof equals the oracle's byte for byte and both verifier restatements accept it."""
-    n = 1 << 16
-    data = T.random_felts(240 * n, 0x5EED0002).reshape(240, n, 2)
-    air = T.synthetic_training_air(n, Z.ProofOptions.reference(), data)
-    proof, ts = gpu_ctx.prove_host(air, np.ascontiguousarray(data).ctypes.data)
+    air, data = T.training_case(240, 1 << 16, Z.ProofOptions.reference(), 0x5EED0002)
+    proof, ts = gpu_ctx.prove_host(air, data.ctypes.data)
     assert ts.n_fri_layers == 4 and ts.n_positions <= 40
     assert Z.verify(proof, air)
     oracle.verify(air, proof)
@@ -368,18 +297,15 @@ def test_randomized_shape_sweep(gpu_ctx, oracle):
             blowup = rng.choice([8, 16, 32])
             p = Z.MimcProver(Z.ProofOptions(rng.randint(1, 60), blowup, rng.randint(0, 8), Z.FieldExtension.NONE, 16, rng.choice([3, 7, 15])),
                              [rng.randrange(P) for _ in range(w)], n)
-            raw = oracle.mimc_trace(p.seeds, n, p.rc)
-            trace = Z.TraceTable(np.frombuffer(raw, dtype=np.uint64).reshape(w, n, 2))
-            air = p.describe(trace)
+            data = np.frombuffer(oracle.mimc_trace(p.seeds, n, p.rc), dtype=np.uint64).reshape(w, n, 2)
+            air = p.describe(Z.TraceTable(data))
         else:
             w = 2 * rng.randint(1, 127)
             blowup = rng.choice([2, 4, 8, 16, 32, 64])
             opts = Z.ProofOptions(rng.randint(1, 60), blowup, rng.randint(0, 8), Z.FieldExtension.NONE, 16, rng.choice([3, 7, 15]))
-            data = T.random_felts(w * n, 1000 + case).reshape(w, n, 2)
-            air = T.synthetic_training_air(n, opts, data)
-            trace = Z.TraceTable(data)
+            air, data = T.training_case(w, n, opts, 1000 + case)
         try:
-            _prove_both(gpu_ctx, oracle, air, trace)
+            T.prove_both(gpu_ctx, oracle, air, data)
         except RuntimeError as e:
             # the only legitimate verifier complaint for arbitrary option combinations (as in Winterfell): the remainder bound
             # does not divide the degree along the FRI layers
@@ -436,8 +362,7 @@ def test_native_prove_batch(gpu_ctx, oracle):
     jobs = []
     for i in range(7):
         p = T.mimc_prover(1 + i, 128, T.options(blowup=8, grinding=4)) if i % 2 else T.training_prover(1 + i // 2, T.options(grinding=4))
-        tr = p.build_trace()
-        jobs.append((p.describe(tr), np.ascontiguousarray(tr.data)))
+        jobs.append(T.prover_case(p))
     proofs = L.prove_batch(lanes, [a for a, _ in jobs], [d.ctypes.data for _, d in jobs])
     for (air, data), proof in zip(jobs, proofs):
         single, _ = gpu_ctx.prove_host(air, data.ctypes.data)

@@ -3,7 +3,6 @@ CPU oracle's verifier (orc_verify) on the same bytes, and every accepted proof's
 import ctypes as C
 import random
 
-import numpy as np
 import pytest
 
 import zk_stark_project_b200 as Z
@@ -36,110 +35,32 @@ def oracle_verdict(oracle, air, proof):
     return MALFORMED, None
 
 
-def opts(folding=16, blowup=16, rem=7, queries=40, grinding=8):
-    return Z.ProofOptions(queries, blowup, grinding, Z.FieldExtension.NONE, folding, rem)
-
-
-def training(w, n, o, seed):
-    data = T.random_felts(w * n, seed).reshape(w, n, 2)
-    return T.synthetic_training_air(n, o, data), np.ascontiguousarray(data)
-
-
-def mimc(oracle, w, n, o):
-    p = T.mimc_prover(w, n, o)
-    if n <= 1024:
-        tr = p.build_trace()
-    else:
-        tr = Z.TraceTable(np.frombuffer(oracle.mimc_trace(p.seeds, n, p.rc), dtype=np.uint64).reshape(w, n, 2))
-    return p.describe(tr), np.ascontiguousarray(tr.data)
-
-
-def prover_case(prover):
-    tr = prover.build_trace()
-    return prover.describe(tr), np.ascontiguousarray(tr.data)
-
-
-def gpu_prove(ctx, air, data):
-    return ctx.prove_host(air, data.ctypes.data)[0]
-
-
-def sections(proof):
-    """Proof::to_bytes() cut into named data sections [(name, start, end)] (length prefixes excluded)."""
-    pos = 0
-    out = []
-
-    def take(name, k):
-        nonlocal pos
-        out.append((name, pos, pos + k))
-        pos += k
-
-    def vint():
-        nonlocal pos
-        first = proof[pos]
-        length = 9 if first == 0 else (first & -first).bit_length()
-        if length == 9:
-            v = int.from_bytes(proof[pos + 1:pos + 9], "little")
-        else:
-            v = int.from_bytes(proof[pos:pos + length], "little") >> length
-        pos += length
-        return v
-
-    def uint(k):
-        nonlocal pos
-        v = int.from_bytes(proof[pos:pos + k], "little")
-        pos += k
-        return v
-
-    take("context", 4 + 2 + 1 + 16 + 8 + 2 + 1)
-    take("commitments", uint(2))
-    for name in ("trace rows", "trace paths", "constraint rows", "constraint paths"):
-        take(name, vint())
-    tl = uint(2)
-    pos += 1
-    take("ood trace", tl - 1)
-    pos += 2
-    take("ood constraints", uint(2))
-    nl = uint(1)
-    for layer in range(nl):
-        take(f"fri values {layer}", uint(4))
-        take(f"fri paths {layer}", uint(4))
-    take("remainder", uint(2))
-    pos += 1
-    take("nonce", 8)
-    assert pos == len(proof)
-    return out
-
-
-def gpu_verdicts(ctx, airs, proofs):
-    return ctx.verify_batch(airs, proofs)
-
-
 # ---- accepted proofs -----------------------------------------------------------------------------------------------------------
 
 def accepted_cases(oracle):
     ref = Z.ProofOptions.reference()
     cases = {
-        "training bs=1": prover_case(T.training_prover(1, ref)),
-        "training bs=2": prover_case(T.training_prover(2, ref)),
-        "configs[1] 2^16 x 240": training(240, 1 << 16, ref, 0x5EED0002),
-        "aggregation 1": prover_case(T.aggregation_prover(1, ref)),
-        "aggregation 6": prover_case(T.aggregation_prover(6, ref)),
-        "aggregation 16": prover_case(T.aggregation_prover(16, ref)),
-        "mimc 1x64": mimc(oracle, 1, 64, opts(blowup=8)),
-        "mimc 4x128": mimc(oracle, 4, 128, opts(blowup=8)),
-        "mimc 64x2^14": mimc(oracle, 64, 1 << 14, opts(blowup=8)),
-        "17 layers": training(2, 1 << 17, opts(2, blowup=2, rem=0), 0xF07D),
-        "0 layers": training(2, 8, opts(4), 0xF05D),
-        "remainder degree 0": training(8, 4096, opts(8, rem=0), 0xF06D),
-        "remainder degree 31": training(8, 1024, opts(4, rem=31), 0xF06E),
-        "1 query": training(8, 1024, opts(queries=1), 0xF101),
-        "255 queries": training(8, 1024, opts(queries=255), 0xF102),
-        "grinding 0": training(8, 1024, opts(grinding=0), 0xF103),
-        "grinding 21": training(8, 1024, opts(grinding=21), 0xF104),
+        "training bs=1": T.prover_case(T.training_prover(1, ref)),
+        "training bs=2": T.prover_case(T.training_prover(2, ref)),
+        "configs[1] 2^16 x 240": T.training_case(240, 1 << 16, ref, 0x5EED0002),
+        "aggregation 1": T.prover_case(T.aggregation_prover(1, ref)),
+        "aggregation 6": T.prover_case(T.aggregation_prover(6, ref)),
+        "aggregation 16": T.prover_case(T.aggregation_prover(16, ref)),
+        "mimc 1x64": T.mimc_case(oracle, 1, 64, T.options(blowup=8)),
+        "mimc 4x128": T.mimc_case(oracle, 4, 128, T.options(blowup=8)),
+        "mimc 64x2^14": T.mimc_case(oracle, 64, 1 << 14, T.options(blowup=8)),
+        "17 layers": T.training_case(2, 1 << 17, T.options(blowup=2, folding=2, rem=0), 0xF07D),
+        "0 layers": T.training_case(2, 8, T.options(folding=4), 0xF05D),
+        "remainder degree 0": T.training_case(8, 4096, T.options(folding=8, rem=0), 0xF06D),
+        "remainder degree 31": T.training_case(8, 1024, T.options(folding=4, rem=31), 0xF06E),
+        "1 query": T.training_case(8, 1024, T.options(queries=1), 0xF101),
+        "255 queries": T.training_case(8, 1024, T.options(queries=255), 0xF102),
+        "grinding 0": T.training_case(8, 1024, T.options(grinding=0), 0xF103),
+        "grinding 21": T.training_case(8, 1024, T.options(grinding=21), 0xF104),
     }
     for f in (2, 4, 8, 16):
-        cases[f"training folding {f}"] = training(8, 1024, opts(f), 0xF200 + f)
-        cases[f"mimc folding {f}"] = mimc(oracle, 4, 256, opts(f, blowup=8))
+        cases[f"training folding {f}"] = T.training_case(8, 1024, T.options(folding=f), 0xF200 + f)
+        cases[f"mimc folding {f}"] = T.mimc_case(oracle, 4, 256, T.options(blowup=8, folding=f))
     return cases
 
 
@@ -149,10 +70,10 @@ def test_accepted_proofs_and_transcripts(gpu_ctx, oracle):
     transcript the oracle verifier re-derives."""
     airs, proofs, names = [], [], []
     for name, (air, data) in accepted_cases(oracle).items():
-        airs.append(air); proofs.append(gpu_prove(gpu_ctx, air, data)); names.append(name + " (zkb_prove)")
+        airs.append(air); proofs.append(gpu_ctx.prove_host(air, data.ctypes.data)[0]); names.append(name + " (zkb_prove)")
         if data.size <= 2 * 8 * 4096 and air["options"]["grinding"] <= 8:
             airs.append(air); proofs.append(oracle.prove(air, data.tobytes())[0]); names.append(name + " (oracle)")
-    verdicts, ts = gpu_verdicts(gpu_ctx, airs, proofs)
+    verdicts, ts = gpu_ctx.verify_batch(airs, proofs)
     for name, air, proof, v, t in zip(names, airs, proofs, verdicts, ts):
         want, ts_o = oracle_verdict(oracle, air, proof)
         assert want == OK, name
@@ -166,10 +87,10 @@ def test_accepted_proofs_and_transcripts(gpu_ctx, oracle):
 def flip_cases(gpu_ctx, oracle):
     """(air, proof) pairs whose sections get flipped: training, MiMC and aggregation, two folding factors"""
     out = []
-    for air, data in (training(8, 1024, opts(), 0xF301), training(8, 1024, opts(4, queries=20), 0xF302),
-                      mimc(oracle, 4, 256, opts(blowup=8)), prover_case(T.aggregation_prover(6, opts()))):
-        out.append((air, gpu_prove(gpu_ctx, air, data)))
-    air, data = training(8, 512, opts(8), 0xF303)
+    for air, data in (T.training_case(8, 1024, T.options(), 0xF301), T.training_case(8, 1024, T.options(queries=20, folding=4), 0xF302),
+                      T.mimc_case(oracle, 4, 256, T.options(blowup=8)), T.prover_case(T.aggregation_prover(6, T.options()))):
+        out.append((air, gpu_ctx.prove_host(air, data.ctypes.data)[0]))
+    air, data = T.training_case(8, 512, T.options(folding=8), 0xF303)
     out.append((air, oracle.prove(air, data.tobytes())[0]))
     return out
 
@@ -181,7 +102,8 @@ def test_section_flips_match_oracle(gpu_ctx, oracle):
     rng = random.Random(0xF11F)
     airs, proofs, want = [], [], []
     for air, proof in flip_cases(gpu_ctx, oracle):
-        for name, a, b in sections(proof):
+        for name, span in T.proof_sections(proof).items():
+            a, b = span.start, span.stop
             if b <= a:
                 continue
             for _ in range(5 if b - a > 64 else 3):
@@ -189,7 +111,7 @@ def test_section_flips_match_oracle(gpu_ctx, oracle):
                 bad[rng.randrange(a, b)] ^= rng.randrange(1, 256)
                 airs.append(air); proofs.append(bytes(bad)); want.append((name, oracle_verdict(oracle, air, bytes(bad))[0]))
     assert len(proofs) >= 200
-    verdicts, _ = gpu_verdicts(gpu_ctx, airs, proofs)
+    verdicts, _ = gpu_ctx.verify_batch(airs, proofs)
     bad = [(n, w, v) for (n, w), v in zip(want, verdicts) if w != v]
     assert not bad, f"{len(bad)} of {len(want)} verdicts differ from the oracle, e.g. {bad[:5]}"
     assert len({w for _, w in want}) >= 8   # the flips reach many different checks
@@ -199,9 +121,9 @@ def test_section_flips_match_oracle(gpu_ctx, oracle):
 def test_truncations_and_other_inputs_match_oracle(gpu_ctx, oracle):
     """Truncation at every section boundary, one trailing byte, changed public input / assertion value / options, and the proof
     of an AIR-violating trace: the GPU verdict equals the oracle's."""
-    air, data = training(8, 1024, opts(), 0xF401)
-    proof = gpu_prove(gpu_ctx, air, data)
-    cases = [(air, proof[:a]) for _, a, _ in sections(proof)] + [(air, proof + b"\0"), (air, b"")]
+    air, data = T.training_case(8, 1024, T.options(), 0xF401)
+    proof = gpu_ctx.prove_host(air, data.ctypes.data)[0]
+    cases = [(air, proof[:span.start]) for span in T.proof_sections(proof).values()] + [(air, proof + b"\0"), (air, b"")]
     pub = dict(air, pub_elems=list(air["pub_elems"]))
     pub["pub_elems"][0] = (pub["pub_elems"][0] + 1) % Z.P
     cases.append((pub, proof))
@@ -211,15 +133,12 @@ def test_truncations_and_other_inputs_match_oracle(gpu_ctx, oracle):
     cases.append((av, proof))
     for k, v in (("num_queries", 41), ("folding", 8), ("blowup", 8)):
         cases.append((dict(air, options=dict(air["options"], **{k: v})), proof))
-    p = T.mimc_prover(2, 128, opts(blowup=8))
-    tr = p.build_trace()
-    mair = p.describe(tr)
-    bad_trace = np.ascontiguousarray(tr.data).copy()
+    mair, bad_trace = T.prover_case(T.mimc_prover(2, 128, T.options(blowup=8)))
     bad_trace[1, 77, 0] ^= 1
     bad_proof, ts = gpu_ctx.prove_host(mair, bad_trace.ctypes.data)
     assert ts.comp_degree_ok == 0
     cases.append((mair, bad_proof))
-    verdicts, _ = gpu_verdicts(gpu_ctx, [a for a, _ in cases], [q for _, q in cases])
+    verdicts, _ = gpu_ctx.verify_batch([a for a, _ in cases], [q for _, q in cases])
     want = [oracle_verdict(oracle, a, q)[0] for a, q in cases]
     assert verdicts == want
     assert want[-1] != OK and OK not in want
@@ -232,25 +151,26 @@ def test_mixed_batch_is_independent(gpu_ctx, oracle):
     """>= 64 proofs of the three AIRs, several shapes and options, valid and invalid interleaved: each gets the verdict it gets
     alone, and a permuted batch gives the permuted verdicts."""
     rng = random.Random(0xBA7C)
-    base = [training(8, 1024, opts(), 0xF501), training(16, 256, opts(2, blowup=4), 0xF502), mimc(oracle, 4, 256, opts(4, blowup=8)),
-            prover_case(T.aggregation_prover(3, opts())), training(2, 8, opts(8), 0xF503)]
+    base = [T.training_case(8, 1024, T.options(), 0xF501), T.training_case(16, 256, T.options(blowup=4, folding=2), 0xF502),
+            T.mimc_case(oracle, 4, 256, T.options(blowup=8, folding=4)), T.prover_case(T.aggregation_prover(3, T.options())),
+            T.training_case(2, 8, T.options(folding=8), 0xF503)]
     airs, proofs = [], []
     for i in range(72):
         air, data = base[i % len(base)]
-        proof = gpu_prove(gpu_ctx, air, data) if i < len(base) else proofs[i % len(base)]
+        proof = gpu_ctx.prove_host(air, data.ctypes.data)[0] if i < len(base) else proofs[i % len(base)]
         if i % 3 == 1:
             bad = bytearray(proof)
             bad[rng.randrange(len(bad))] ^= 0x40
             proof = bytes(bad)
         airs.append(air); proofs.append(proof)
-    together, _ = gpu_verdicts(gpu_ctx, airs, proofs)
-    alone = [gpu_verdicts(gpu_ctx, [a], [p])[0][0] for a, p in zip(airs, proofs)]
+    together, _ = gpu_ctx.verify_batch(airs, proofs)
+    alone = [gpu_ctx.verify_batch([a], [p])[0][0] for a, p in zip(airs, proofs)]
     assert together == alone
     assert together == [oracle_verdict(oracle, a, p)[0] for a, p in zip(airs, proofs)]
     assert OK in together and any(v != OK for v in together)
     perm = list(range(len(airs)))
     rng.shuffle(perm)
-    permuted, _ = gpu_verdicts(gpu_ctx, [airs[i] for i in perm], [proofs[i] for i in perm])
+    permuted, _ = gpu_ctx.verify_batch([airs[i] for i in perm], [proofs[i] for i in perm])
     assert permuted == [together[i] for i in perm]
 
 
@@ -260,11 +180,11 @@ def test_256_proofs_in_one_call(gpu_ctx):
     ref = Z.ProofOptions.reference()
     airs, proofs = [], []
     for k in range(4):
-        air, data = prover_case(T.training_prover(1, ref, seed=0x5EED0100 + k))
-        proof = gpu_prove(gpu_ctx, air, data)
+        air, data = T.prover_case(T.training_prover(1, ref, seed=0x5EED0100 + k))
+        proof = gpu_ctx.prove_host(air, data.ctypes.data)[0]
         airs += [air] * 64
         proofs += [proof] * 64
-    verdicts, _ = gpu_verdicts(gpu_ctx, airs, proofs)
+    verdicts, _ = gpu_ctx.verify_batch(airs, proofs)
     assert verdicts == [OK] * 256
 
 
@@ -274,8 +194,8 @@ def test_256_proofs_in_one_call(gpu_ctx):
 def test_arguments(gpu_ctx):
     lib = gpu_ctx.lib
     assert lib.zkb_verify_batch(gpu_ctx.handle, None, None, None, C.c_uint32(0), None, None) == 0
-    air, data = training(8, 64, opts(), 0xF601)
-    proof = gpu_prove(gpu_ctx, air, data)
+    air, data = T.training_case(8, 64, T.options(), 0xF601)
+    proof = gpu_ctx.prove_host(air, data.ctypes.data)[0]
     d = L.make_desc(air)
     airs = (C.POINTER(L.AirDesc) * 1)(C.pointer(d))
     proofs = (C.c_char_p * 1)(proof)
@@ -300,18 +220,18 @@ def test_verify_prove_verify_matches_fresh_context(oracle):
     """Verify, prove, verify on one context: proofs are byte-identical to a fresh context's, including an aggregation proof
     replayed from a CUDA graph after the verifier's buffers grew."""
     ctx = L.Context(0)
-    agg_air, agg = prover_case(T.aggregation_prover(16, Z.ProofOptions.reference()))
-    big_air, big = training(240, 1 << 12, opts(), 0xF701)
-    first = [gpu_prove(ctx, agg_air, agg) for _ in range(3)]   # eager, capture, replay
+    agg_air, agg = T.prover_case(T.aggregation_prover(16, Z.ProofOptions.reference()))
+    big_air, big = T.training_case(240, 1 << 12, T.options(), 0xF701)
+    first = [ctx.prove_host(agg_air, agg.ctypes.data)[0] for _ in range(3)]   # eager, capture, replay
     assert ctx.verify_batch([agg_air] * 3, first)[0] == [OK] * 3
-    proofs = [gpu_prove(ctx, big_air, big)]
+    proofs = [ctx.prove_host(big_air, big.ctypes.data)[0]]
     v, _ = ctx.verify_batch([big_air] * 200, proofs * 200)    # grows the verifier's buffers
     assert v == [OK] * 200
-    again = [gpu_prove(ctx, agg_air, agg) for _ in range(3)]
+    again = [ctx.prove_host(agg_air, agg.ctypes.data)[0] for _ in range(3)]
     fresh = L.Context(0)
-    ref = gpu_prove(fresh, agg_air, agg)
+    ref = fresh.prove_host(agg_air, agg.ctypes.data)[0]
     assert all(p == ref for p in first + again)
-    assert gpu_prove(ctx, big_air, big) == gpu_prove(fresh, big_air, big) == proofs[0]
+    assert ctx.prove_host(big_air, big.ctypes.data)[0] == fresh.prove_host(big_air, big.ctypes.data)[0] == proofs[0]
     assert ctx.verify_batch([agg_air, big_air], [again[-1], proofs[0]])[0] == [OK, OK]
     ctx.close(); fresh.close()
 

@@ -224,3 +224,25 @@ def test_bench_algorithmic_bytes_match_survey():
     assert abs(bench.algorithmic_bytes(1 << 16, 240, 16, 2, 1)["total"] / gib - 9.47) < 0.02
     assert abs(bench.algorithmic_bytes(1 << 20, 64, 8, 8, 6)["total"] / gib - 33.5) < 0.1
     assert abs(bench.algorithmic_bytes(1 << 20, 240, 16, 2, 1)["total"] / gib - 151.6) < 0.2
+
+
+def test_library_rebuilds_when_any_source_changes(tmp_path, monkeypatch):
+    """build.needs_build() watches every file in csrc/, not a list of names: a newer coin.cuh (the device Fiat-Shamir channel,
+    included by kernels.cuh) makes the library stale."""
+    import os
+    import shutil
+    from zk_stark_project_b200 import build
+    csrc = tmp_path / "zk_stark_project_b200" / "csrc"
+    shutil.copytree(build.CSRC, csrc)
+    (tmp_path / "include").mkdir()
+    shutil.copy(os.path.join(build.CSRC, "..", "..", "include", "zkb200.h"), tmp_path / "include")
+    lib = tmp_path / "zk_stark_project_b200" / "libzkb200.so"
+    lib.write_bytes(b"")
+    monkeypatch.setattr(build, "CSRC", str(csrc))
+    monkeypatch.setattr(build, "LIB", str(lib))
+    t = os.path.getmtime(lib)
+    for f in list(csrc.iterdir()) + [tmp_path / "include" / "zkb200.h"]:
+        os.utime(f, (t - 60, t - 60))
+    assert not build.needs_build()
+    os.utime(csrc / "coin.cuh", (t + 60, t + 60))
+    assert build.needs_build()

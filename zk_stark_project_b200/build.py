@@ -6,16 +6,18 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libzkb200.so")
 SOURCES = ["zkb200.cu"]
-HEADERS = ["f128.cuh", "blake3.cuh", "kernels.cuh", "verify.cuh", "host.hpp", "hostfield.hpp", "nccl_loader.hpp", "../../include/zkb200.h"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-shared",
               "-Xcompiler", "-fPIC", "-diag-suppress", "550"]
 
 
 def needs_build():
+    """True when the library is missing or older than a file it is compiled from: any file in csrc/, or the public header
+    that csrc/host.hpp includes."""
     if not os.path.exists(LIB):
         return True
     t = os.path.getmtime(LIB)
-    return any(os.path.getmtime(os.path.join(CSRC, f)) > t for f in SOURCES + HEADERS)
+    files = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(CSRC, "..", "..", "include", "zkb200.h")]
+    return any(os.path.getmtime(f) > t for f in files)
 
 
 def build(force=False, verbose=False):
